@@ -12,6 +12,9 @@ synthetic positions (SURVEY.md section 8d generator, random-init ConvNetV1 weigh
             algorithmic FLOP (2*MAC, unpadded) / average duration vs the measured bf16 peak of MEASURED_PEAKS.json.
   cpu_baseline  the oracle's restatement of the reference's torch-py CPU engine on the box's host cores (rank 0, N=1).
 
+`--dump-outputs DIR` writes what `value` and `e2e` returned in their last timed step.  Weights and positions are seeded, so
+two builds run with the same arguments can be compared output for output.
+
 `--impl reference` times that CPU path alone (the reference has no GPU code of its own and its Rust engines cannot be
 built here: no cargo/rustc, no ONNX Runtime / tract / ExecuTorch wheels -- see DESIGN.md).
 
@@ -35,6 +38,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the tree this runs from may be read-only: the bench writes nothing there
 
 WORKLOADS = {
     # name: (oracle config, device batch, device batches per step)
@@ -228,6 +232,32 @@ def make_inputs(cfg, n, seed):
         return games.synth_chess_positions(n, seed)
     words, _ = games.synth_hex_positions(n, cfg.board_size, seed)
     return words, None
+
+
+DUMP_BYTES = 60 << 20  # what --dump-outputs writes in all stays under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each (probs, offsets, values) triple of `outputs` ({prefix: what eval_batch returns}) as
+    out_dir/<prefix>_{probs,offsets,values,positions}.npy: probs and values float32, offsets and position indices float64
+    (exact).  If all of it would exceed DUMP_BYTES, every triple is cut to the same share of its positions, a fixed seeded
+    sample, and offsets index the sampled probabilities."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    total = sum(p.size * 4 + o.size * 8 + v.size * 4 + v.size * 8 for p, o, v in outputs.values())
+    share = min(1.0, DUMP_BYTES / max(1, total))
+    for prefix, (probs, offsets, values) in outputs.items():
+        n = len(values)
+        offsets = offsets.astype(np.int64)
+        pos = np.arange(n)
+        if share < 1.0:
+            pos = np.sort(np.random.default_rng(0).choice(n, max(1, int(n * share)), replace=False))
+            probs = np.concatenate([probs[offsets[i]:offsets[i + 1]] for i in pos])
+            offsets = np.concatenate([[0], np.cumsum(np.diff(offsets)[pos])])
+        np.save(out_dir / f"{prefix}_probs.npy", np.asarray(probs, dtype=np.float32))
+        np.save(out_dir / f"{prefix}_offsets.npy", offsets.astype(np.float64))
+        np.save(out_dir / f"{prefix}_values.npy", np.asarray(values[pos], dtype=np.float32))
+        np.save(out_dir / f"{prefix}_positions.npy", pos.astype(np.float64))
 
 
 def cpu_reference_step(model, cfg, words, bitmaps, liboracle):
@@ -498,7 +528,12 @@ def main():
     ap.add_argument("--single-search", action="store_true", default=True,
                     help="also time ONE tree searching with --sim-num 10000 (BASELINE configs[4]'s UCI setting, on the self-play game): "
                          "two games, one thread, one leaf at a time through cattus_b200_eval")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed paths returned in their last step (rank 0): resident_* from the device-resident "
+                         "batch of `value`, e2e_* from the host-buffer call of `e2e`, as DIR/<name>.npy (float32 / float64, < 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "cattus_b200":
+        ap.error("--dump-outputs applies to --impl cattus_b200")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -578,6 +613,9 @@ def main():
     barrier()
     clocks = sampler.end()
     t_value = max_over_ranks(float(ms_all.sum()) * 1e-3)
+    dumped = {}
+    if args.dump_outputs and rank == 0:
+        dumped["resident"] = nw.resident_download(batch)
     if rank == 0:
         sweep.append({"batch": batch, "ms": float(np.mean(ms_all)), "positions_per_sec": batch / (float(np.mean(ms_all)) * 1e-3)})
 
@@ -615,6 +653,9 @@ def main():
     barrier()
     clocks_e2e = sampler.end(t_e2e0)
     t_e2e = max_over_ranks(t_e2e_local)
+    if args.dump_outputs and rank == 0:
+        dumped["e2e"] = (probs, offsets, values)
+        dump_outputs(args.dump_outputs, dumped)
     launches = nw.metrics()["model.kernel_launches"] - launches0
     # per position: 8-byte prefix (probability offset, #legal) + packed planes (+ the legal bitmap padded to 8 B for chess)
     rec_bytes = 8 + cfg.planes * ((cfg.board_size ** 2 + 63) // 64) * 8 + (((cfg.moves + 31) // 32 * 4 + 7) // 8 * 8 if bitmaps is not None else 0)
