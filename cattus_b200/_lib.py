@@ -13,7 +13,8 @@ from . import build as _build
 
 OK, EINVAL, ENODEV, ECUDA, ENOMEM, ERANGE, EDEVICE = 0, -1, -2, -3, -4, -5, -6
 GAME_TTT, GAME_HEX, GAME_CHESS = 0, 1, 2
-PRECISION_BF16, PRECISION_FP32_CHECK = 0, 1
+PRECISION_BF16, PRECISION_FP32_CHECK, PRECISION_FP8 = 0, 1, 2
+PRECISION_IDS = {"bf16": PRECISION_BF16, "fp32-check": PRECISION_FP32_CHECK, "fp8": PRECISION_FP8}
 TRUNK_PER_LAYER, TRUNK_FUSED, TRUNK_SMALL, TRUNK_FP32, TRUNK_DENSE = 0, 1, 2, 3, 4
 TRUNK_PATH_NAMES = {TRUNK_PER_LAYER: "per-layer", TRUNK_FUSED: "fused", TRUNK_SMALL: "small", TRUNK_FP32: "fp32-check", TRUNK_DENSE: "dense"}
 GAME_IDS = {"ttt": GAME_TTT, "hex": GAME_HEX, "chess": GAME_CHESS}

@@ -171,7 +171,7 @@ Engine::Engine(const cattus_b200_desc& desc, const void* blob_bytes, size_t blob
     chk(desc.policy_channels, d_.ph, "policy_channels");
     if (desc.game != d_.game) throw Error(CATTUS_B200_EINVAL, "descriptor game does not match the weight blob");
     if (desc.max_batch == 0 || desc.max_batch > (1u << 16)) throw Error(CATTUS_B200_EINVAL, "max_batch must be in 1..65536");
-    if (desc.precision > CATTUS_B200_PRECISION_FP32_CHECK) throw Error(CATTUS_B200_EINVAL, "unknown precision");
+    if (desc.precision > CATTUS_B200_PRECISION_FP8) throw Error(CATTUS_B200_EINVAL, "unknown precision");
     max_batch_ = desc.max_batch;
     precision_ = desc.precision;
     const uint32_t n_streams = std::max<uint32_t>(1, std::min<uint32_t>(desc.n_streams, 32));
@@ -226,12 +226,24 @@ Engine::Engine(const cattus_b200_desc& desc, const void* blob_bytes, size_t blob
     CB2_CUDA(cudaFuncSetAttribute(tc_gemm_dual_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes(kTcStages)));
     CB2_CUDA(cudaFuncSetAttribute(tc_gemm_dual_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes(kTcStagesDeep)));
     // whole-trunk kernel: 8x8 boards, 128 filters (flags bit 0 forces the per-layer path, used by the parity tests)
-    fused_trunk_ = !simple_ && precision_ == CATTUS_B200_PRECISION_BF16 && d_.s == 8 && (d_.f == 64 || d_.f == 128 || d_.f == 256) && d_.c_in <= 32 &&
-                   d_.wpp() == 1 && (desc.flags & 1u) == 0 && (sm_count_ >= 2) && vhp_ + php_ <= 64;
+    // FP8 exists only as an instantiation of this kernel: every other shape is refused rather than run in another precision
+    fp8_ = precision_ == CATTUS_B200_PRECISION_FP8;
+    const bool fused_shape = !simple_ && d_.s == 8 && (d_.f == 64 || d_.f == 128 || d_.f == 256) && d_.c_in <= 32 && d_.wpp() == 1 &&
+                             (desc.flags & 1u) == 0 && (sm_count_ >= 2) && vhp_ + php_ <= 64;
+    if (fp8_ && !fused_shape)
+        throw Error(CATTUS_B200_EINVAL, "precision FP8 is only available on the whole-trunk kernel: ConvNetV1 with 8x8 boards, 64 / 128 / 256 filters, "
+                                        "<= 32 input planes, value + policy head channels (each padded to 16) <= 64, and flags bit 0 clear; this net has S=" +
+                                            std::to_string(d_.s) + " F=" + std::to_string(d_.f) + " C_in=" + std::to_string(d_.c_in) + " VH=" +
+                                            std::to_string(d_.vh) + " PH=" + std::to_string(d_.ph) + (simple_ ? " (SimpleTwoHeadedModel)" : "") +
+                                            ((desc.flags & 1u) ? " flags bit 0 set" : ""));
+    fused_trunk_ = fused_shape && (precision_ == CATTUS_B200_PRECISION_BF16 || fp8_);
     if (fused_trunk_) {
-        if (d_.f == 64) CB2_CUDA(cudaFuncSetAttribute(trunk_fused_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, FtG<64>::kSmemBytes));
-        if (d_.f == 128) CB2_CUDA(cudaFuncSetAttribute(trunk_fused_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, FtG<128>::kSmemBytes));
-        if (d_.f == 256) CB2_CUDA(cudaFuncSetAttribute(trunk_fused_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, FtG<256>::kSmemBytes));
+        auto smem = [](auto kernel, int bytes) { CB2_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes)); };
+        using B = __nv_bfloat16;
+        using E8 = __nv_fp8_e4m3;
+        if (d_.f == 64) fp8_ ? smem(trunk_fused_kernel<64, E8>, FtG<64, E8>::kSmemBytes) : smem(trunk_fused_kernel<64, B>, FtG<64, B>::kSmemBytes);
+        if (d_.f == 128) fp8_ ? smem(trunk_fused_kernel<128, E8>, FtG<128, E8>::kSmemBytes) : smem(trunk_fused_kernel<128, B>, FtG<128, B>::kSmemBytes);
+        if (d_.f == 256) fp8_ ? smem(trunk_fused_kernel<256, E8>, FtG<256, E8>::kSmemBytes) : smem(trunk_fused_kernel<256, B>, FtG<256, B>::kSmemBytes);
     }
     // 16-filter nets (every shipped training config): whole trunk + both head convs in one kernel
     small_trunk_ = !simple_ && precision_ == CATTUS_B200_PRECISION_BF16 && d_.f == 16 && d_.c_in <= 32 && d_.s >= 3 && d_.s <= 11 && vhp_ + php_ <= 32 &&
@@ -304,6 +316,7 @@ Engine::~Engine() {
     vfc2_w_.free_();
     fused_w_.free_();
     fused_b_.free_();
+    fused_s_.free_();
     small_w_.free_();
     small_b_.free_();
     trace_.free_();
@@ -422,42 +435,65 @@ void Engine::upload_weights(const Blob& blob) {
     conv3(convs_[0], blob.stem, cin_pad_);
     for (size_t i = 0; i < blob.block_conv.size(); ++i) conv3(convs_[1 + i], blob.block_conv[i], ca_);
     if (fused_trunk_) {
-        // trunk_fused.cuh weight image: for each layer, each 16-channel k-chunk, each CTA rank (= half of the output
-        // channels) one block [tap 9][k-half 2][oc F / 2][ic 8] bf16, streamed as one TMA stage (F <= 128) or three (F = 256:
-        // 3 taps each).  Stem input channels padded to 32.  Last block per rank: the two head convs, 8 k-chunks per stage.
+        // trunk_fused.cuh weight image: for each layer, each k-chunk (16 input channels bf16, 32 e4m3), each CTA rank (= half of
+        // the output channels) one block [tap 9][k-half 2][oc F / 2][16 bytes of ic] (8 bf16 / 16 e4m3 channels), streamed as one
+        // TMA stage (F <= 128) or three (F = 256: 3 taps each).  Stem input channels padded to 32.  Last block per rank: the two
+        // head convs, 8 k-chunks per stage.
+        // FP8: every output channel of every conv (stem, block convs, head convs) is quantised on its own: amax_oc = max |w_oc|,
+        // q = e4m3_rn_satfinite(w * (448 / amax_oc)), dequantisation factor d_oc = amax_oc / 448 (1 for an all-zero channel),
+        // applied in the kernel's epilogue.  oracle/fp8.py: convnet_forward_fp8 does the same.
         const uint32_t layers = 1 + static_cast<uint32_t>(blob.block_conv.size());
-        const uint32_t F = d_.f, kcn = F / 16, npc = F / 2;
-        const size_t block_elems = static_cast<size_t>(9) * 2 * npc * 8;                   // FtG<F>::kBlockBytes / 2
-        const size_t stage_elems = static_cast<size_t>(F <= 128 ? 9 : 3) * 2 * npc * 8;   // FtG<F>::kWStage / 2
+        const uint32_t F = d_.f, ec = fp8_ ? 16 : 8, kcn = F / (2 * ec), stem_kc = 32 / (2 * ec), npc = F / 2;
+        const size_t block_elems = static_cast<size_t>(9) * 2 * npc * ec;                   // FtG<F, E>::kBlockBytes / sizeof(E)
+        const size_t stage_elems = static_cast<size_t>(F <= 128 ? 9 : 3) * 2 * npc * ec;   // FtG<F, E>::kWStage / sizeof(E)
         const uint32_t head_stages = kcn > 8 ? kcn / 8 : 1, head_kc = kcn / head_stages;
-        const size_t blocks = 2 + static_cast<size_t>(layers - 1) * kcn + 1;  // + one block for the two head convs
+        const size_t blocks = stem_kc + static_cast<size_t>(layers - 1) * kcn + 1;  // + one block for the two head convs
         std::vector<float> img(blocks * 2 * block_elems, 0.0f), bias(static_cast<size_t>(layers + 1) * F, 0.0f);
+        std::vector<float> dq(bias.size(), 1.0f), qs(bias.size(), 1.0f);  // FP8: d_oc and 448 / amax_oc per [layer][oc]
+        auto set_scale = [&](size_t row, float amax) {
+            if (fp8_ && amax > 0.0f) {
+                qs[row] = 448.0f / amax;
+                dq[row] = amax / 448.0f;
+            }
+        };
         for (uint32_t l = 0; l < layers; ++l) {
             const Blob::Conv& c = l == 0 ? blob.stem : blob.block_conv[l - 1];
-            const uint32_t nkc = l == 0 ? 2 : kcn;
-            const size_t base = l == 0 ? 0 : 2 + static_cast<size_t>(l - 1) * kcn;
-            for (uint32_t o = 0; o < F; ++o) bias[l * F + o] = D[c.b + o];
+            const uint32_t nkc = l == 0 ? stem_kc : kcn;
+            const size_t base = l == 0 ? 0 : stem_kc + static_cast<size_t>(l - 1) * kcn;
+            for (uint32_t o = 0; o < F; ++o) {
+                bias[l * F + o] = D[c.b + o];
+                float amax = 0.0f;
+                for (size_t i = 0; i < static_cast<size_t>(c.ci) * 9; ++i) amax = std::max(amax, std::fabs(D[c.w + static_cast<size_t>(o) * c.ci * 9 + i]));
+                set_scale(static_cast<size_t>(l) * F + o, amax);
+            }
             for (uint32_t kc = 0; kc < nkc; ++kc)
                 for (uint32_t rk = 0; rk < 2; ++rk) {
                     float* blk = img.data() + ((base + kc) * 2 + rk) * block_elems;
                     for (uint32_t tap = 0; tap < 9; ++tap)
                         for (uint32_t kh = 0; kh < 2; ++kh)
                             for (uint32_t n = 0; n < npc; ++n)
-                                for (uint32_t e2 = 0; e2 < 8; ++e2) {
-                                    const uint32_t ic = kc * 16 + kh * 8 + e2, oc = rk * npc + n;
-                                    if (ic < c.ci) blk[((tap * 2 + kh) * npc + n) * 8 + e2] = D[c.w + (static_cast<size_t>(oc) * c.ci + ic) * 9 + tap];
+                                for (uint32_t e2 = 0; e2 < ec; ++e2) {
+                                    const uint32_t ic = kc * 2 * ec + kh * ec + e2, oc = rk * npc + n;
+                                    if (ic < c.ci)
+                                        blk[((tap * 2 + kh) * npc + n) * ec + e2] = D[c.w + (static_cast<size_t>(oc) * c.ci + ic) * 9 + tap] * qs[static_cast<size_t>(l) * F + oc];
                                 }
                 }
         }
         {
-            // head stages: [k-chunk][k-half 2][oc (vhp + php) / 2][ic 8] per CTA rank; channel list = value | policy
+            // head stages: [k-chunk][k-half 2][oc (vhp + php) / 2][16 bytes of ic] per CTA rank; channel list = value | policy
             const uint32_t nh = vhp_ + php_, half = nh / 2;
-            const size_t base = 2 + static_cast<size_t>(layers - 1) * kcn;
+            const size_t base = stem_kc + static_cast<size_t>(layers - 1) * kcn;
+            const size_t hrow = static_cast<size_t>(layers) * F;
             auto head_w = [&](uint32_t ch, uint32_t ic) -> float {
                 if (ch < vhp_) return ch < d_.vh ? D[blob.vconv.w + static_cast<size_t>(ch) * F + ic] : 0.0f;
                 const uint32_t pc = ch - vhp_;
                 return pc < d_.ph ? D[blob.pconv.w + static_cast<size_t>(pc) * F + ic] : 0.0f;
             };
+            for (uint32_t ch = 0; ch < nh; ++ch) {
+                float amax = 0.0f;
+                for (uint32_t ic = 0; ic < F; ++ic) amax = std::max(amax, std::fabs(head_w(ch, ic)));
+                set_scale(hrow + ch, amax);
+            }
             for (uint32_t rk = 0; rk < 2; ++rk) {
                 float* blk = img.data() + (base * 2 + rk) * block_elems;
                 for (uint32_t kc = 0; kc < kcn; ++kc) {
@@ -465,13 +501,21 @@ void Engine::upload_weights(const Blob& blob) {
                     const uint32_t k8 = kc % head_kc;
                     for (uint32_t kh = 0; kh < 2; ++kh)
                         for (uint32_t n = 0; n < half; ++n)
-                            for (uint32_t e2 = 0; e2 < 8; ++e2) st[((k8 * 2 + kh) * half + n) * 8 + e2] = head_w(rk * half + n, kc * 16 + kh * 8 + e2);
+                            for (uint32_t e2 = 0; e2 < ec; ++e2)
+                                st[((k8 * 2 + kh) * half + n) * ec + e2] = head_w(rk * half + n, kc * 2 * ec + kh * ec + e2) * qs[hrow + rk * half + n];
                 }
             }
-            for (uint32_t o = 0; o < d_.vh; ++o) bias[static_cast<size_t>(layers) * F + o] = D[blob.vconv.b + o];
-            for (uint32_t o = 0; o < d_.ph; ++o) bias[static_cast<size_t>(layers) * F + vhp_ + o] = D[blob.pconv.b + o];
+            for (uint32_t o = 0; o < d_.vh; ++o) bias[hrow + o] = D[blob.vconv.b + o];
+            for (uint32_t o = 0; o < d_.ph; ++o) bias[hrow + vhp_ + o] = D[blob.pconv.b + o];
         }
-        upload(fused_w_, to_bf16(img));
+        if (fp8_) {
+            std::vector<uint8_t> q(img.size());
+            for (size_t i = 0; i < img.size(); ++i) q[i] = static_cast<uint8_t>(__nv_cvt_float_to_fp8(img[i], __NV_SATFINITE, __NV_E4M3));
+            upload(fused_w_, q);
+            upload(fused_s_, dq);
+        } else {
+            upload(fused_w_, to_bf16(img));
+        }
         upload(fused_b_, bias);
     }
     if (small_trunk_) {
@@ -962,7 +1006,8 @@ void Engine::build_ops_bf16(Lane& lane, uint32_t bucket, std::vector<Op>& ops, b
         {
             cuuint64_t gdim[2] = {256, w_rows};
             cuuint64_t gstr[1] = {256};
-            const int rows_per_stage = d_.f == 64 ? FtG<64>::kWRowsPerStage : d_.f == 128 ? FtG<128>::kWRowsPerStage : FtG<256>::kWRowsPerStage;
+            using B = __nv_bfloat16;  // stage bytes are the same for both element types
+            const int rows_per_stage = d_.f == 64 ? FtG<64, B>::kWRowsPerStage : d_.f == 128 ? FtG<128, B>::kWRowsPerStage : FtG<256, B>::kWRowsPerStage;
             cuuint32_t box[2] = {256, static_cast<cuuint32_t>(rows_per_stage)};
             cuuint32_t estr[2] = {1, 1};
             CUresult r = reinterpret_cast<EncodeTiledFn>(encode_tiled_)(&fp.tma_w, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, fused_w_.p, gdim, gstr, box, estr,
@@ -973,6 +1018,7 @@ void Engine::build_ops_bf16(Lane& lane, uint32_t bucket, std::vector<Op>& ops, b
         fp.recs = recs;
         fp.n_ptr = n_ptr;
         fp.bias = fused_b_.as<float>();
+        fp.scale = fp8_ ? fused_s_.as<float>() : nullptr;
         fp.out_v = lane.d_hv.as<__nv_bfloat16>();
         fp.out_p = lane.d_hp.as<__nv_bfloat16>();
         fp.vhp = static_cast<int>(vhp_);
@@ -993,13 +1039,21 @@ void Engine::build_ops_bf16(Lane& lane, uint32_t bucket, std::vector<Op>& ops, b
         const int pairs = std::min(sm / 2, fp.num_rounds);
         Op op;
         op.stage = 1;
-        op.name = "trunk_fused";
-        if (d_.f == 64)
-            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<64><<<2 * pairs, kFtThreads, FtG<64>::kSmemBytes, st>>>(fp); };
+        op.name = fp8_ ? "trunk_fused_fp8" : "trunk_fused";
+        using B = __nv_bfloat16;
+        using E8 = __nv_fp8_e4m3;
+        if (d_.f == 64 && !fp8_)
+            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<64, B><<<2 * pairs, kFtThreads, FtG<64, B>::kSmemBytes, st>>>(fp); };
+        else if (d_.f == 128 && !fp8_)
+            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<128, B><<<2 * pairs, kFtThreads, FtG<128, B>::kSmemBytes, st>>>(fp); };
+        else if (!fp8_)
+            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<256, B><<<2 * pairs, kFtThreads, FtG<256, B>::kSmemBytes, st>>>(fp); };
+        else if (d_.f == 64)
+            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<64, E8><<<2 * pairs, kFtThreads, FtG<64, E8>::kSmemBytes, st>>>(fp); };
         else if (d_.f == 128)
-            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<128><<<2 * pairs, kFtThreads, FtG<128>::kSmemBytes, st>>>(fp); };
+            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<128, E8><<<2 * pairs, kFtThreads, FtG<128, E8>::kSmemBytes, st>>>(fp); };
         else
-            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<256><<<2 * pairs, kFtThreads, FtG<256>::kSmemBytes, st>>>(fp); };
+            op.launch = [fp, pairs](cudaStream_t st) { trunk_fused_kernel<256, E8><<<2 * pairs, kFtThreads, FtG<256, E8>::kSmemBytes, st>>>(fp); };
         ops.push_back(op);
     } else if (small) {
         // encode + stem + all residual blocks + both 1x1 head convs in one launch (trunk_small.cuh)
@@ -1677,6 +1731,8 @@ void Engine::encode(const uint64_t* planes, uint32_t n, uint32_t batch, float* n
 }
 
 void Engine::run_dense(const float* nchw, uint32_t n, float* logits_out, float* values_out) {
+    if (fp8_) throw Error(CATTUS_B200_EINVAL, "run_dense: there is no dense-input path at precision FP8 (the FP8 trunk reads packed bitboards); "
+                                              "use a BF16 or FP32_CHECK handle");
     if (n == 0) return;
     if (!nchw || !logits_out || !values_out) throw Error(CATTUS_B200_EINVAL, "null argument");
     CB2_CUDA(cudaSetDevice(device_));

@@ -223,7 +223,8 @@ class Engine {
     uint32_t precision_ = 0;
     RecLayout rec_{};
     bool derive_legal_ = false;
-    bool fused_trunk_ = false;  // S == 8 && F == 128: whole-trunk kernel (trunk_fused.cuh)
+    bool fused_trunk_ = false;  // S == 8 && F in {64, 128, 256}: whole-trunk kernel (trunk_fused.cuh)
+    bool fp8_ = false;          // precision FP8: the whole-trunk kernel's e4m3 instantiation (only where fused_trunk_ holds)
     bool small_trunk_ = false;  // F == 16: whole trunk + head convs in one kernel (trunk_small.cuh)
     bool simple_ = false;       // SimpleTwoHeadedModel: three dense layers, no convolutions
 
@@ -244,6 +245,7 @@ class Engine {
     DeviceBuf vfc2_w_;
     float vfc2_b_ = 0.0f;
     DeviceBuf fused_w_, fused_b_;  // trunk_fused.cuh weight images + biases
+    DeviceBuf fused_s_;            // FP8: per-output-channel dequantisation factors, [layers + 1][F] like fused_b_
     DeviceBuf small_w_, small_b_;  // trunk_small.cuh weight image + biases
     DeviceBuf trace_;              // optional clock64 trace of trunk_small (CATTUS_B200_TRACE_TRUNK=1)
     uint32_t small_stem_kc_ = 1;

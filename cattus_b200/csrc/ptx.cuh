@@ -240,6 +240,18 @@ __device__ __forceinline__ void umma_bf16_ss_pair_lohi(uint32_t tmem_d, uint32_t
         "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// kind::f8f6f4 form of umma_bf16_ss_pair_lohi: 8-bit A and B (the formats are in `idesc`), K = 32 per instruction.
+__device__ __forceinline__ void umma_f8_ss_pair_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
+                                                     uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+        "setp.ne.b32 p, %6, 0;\n\t"
+        "mov.b64 da, {%1, %2};\n\t"
+        "mov.b64 db, {%3, %4};\n\t"
+        "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], da, db, %5, p;\n\t}" ::"r"(tmem_d),
+        "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 // commit of the pair's MMAs, arriving on the barrier at the same offset in every CTA of `cta_mask`
 __device__ __forceinline__ void umma_commit_pair_multicast(uint64_t* bar, uint16_t cta_mask) {
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
@@ -306,6 +318,21 @@ __device__ __forceinline__ uint64_t umma_desc_none(uint64_t hi, uint32_t smem_ad
 // N>>3 at [17,23), M>>4 at [24,29).
 __host__ __device__ constexpr uint32_t umma_idesc_bf16(uint32_t m, uint32_t n) {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// Instruction descriptor for kind::f8f6f4 with A = B = E4M3 (format code 0 in [7,10) and [10,13)), D fp32, both K-major.
+__host__ __device__ constexpr uint32_t umma_idesc_e4m3(uint32_t m, uint32_t n) {
+    return (1u << 4) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+
+// Two fp32 -> two e4m3 (round to nearest even, saturating to +-448), `lo` in the low byte: the byte at the lower address.
+__device__ __forceinline__ uint16_t cvt_e4m3x2(float lo, float hi) {
+    uint16_t r;
+    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(r) : "f"(hi), "f"(lo));
+    return r;
+}
+// Four fp32 -> four e4m3 packed little-endian into one 32-bit word.
+__device__ __forceinline__ uint32_t cvt_e4m3x4(float a, float b, float c, float d) {
+    return static_cast<uint32_t>(cvt_e4m3x2(a, b)) | (static_cast<uint32_t>(cvt_e4m3x2(c, d)) << 16);
 }
 
 }  // namespace ptx

@@ -30,7 +30,11 @@ def _ptr(a: np.ndarray, typ):
 class CudaNetwork:
     def __init__(self, model, game: str, *, device: int = 0, batch_size: int = 64, n_streams: int = 2,
                  precision: str = "bf16", cache: Optional[ValueFuncCache] = None, fused_trunk: bool = True, fault_inject: bool = False):
-        """model: path to a .cb2 blob, or the blob bytes (cattus_b200.export.export_blob)."""
+        """model: path to a .cb2 blob, or the blob bytes (cattus_b200.export.export_blob).
+
+        precision: "bf16" (default), "fp32-check" (CUDA-core fp32, for parity checks) or "fp8" (opt-in: the conv trunk in
+        e4m3 on the whole-trunk kernel; only 8x8 nets with 64 / 128 / 256 filters, anything else raises EINVAL -- see
+        CATTUS_B200_PRECISION_FP8 in include/cattus_b200.h for its numerics)."""
         self._lib = _lib.load()
         self._h = C.c_void_p()
         self.cache = cache
@@ -44,7 +48,7 @@ class CudaNetwork:
         desc.flags = 0 if fused_trunk else 1  # bit 0: force the per-layer kernels (parity tests compare both paths)
         if fault_inject:
             desc.flags |= 2  # bit 1: tests only -- a head GEMM tile never publishes its accumulator (include/cattus_b200.h)
-        desc.precision = {"bf16": _lib.PRECISION_BF16, "fp32-check": _lib.PRECISION_FP32_CHECK}[precision]
+        desc.precision = _lib.PRECISION_IDS[precision]
         if isinstance(model, (bytes, bytearray, memoryview)):
             buf = bytes(model)
             check(self._lib.cattus_b200_create_from_memory(C.byref(desc), buf, len(buf), C.byref(self._h)))

@@ -8,6 +8,7 @@ invokes it (training/cattus_train/train_process.py:159-170, :341-352):
 
 * the game and board size are read from the model blob's header (the reference has one binary per game);
 * `config.model.inference` may carry `{"engine": "cuda-b200", "device": 0, "precision": "bf16", "streams": 4}`;
+  `precision` is "bf16" (default), "fp32-check" or the opt-in "fp8" (8x8 nets with 64 / 128 / 256 filters only);
   `config.model.batch_size` is the evaluator's max batch; the optional top-level keys `games_per_thread`, `leaf_queue`
   and `seed` select this backend's many-games-per-thread arrangement (default 64 games per worker thread);
 * with few games per worker thread (`games_num / threads` <= 96) `speculate` defaults on: likely next leaves are evaluated

@@ -7,7 +7,8 @@ the `StockfishNet` placeholder it is built with today (cattus.rs:57-64; SURVEY.m
 `cfg.json` is the reference's config (cattus.rs:16-42): {"model": {"model_path", "inference", "batch_size"},
 "mcts": {"sim_num", "explore_factor", "temperature_policy", "prior_noise_alpha", "prior_noise_epsilon", "cache_size"},
 "threads"}; `model.model_path` is a `.cb2` blob (cattus_b200.export) and `model.inference` may carry
-{"engine": "cuda-b200", "device": 0, "precision": "bf16"}.
+{"engine": "cuda-b200", "device": 0, "precision": "bf16"} (precision "bf16", "fp32-check" or the opt-in "fp8" for 8x8 nets
+with 64 / 128 / 256 filters).
 
 `speculate` (top-level key, default 31; 0 = the reference's behaviour) lets up to that many likely next leaves ride along
 with the leaf the search is waiting for; they only land in the value-function cache, so the moves played are unchanged

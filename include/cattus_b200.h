@@ -56,6 +56,16 @@ extern "C" {
 /* precision: replaces the serde-tagged `InferenceConfig` variant (engine/src/net/model.rs:17-25) */
 #define CATTUS_B200_PRECISION_BF16 0       /* tcgen05 bf16 x bf16 -> fp32 accumulate */
 #define CATTUS_B200_PRECISION_FP32_CHECK 1 /* CUDA-core fp32 everywhere; the <=1e-4 check mode */
+/* Opt-in, never a default: the conv trunk (stem, residual blocks, both 1x1 head convs) on tcgen05 kind::f8f6f4, e4m3 x e4m3 ->
+ * fp32 accumulate, in the whole-trunk kernel only.  Weights are quantised per output channel at load (amax -> 448, scale applied
+ * in the epilogue); activations are cast to e4m3 (round to nearest even, saturating) without a scale; the residual stream, the
+ * head convs' outputs, the head FCs and the softmax stay bf16 / fp32.  About 10x the bf16 path's error against fp32 on the
+ * project's random-init nets; playing strength on a trained net is not measured.
+ * `create` accepts it only where CATTUS_B200_TRUNK_FUSED applies -- 8x8 boards, 64 / 128 / 256 filters, <= 32 planes,
+ * VH + PH <= 64 (each padded to 16), `flags` bit 0 clear -- and fails with CATTUS_B200_EINVAL otherwise (16-filter nets,
+ * SimpleTwoHeadedModel, the forced per-layer path).  Such a handle reports precision 2 and trunk_path FUSED;
+ * cattus_b200_run_dense on it returns CATTUS_B200_EINVAL (there is no dense-input FP8 path). */
+#define CATTUS_B200_PRECISION_FP8 2
 
 typedef struct cattus_b200 cattus_b200_t;
 
