@@ -84,6 +84,14 @@ class ChessInfo(C.Structure):
     ]
 
 
+class AnalysisPosition(C.Structure):
+    """cattus_b200_analysis_position (include/cattus_b200_analysis.h)."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("status", C.c_uint32), ("n_children", C.c_uint32), ("pv_len", C.c_uint32),
+        ("simulations", C.c_uint32), ("best_move", C.c_uint16), ("pad", C.c_uint16), ("q", C.c_float),
+    ]
+
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 _H = C.c_void_p
 _u16p = C.POINTER(C.c_uint16)
@@ -122,6 +130,13 @@ SYMBOLS = {
     "cattus_b200_chess_search_create_with": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(SelfPlayCfg), C.POINTER(_H)]),
     "cattus_b200_chess_search_go": (C.c_int, [_H, C.c_char_p, _u16p, C.c_uint32, _u16p, C.POINTER(ChessSearchStats)]),
     "cattus_b200_chess_search_destroy": (None, [_H]),
+    # include/cattus_b200_analysis.h
+    "cattus_b200_analyse": (C.c_int, [_H, C.POINTER(SelfPlayCfg), C.c_uint32, C.POINTER(C.c_char_p), _u16p, _u32p, C.POINTER(_H)]),
+    "cattus_b200_analysis_count": (C.c_int, [_H, _u32p]),
+    "cattus_b200_analysis_get": (C.c_int, [_H, C.c_uint32, C.POINTER(AnalysisPosition)]),
+    "cattus_b200_analysis_children": (C.c_int, [_H, C.c_uint32, _u16p, _u32p, _f32p, _f32p, C.c_uint32]),
+    "cattus_b200_analysis_pv": (C.c_int, [_H, C.c_uint32, _u16p, C.c_uint32]),
+    "cattus_b200_analysis_free": (None, [_H]),
     # include/cattus_b200_chess.h
     "cattus_b200_chess_position": (C.c_int, [C.c_char_p, _u16p, C.c_uint32, C.POINTER(ChessInfo)]),
     "cattus_b200_chess_perft": (C.c_int, [C.c_char_p, C.c_uint32, C.POINTER(C.c_uint64)]),

@@ -9,6 +9,7 @@
 // coming out through mapped pinned memory.
 #pragma once
 
+#include "dsearch_analysis.hpp"
 #include "dsearch_api.hpp"
 #include "dsearch_host.hpp"
 #include "engine.hpp"
@@ -61,13 +62,16 @@ struct DsPopulation {
     cudaEvent_t fork = nullptr, join = nullptr;
     cudaGraphExec_t graph = nullptr;
     void *d_cmds = nullptr, *d_status = nullptr, *d_cache_meta[2] = {nullptr, nullptr}, *d_cache_entries[2] = {nullptr, nullptr};
+    void* d_roots = nullptr;  // analysis: root histories of the population's current wave
 };
 
 template <class Rules>
 class DsCudaBackend {
   public:
+    // `analysis` (optional) switches the finished searches to the analysis result layout and adds the per-wave root upload
+    // of kCmdSetRoot; without it everything is the self-play arrangement.
     DsCudaBackend(const void* rules_blob, size_t rules_bytes, uint32_t max_children, Engine* e1, Engine* e2, const cattus_b200_selfplay_cfg& cfg,
-                  const sp::Params params[2], uint32_t n_slots)
+                  const sp::Params params[2], uint32_t n_slots, const ds::AnalysisOpts* analysis = nullptr)
         : max_children_(max_children), n_slots_(n_slots) {
         eng_[0] = e1;
         eng_[1] = e2;
@@ -135,7 +139,11 @@ class DsCudaBackend {
             const uint32_t hist_cap = Rules::kChess ? 128u : 1u;
             alloc(d_hist_, sizeof(typename Rules::Pos) * static_cast<size_t>(n_slots) * hist_cap);
             cmd_stride_ = ds::cmd_stride_for(max_children);
-            result_stride_ = ds::result_stride_for(max_children);
+            result_stride_ = analysis ? ds::analysis_stride_for(max_children) : ds::result_stride_for(max_children);
+            if (analysis) {
+                roots_cap_ = analysis->roots_cap;
+                CB2_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&h_roots_), sizeof(typename Rules::Pos) * roots_cap_ * n_bufs_, cudaHostAllocDefault));
+            }
             cmd_bytes_ = 16 + static_cast<size_t>(n_slots) * cmd_stride_;
             result_buf_bytes_ = static_cast<size_t>(n_slots) * result_stride_;
             CB2_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&h_results_), result_buf_bytes_ * n_bufs_, cudaHostAllocMapped));
@@ -219,6 +227,12 @@ class DsCudaBackend {
                 // evaluator / expand; its slots take part from the population's next wave on
                 p.begin_lead = begin_lead;
                 p.visit_budget = visit_budget;
+                if (analysis) {
+                    alloc(P.d_roots, sizeof(typename Rules::Pos) * roots_cap_);
+                    p.roots = static_cast<const typename Rules::Pos*>(P.d_roots);
+                    p.analysis = 1;
+                    p.pv_max = std::min<uint32_t>(analysis->pv_max, ds::kPvMax);
+                }
                 if (begin_lead) {
                     CB2_CUDA(cudaStreamCreateWithFlags(&P.side, cudaStreamNonBlocking));
                     CB2_CUDA(cudaEventCreateWithFlags(&P.fork, cudaEventDisableTiming));
@@ -244,11 +258,16 @@ class DsCudaBackend {
     uint32_t population_of(uint32_t slot) const { return slot >= split_ ? 1u : 0u; }
     double setup_seconds() const { return setup_seconds_; }
     uint8_t* cmd_block(uint32_t wave) { return h_cmds_ + static_cast<size_t>(wave % n_bufs_) * cmd_bytes_; }
+    // analysis: where the host stages a wave's root histories (roots_cap() positions), uploaded by submit()
+    typename Rules::Pos* roots_block(uint32_t wave) { return h_roots_ + static_cast<size_t>(wave % n_bufs_) * roots_cap_; }
+    uint32_t roots_cap() const { return roots_cap_; }
 
-    void submit(uint32_t wave, uint32_t pop, uint32_t n_cmds) {
+    void submit(uint32_t wave, uint32_t pop, uint32_t n_cmds, uint32_t n_roots = 0) {
         const uint32_t b = wave % n_bufs_;
         DsPopulation<Rules>& P = pop_[pop];
         wave_pop_[b] = pop;
+        if (n_roots)  // the previous wave's begin kernel is done with the buffer: same stream, earlier graph
+            CB2_CUDA(cudaMemcpyAsync(P.d_roots, roots_block(wave), sizeof(typename Rules::Pos) * n_roots, cudaMemcpyHostToDevice, P.stream));
         CB2_CUDA(cudaMemcpyAsync(P.d_cmds, cmd_block(wave), 16 + static_cast<size_t>(n_cmds) * cmd_stride_, cudaMemcpyHostToDevice, P.stream));
         CB2_CUDA(cudaGraphLaunch(P.graph, P.stream));
         CB2_CUDA(cudaMemcpyAsync(h_status_ + 64 * b, P.d_status, 64, cudaMemcpyDeviceToHost, P.stream));
@@ -339,7 +358,7 @@ class DsCudaBackend {
             if (P.fork) cudaEventDestroy(P.fork);
             if (P.join) cudaEventDestroy(P.join);
             P.fork = P.join = nullptr;
-            for (void** q : {&P.d_cmds, &P.d_status, &P.d_cache_meta[0], &P.d_cache_meta[1], &P.d_cache_entries[0], &P.d_cache_entries[1]}) {
+            for (void** q : {&P.d_cmds, &P.d_status, &P.d_cache_meta[0], &P.d_cache_meta[1], &P.d_cache_entries[0], &P.d_cache_entries[1], &P.d_roots}) {
                 if (*q) cudaFree(*q);
                 *q = nullptr;
             }
@@ -359,16 +378,19 @@ class DsCudaBackend {
         if (h_results_) cudaFreeHost(h_results_);
         if (h_cmds_) cudaFreeHost(h_cmds_);
         if (h_status_) cudaFreeHost(h_status_);
+        if (h_roots_) cudaFreeHost(h_roots_);
         h_results_ = h_cmds_ = h_status_ = nullptr;
+        h_roots_ = nullptr;
     }
 
     DsPopulation<Rules> pop_[2];
     Engine* eng_[2] = {nullptr, nullptr};
     uint32_t n_evals_ = 1, n_pops_ = 1, split_ = 0, depth_ = 2, n_bufs_ = 3, max_children_ = 0, n_slots_ = 0, pool_words_ = 0, cmd_stride_ = 0,
-             result_stride_ = 0, kernels_per_wave_ = 0;
+             result_stride_ = 0, kernels_per_wave_ = 0, roots_cap_ = 0;
     size_t cmd_bytes_ = 0, result_buf_bytes_ = 0;
     void *d_rules_ = nullptr, *d_slots_ = nullptr, *d_pools_ = nullptr, *d_paths_ = nullptr, *d_noise_ = nullptr, *d_hist_ = nullptr;
     uint8_t *h_results_ = nullptr, *h_cmds_ = nullptr, *h_status_ = nullptr;
+    typename Rules::Pos* h_roots_ = nullptr;
     std::vector<cudaEvent_t> events_;
     std::vector<uint32_t> wave_pop_;
     uint64_t waves_ = 0;
@@ -396,6 +418,67 @@ static void dsearch_run_rules(const Rules& rules, const void* blob, size_t blob_
         std::fprintf(stderr, "device search: fullest tree buffer used %u of %u words (%.0f %%)\n", be.max_used(), be.pool_words(),
                      100.0 * be.max_used() / std::max(1u, be.pool_words()));
     e1->note_resident(waves, sh.evaluations, waves * be.kernels_per_wave(), waves ? secs / static_cast<double>(waves) : 0.0);
+}
+
+// Batched analysis of given positions (dsearch_analysis.hpp) on model's device: the self-play backend with the analysis
+// result layout and kCmdSetRoot's root upload.
+template <class Rules>
+static void analyse_rules(const Rules& rules, const void* blob, size_t blob_bytes, uint32_t max_children, Engine* e, const cattus_b200_selfplay_cfg& cfg,
+                          uint32_t n, const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, std::vector<ds::AnalysisResult>& out) {
+    const sp::Params params[2] = {ds::analysis_params(cfg), ds::analysis_params(cfg)};
+    const auto hist = ds::analysis_histories(rules, n, fens, moves, move_offsets);
+    cattus_b200_info info;
+    e->get_info(&info);
+    if (info.game != cfg.game || (cfg.game == CATTUS_B200_GAME_HEX && info.board_size != cfg.board_size))
+        throw Error(CATTUS_B200_EINVAL, "analysis: the model was made for another game or board size than cfg");
+    if (cfg.device_games > info.max_batch)
+        throw Error(CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(cfg.device_games) + ") exceeds the evaluator's max_batch (" +
+                                            std::to_string(info.max_batch) + ")");
+    const uint32_t want = cfg.device_games ? cfg.device_games : info.max_batch;
+    const uint32_t n_slots = std::max<uint32_t>(1, std::min<uint32_t>(want, n));
+    if (n == 0) {
+        out.clear();
+        return;
+    }
+    // a wave's root upload: a few history positions per slot on average; a longer run of long histories waits a wave
+    const ds::AnalysisOpts opts{ds::kPvMax, n_slots * 8u + ds::hist_cap_for<Rules>()};
+    const auto t0 = std::chrono::steady_clock::now();
+    DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e, nullptr, cfg, params, n_slots, &opts);
+    ds::AnalysisDriver<Rules, DsCudaBackend<Rules>> drv(rules, params[0], be, hist, out);
+    drv.run();
+    const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    const uint64_t waves = be.waves();
+    e->note_resident(waves, drv.counters()[1], waves * be.kernels_per_wave(), waves ? secs / static_cast<double>(waves) : 0.0);
+}
+
+void analyse_run(cattus_b200_t* m, const cattus_b200_selfplay_cfg& cfg, uint32_t n, const char* const* fens, const uint16_t* moves,
+                 const uint32_t* move_offsets, std::vector<ds::AnalysisResult>& out) {
+    try {
+        if (!m) throw Error(CATTUS_B200_EINVAL, "null evaluator handle (there is no CPU fallback)");
+        if (cfg.struct_size != sizeof(cattus_b200_selfplay_cfg)) throw Error(CATTUS_B200_EINVAL, "selfplay cfg struct_size mismatch");
+        if (cfg.game == CATTUS_B200_GAME_HEX) {
+            const int s = static_cast<int>(cfg.board_size);
+            if (s < 2 || s > 11) throw Error(CATTUS_B200_EINVAL, "hex board_size must be 2..11");
+            if (s <= 8) {
+                sp::HexRulesT<uint64_t> rules(s);
+                analyse_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, n, fens, moves, move_offsets, out);
+            } else {
+                sp::HexRulesT<sp::u128> rules(s);
+                analyse_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, n, fens, moves, move_offsets, out);
+            }
+        } else if (cfg.game == CATTUS_B200_GAME_CHESS) {
+            sp::ChessRules rules;
+            analyse_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), m->engine, cfg, n, fens,
+                          moves, move_offsets, out);
+        } else if (cfg.game == CATTUS_B200_GAME_TTT) {
+            sp::TttRules rules;
+            analyse_rules(rules, &rules, sizeof(rules), 9u, m->engine, cfg, n, fens, moves, move_offsets, out);
+        } else {
+            throw Error(CATTUS_B200_EINVAL, "unknown game");
+        }
+    } catch (const sp::SpError& e) {
+        throw Error(e.code ? e.code : CATTUS_B200_EINVAL, e.msg);
+    }
 }
 
 void dsearch_run(cattus_b200_t* m1, cattus_b200_t* m2, const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], sp::Shared& sh) {

@@ -184,7 +184,7 @@ CB2_HD inline float fsqrt(float a) {
 
 // ------------------------------------------------------------------------------------------------ layouts
 enum Phase : uint32_t { kIdle = 0, kRun = 1, kWaitEval = 2, kDone = 3 };
-enum CmdFlags : uint32_t { kCmdNewGame = 1, kCmdMove = 2, kCmdStop = 4 };
+enum CmdFlags : uint32_t { kCmdNewGame = 1, kCmdMove = 2, kCmdStop = 4, kCmdSetRoot = 8 };
 enum ErrBits : uint32_t { kErrPool = 1, kErrPath = 2, kErrRows = 4, kErrNoise = 8 };
 
 // One per concurrent game.  Scalars only; the per-slot arrays (tree pools, path, noise, history) are separate.
@@ -239,14 +239,21 @@ struct CacheIo {
 };
 
 // Command block written by the host for one wave: [u32 n_cmds][u32 wave][8 B pad] then n_cmds commands of cmd_stride
-// bytes: Cmd header + noise[max_children] f32.
+// bytes: Cmd header + noise[max_children] f32.  kCmdSetRoot takes the slot's history from Params::roots[root_at, root_at +
+// root_len) (oldest first, the root last).
 struct Cmd {
-    uint32_t slot, flags, move, cur, noise_n, pad[3];
+    uint32_t slot, flags, move, cur, noise_n, root_at, root_len, pad;
 };
 // Result of one finished search, written by the device into mapped host memory: header + n[max_children] u32 +
 // move[max_children] u16 (in insertion order; the host turns them into edges() order).
 struct ResultHdr {
     uint32_t slot, count, pad[2];
+};
+// Result of one finished search in analysis mode (Params::analysis): header + pv[kPvMax] u16 + n[max_children] u32 +
+// w[max_children] f32 + init[max_children] f32 + move[max_children] u16, root children in insertion order.
+constexpr uint32_t kPvMax = 16;
+struct AnalysisHdr {
+    uint32_t slot, count, pv_len, pad;
 };
 
 template <class Rules>
@@ -279,6 +286,10 @@ struct Params {
     uint32_t begin_lead;            // 0: begin runs before select in the same wave; 1: overlapped, effective next wave
     uint32_t visit_budget;          // node visits per slot and wave after which select stops starting new simulations
     uint32_t slot_base;             // the host's number of this population's slot 0 (two populations alternate waves)
+    // analysis of given positions (dsearch_analysis.hpp); all zero in self-play
+    const typename Rules::Pos* roots;  // root histories of this wave's kCmdSetRoot commands
+    uint32_t analysis;                 // 1: finished searches post the AnalysisHdr layout instead of ResultHdr
+    uint32_t pv_max;                   // principal variation plies to post (<= kPvMax)
 };
 
 template <class Pos>
@@ -427,6 +438,10 @@ struct Core {
 
     // The finished search's root rows, for the host: calc_moves_probabilities' tail and the move choice run there.
     CB2_HD static void post_results(const P& p, uint32_t wave, uint32_t si, uint32_t* pool, int32_t root) {
+        if (p.analysis) {
+            post_analysis(p, wave, si, pool, root);
+            return;
+        }
         const int ln = lane();
         const int count = T::hdr(pool, root)->count;
         uint32_t k = 0;
@@ -444,6 +459,62 @@ struct Core {
         for (int i = ln; i < count; i += DS_LANES) {
             rn[i] = static_cast<uint32_t>(ch[i].n);
             rm[i] = static_cast<uint16_t>(move_at(pool, root, count, i));
+        }
+    }
+
+    // Analysis result: every root row, and the principal variation -- from the root, repeatedly the child with the most
+    // visits, equal counts going to the smallest insertion index (the last maximum in edges() order, as
+    // choose_move_from_probabilities at temperature 0 picks), until a node that was never expanded or pv_max plies.
+    CB2_HD static void post_analysis(const P& p, uint32_t wave, uint32_t si, uint32_t* pool, int32_t root) {
+        const int ln = lane();
+        const int count = T::hdr(pool, root)->count;
+        uint32_t k = 0;
+        if (ln == 0) k = atomic_add_u32(p.done_count, 1u);
+        k = wbcast(k);
+        uint8_t* e = p.results + static_cast<unsigned long long>(wave % p.n_result_bufs) * p.result_buf_bytes + static_cast<size_t>(k) * p.result_stride;
+        uint16_t* pv = reinterpret_cast<uint16_t*>(e + sizeof(AnalysisHdr));
+        uint32_t* rn = reinterpret_cast<uint32_t*>(e + sizeof(AnalysisHdr) + 2u * kPvMax);
+        float* rw = reinterpret_cast<float*>(rn + p.max_children);
+        float* ri = rw + p.max_children;
+        uint16_t* rm = reinterpret_cast<uint16_t*>(ri + p.max_children);
+        const Child* ch = T::child(pool, root);
+        for (int i = ln; i < count; i += DS_LANES) {
+            const Child c = ch[i];
+            rn[i] = static_cast<uint32_t>(c.n);
+            rw[i] = c.w;
+            ri[i] = c.init;
+            rm[i] = static_cast<uint16_t>(move_at(pool, root, count, i));
+        }
+        int32_t node = root;
+        uint32_t len = 0;
+        while (len < p.pv_max) {
+            const Hdr* h = T::hdr(pool, node);
+            const int cnt = h->count;
+            if (!h->expanded || cnt == 0) break;
+            const Child* c = T::child(pool, node);
+            float bv = -1.0f;
+            int bi = 0x7FFFFFFF;
+            uint32_t be = 0;
+            for (int i = ln; i < cnt; i += DS_LANES) {  // ascending i with a strict > keeps the smallest index among equals
+                const float v = static_cast<float>(c[i].n);
+                if (bi == 0x7FFFFFFF || v > bv) {
+                    bv = v;
+                    bi = i;
+                    be = c[i].edge;
+                }
+            }
+            wargmax(bv, bi, be);
+            if (ln == 0) pv[len] = static_cast<uint16_t>(move_at(pool, node, cnt, bi));
+            len += 1;
+            node = T::edge_child(be);
+            if (node < 0) break;
+        }
+        if (ln == 0) {
+            AnalysisHdr* ah = reinterpret_cast<AnalysisHdr*>(e);
+            ah->slot = si + p.slot_base;
+            ah->count = static_cast<uint32_t>(count);
+            ah->pv_len = len;
+            ah->pad = 0;
         }
     }
 
@@ -1068,6 +1139,14 @@ struct Core {
             buf[1] = 1;
             hist_len = 1;
             if (ln == 0) hist[0] = R.initial();
+        } else if (cmd.flags & kCmdSetRoot) {
+            // a fresh tree at a position the host gives, with the history detect_repetition looks back into
+            root[0] = root[1] = -1;
+            used[0] = used[1] = 0;
+            buf[0] = 0;
+            buf[1] = 1;
+            hist_len = cmd.root_len;
+            for (uint32_t i = static_cast<uint32_t>(ln); i < hist_len; i += DS_LANES) hist[i] = p.roots[cmd.root_at + i];
         } else if (cmd.flags & kCmdMove) {
             if (ln == 0) {
                 Pos np = R.moved(hist[(hist_len - 1u) & hmask], static_cast<typename Rules::Move>(cmd.move));

@@ -2210,6 +2210,39 @@ int cattus_b200_get_metrics(const cattus_b200_t* h, cattus_b200_metrics* out) {
     });
 }
 
+// ---------------------------------------------------------------- batched analysis (include/cattus_b200_analysis.h)
+struct cattus_b200_analysis {
+    std::vector<ds::AnalysisResult> res;
+};
+
+int cattus_b200_analyse(cattus_b200_t* model, const cattus_b200_selfplay_cfg* cfg, uint32_t n, const char* const* fens, const uint16_t* moves,
+                        const uint32_t* move_offsets, cattus_b200_analysis_t** out) {
+    return guarded([&] {
+        if (!cfg || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        *out = nullptr;
+        std::unique_ptr<cattus_b200_analysis> r(new cattus_b200_analysis());
+        cb2::analyse_run(model, *cfg, n, fens, moves, move_offsets, r->res);
+        *out = r.release();
+    });
+}
+
+int cattus_b200_analysis_count(const cattus_b200_analysis_t* r, uint32_t* n) {
+    if (!r || !n) return CATTUS_B200_EINVAL;
+    *n = static_cast<uint32_t>(r->res.size());
+    return CATTUS_B200_OK;
+}
+int cattus_b200_analysis_get(const cattus_b200_analysis_t* r, uint32_t k, cattus_b200_analysis_position* out) {
+    return r ? ds::analysis_get(r->res, k, out) : CATTUS_B200_EINVAL;
+}
+int cattus_b200_analysis_children(const cattus_b200_analysis_t* r, uint32_t k, uint16_t* moves, uint32_t* visits, float* w, float* priors,
+                                  uint32_t cap) {
+    return r ? ds::analysis_children(r->res, k, moves, visits, w, priors, cap) : CATTUS_B200_EINVAL;
+}
+int cattus_b200_analysis_pv(const cattus_b200_analysis_t* r, uint32_t k, uint16_t* pv, uint32_t cap) {
+    return r ? ds::analysis_pv(r->res, k, pv, cap) : CATTUS_B200_EINVAL;
+}
+void cattus_b200_analysis_free(cattus_b200_analysis_t* r) { delete r; }
+
 const char* cattus_b200_last_error(void) { return g_last_error.c_str(); }
 uint32_t cattus_b200_abi_version(void) { return CATTUS_B200_ABI_VERSION; }
 

@@ -1,0 +1,70 @@
+"""ctypes wrapper of tests/emul/libanalysis_emul.so (TEST INFRASTRUCTURE): the batched analysis driver over the host
+emulation of the device-resident search, with a Python evaluator callback."""
+from __future__ import annotations
+
+import ctypes as C
+import subprocess
+from pathlib import Path
+
+from cattus_b200 import _lib
+from cattus_b200.analysis import collect, encode_positions
+from cattus_b200.selfplay import SelfPlayRunner, _eval_thunk, parse_game
+
+HERE = Path(__file__).resolve().parent
+SO = HERE / "libanalysis_emul.so"
+SRC = HERE / "analysis_emul.cpp"
+CSRC = HERE.parent.parent / "cattus_b200" / "csrc"
+
+
+def build() -> Path:
+    deps = [SRC, HERE / "dsearch_emul.cpp"] + sorted(CSRC.glob("*.hpp")) + sorted((HERE.parent.parent / "include").glob("*.h"))
+    if SO.exists() and all(d.stat().st_mtime <= SO.stat().st_mtime for d in deps):
+        return SO
+    subprocess.run(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-ffp-contract=off", "-fno-strict-aliasing", "-o", str(SO), str(SRC)],
+                   check=True)
+    return SO
+
+
+_cached = None
+
+
+def load():
+    global _cached
+    if _cached is None:
+        lib = C.CDLL(str(build()))
+        lib.analysis_emul_run.restype = C.c_void_p
+        lib.analysis_emul_run.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_char_p), C.POINTER(C.c_uint16),
+                                          C.POINTER(C.c_uint32), C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]
+        lib.analysis_emul_error.restype = C.c_char_p
+        lib.analysis_emul_error.argtypes = [C.c_void_p]
+        lib.analysis_emul_count.argtypes = [C.c_void_p, C.POINTER(C.c_uint32)]
+        lib.analysis_emul_get.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(_lib.AnalysisPosition)]
+        lib.analysis_emul_children.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint16), C.POINTER(C.c_uint32), C.POINTER(C.c_float),
+                                               C.POINTER(C.c_float), C.c_uint32]
+        lib.analysis_emul_pv.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint16), C.c_uint32]
+        lib.analysis_emul_free.argtypes = [C.c_void_p]
+        _cached = lib
+    return _cached
+
+
+def analyse(game: str, positions, cfg: dict, eval_fn, *, n_slots: int, pool_words: int = 1 << 16, depth: int = 2, roots_cap: int = 0):
+    """-> [PositionAnalysis]; raises RuntimeError with the driver's message.  depth: dsearch_emul_run's knobs (waves in
+    flight | 256 begin overlapped | 512 two populations); roots_cap: history positions one wave uploads."""
+    lib = load()
+    c = SelfPlayRunner(game, cfg)._fill(2, None, None, False, 0, 1)
+    g, s = parse_game(game)
+    chess = g == _lib.GAME_CHESS
+    words = 18 if chess else 3 * ((s * s + 63) // 64)
+    errors: list = []
+    thunk = _eval_thunk(eval_fn, words, chess, errors)
+    n, fa, ma, oa = encode_positions(game, positions)
+    h = lib.analysis_emul_run(C.cast(thunk, C.c_void_p), C.byref(c), n, fa, ma, oa, n_slots, pool_words, depth, roots_cap)
+    try:
+        if errors:
+            raise errors[0]
+        err = lib.analysis_emul_error(h)
+        if err:
+            raise RuntimeError(err.decode())
+        return collect(lib.analysis_emul_count, lib.analysis_emul_get, lib.analysis_emul_children, lib.analysis_emul_pv, h)
+    finally:
+        lib.analysis_emul_free(h)
