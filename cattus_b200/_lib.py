@@ -92,6 +92,25 @@ class AnalysisPosition(C.Structure):
     ]
 
 
+class MatchSide(C.Structure):
+    """cattus_b200_match_side (include/cattus_b200_match.h)."""
+    _fields_ = [("struct_size", C.c_uint32), ("sim_num", C.c_uint32), ("explore_factor", C.c_float)]
+
+
+class MatchSummary(C.Structure):
+    """cattus_b200_match_summary (include/cattus_b200_match.h)."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("a_wins", C.c_uint32), ("b_wins", C.c_uint32), ("draws", C.c_uint32), ("games", C.c_uint32),
+        ("openings", C.c_uint32), ("skipped", C.c_uint32), ("pairs", C.c_uint32 * 5), ("simulations", C.c_uint64),
+        ("evaluations", C.c_uint64), ("seconds", C.c_double),
+    ]
+
+
+class MatchGame(C.Structure):
+    """cattus_b200_match_game (include/cattus_b200_match.h)."""
+    _fields_ = [(n, C.c_uint32) for n in ("struct_size", "opening", "a_is_player1", "winner", "termination", "n_moves")]
+
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 _H = C.c_void_p
 _u16p = C.POINTER(C.c_uint16)
@@ -137,6 +156,14 @@ SYMBOLS = {
     "cattus_b200_analysis_children": (C.c_int, [_H, C.c_uint32, _u16p, _u32p, _f32p, _f32p, C.c_uint32]),
     "cattus_b200_analysis_pv": (C.c_int, [_H, C.c_uint32, _u16p, C.c_uint32]),
     "cattus_b200_analysis_free": (None, [_H]),
+    # include/cattus_b200_match.h
+    "cattus_b200_match_run": (C.c_int, [_H, _H, C.POINTER(SelfPlayCfg), C.POINTER(MatchSide), C.c_uint32, C.POINTER(C.c_char_p), _u16p, _u32p,
+                                        C.POINTER(_H)]),
+    "cattus_b200_match_summary_get": (C.c_int, [_H, C.POINTER(MatchSummary)]),
+    "cattus_b200_match_opening_status": (C.c_int, [_H, C.c_uint32, _u32p]),
+    "cattus_b200_match_game_get": (C.c_int, [_H, C.c_uint32, C.POINTER(MatchGame)]),
+    "cattus_b200_match_game_moves": (C.c_int, [_H, C.c_uint32, _u16p, C.c_uint32]),
+    "cattus_b200_match_free": (None, [_H]),
     # include/cattus_b200_chess.h
     "cattus_b200_chess_position": (C.c_int, [C.c_char_p, _u16p, C.c_uint32, C.POINTER(ChessInfo)]),
     "cattus_b200_chess_perft": (C.c_int, [C.c_char_p, C.c_uint32, C.POINTER(C.c_uint64)]),

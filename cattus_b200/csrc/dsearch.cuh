@@ -12,6 +12,7 @@
 #include "dsearch_analysis.hpp"
 #include "dsearch_api.hpp"
 #include "dsearch_host.hpp"
+#include "dsearch_match.hpp"
 #include "engine.hpp"
 
 namespace cb2 {
@@ -62,16 +63,17 @@ struct DsPopulation {
     cudaEvent_t fork = nullptr, join = nullptr;
     cudaGraphExec_t graph = nullptr;
     void *d_cmds = nullptr, *d_status = nullptr, *d_cache_meta[2] = {nullptr, nullptr}, *d_cache_entries[2] = {nullptr, nullptr};
-    void* d_roots = nullptr;  // analysis: root histories of the population's current wave
+    void* d_roots = nullptr;  // root upload: root histories of the population's current wave
 };
 
 template <class Rules>
 class DsCudaBackend {
   public:
-    // `analysis` (optional) switches the finished searches to the analysis result layout and adds the per-wave root upload
-    // of kCmdSetRoot; without it everything is the self-play arrangement.
+    // `roots_cap` > 0 adds the per-wave root upload of kCmdSetRoot (analysis, matches from openings): up to that many
+    // history positions per wave.  `analysis` (optional) switches the finished searches to the analysis result layout.
+    // Without either everything is the self-play arrangement.
     DsCudaBackend(const void* rules_blob, size_t rules_bytes, uint32_t max_children, Engine* e1, Engine* e2, const cattus_b200_selfplay_cfg& cfg,
-                  const sp::Params params[2], uint32_t n_slots, const ds::AnalysisOpts* analysis = nullptr)
+                  const sp::Params params[2], uint32_t n_slots, uint32_t roots_cap = 0, const ds::AnalysisOpts* analysis = nullptr)
         : max_children_(max_children), n_slots_(n_slots) {
         eng_[0] = e1;
         eng_[1] = e2;
@@ -140,8 +142,8 @@ class DsCudaBackend {
             alloc(d_hist_, sizeof(typename Rules::Pos) * static_cast<size_t>(n_slots) * hist_cap);
             cmd_stride_ = ds::cmd_stride_for(max_children);
             result_stride_ = analysis ? ds::analysis_stride_for(max_children) : ds::result_stride_for(max_children);
-            if (analysis) {
-                roots_cap_ = analysis->roots_cap;
+            if (roots_cap) {
+                roots_cap_ = roots_cap;
                 CB2_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&h_roots_), sizeof(typename Rules::Pos) * roots_cap_ * n_bufs_, cudaHostAllocDefault));
             }
             cmd_bytes_ = 16 + static_cast<size_t>(n_slots) * cmd_stride_;
@@ -227,9 +229,11 @@ class DsCudaBackend {
                 // evaluator / expand; its slots take part from the population's next wave on
                 p.begin_lead = begin_lead;
                 p.visit_budget = visit_budget;
-                if (analysis) {
+                if (roots_cap_) {
                     alloc(P.d_roots, sizeof(typename Rules::Pos) * roots_cap_);
                     p.roots = static_cast<const typename Rules::Pos*>(P.d_roots);
+                }
+                if (analysis) {
                     p.analysis = 1;
                     p.pv_max = std::min<uint32_t>(analysis->pv_max, ds::kPvMax);
                 }
@@ -258,7 +262,7 @@ class DsCudaBackend {
     uint32_t population_of(uint32_t slot) const { return slot >= split_ ? 1u : 0u; }
     double setup_seconds() const { return setup_seconds_; }
     uint8_t* cmd_block(uint32_t wave) { return h_cmds_ + static_cast<size_t>(wave % n_bufs_) * cmd_bytes_; }
-    // analysis: where the host stages a wave's root histories (roots_cap() positions), uploaded by submit()
+    // root upload: where the host stages a wave's root histories (roots_cap() positions), uploaded by submit()
     typename Rules::Pos* roots_block(uint32_t wave) { return h_roots_ + static_cast<size_t>(wave % n_bufs_) * roots_cap_; }
     uint32_t roots_cap() const { return roots_cap_; }
 
@@ -441,9 +445,9 @@ static void analyse_rules(const Rules& rules, const void* blob, size_t blob_byte
         return;
     }
     // a wave's root upload: a few history positions per slot on average; a longer run of long histories waits a wave
-    const ds::AnalysisOpts opts{ds::kPvMax, n_slots * 8u + ds::hist_cap_for<Rules>()};
+    const ds::AnalysisOpts opts{ds::kPvMax};
     const auto t0 = std::chrono::steady_clock::now();
-    DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e, nullptr, cfg, params, n_slots, &opts);
+    DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e, nullptr, cfg, params, n_slots, n_slots * 8u + ds::hist_cap_for<Rules>(), &opts);
     ds::AnalysisDriver<Rules, DsCudaBackend<Rules>> drv(rules, params[0], be, hist, out);
     drv.run();
     const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
@@ -473,6 +477,74 @@ void analyse_run(cattus_b200_t* m, const cattus_b200_selfplay_cfg& cfg, uint32_t
         } else if (cfg.game == CATTUS_B200_GAME_TTT) {
             sp::TttRules rules;
             analyse_rules(rules, &rules, sizeof(rules), 9u, m->engine, cfg, n, fens, moves, move_offsets, out);
+        } else {
+            throw Error(CATTUS_B200_EINVAL, "unknown game");
+        }
+    } catch (const sp::SpError& e) {
+        throw Error(e.code ? e.code : CATTUS_B200_EINVAL, e.msg);
+    }
+}
+
+// A match from openings (dsearch_match.hpp) between e1 (A) and e2 (B; nullptr: the same handle): the self-play backend
+// and result layout with kCmdSetRoot's root upload.
+template <class Rules>
+static void match_rules(const Rules& rules, const void* blob, size_t blob_bytes, uint32_t max_children, Engine* e1, Engine* e2,
+                        const cattus_b200_selfplay_cfg& cfg, const cattus_b200_match_side* side_b, uint32_t n, const char* const* fens,
+                        const uint16_t* moves, const uint32_t* move_offsets, ds::MatchResult& out) {
+    const auto t0 = std::chrono::steady_clock::now();
+    sp::Params params[2];
+    ds::match_params(cfg, side_b, params);
+    uint32_t max_batch = 0xFFFFFFFFu;
+    for (Engine* e : {e1, e2}) {
+        if (!e) continue;
+        cattus_b200_info info;
+        e->get_info(&info);
+        if (info.game != cfg.game || (cfg.game == CATTUS_B200_GAME_HEX && info.board_size != cfg.board_size))
+            throw Error(CATTUS_B200_EINVAL, "match: a model was made for another game or board size than cfg");
+        if (cfg.device_games > info.max_batch)
+            throw Error(CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(cfg.device_games) + ") exceeds the evaluator's max_batch (" +
+                                                std::to_string(info.max_batch) + ")");
+        max_batch = std::min(max_batch, info.max_batch);
+    }
+    if (e2 && e2->device() != e1->device()) throw Error(CATTUS_B200_EINVAL, "match: both models must live on the same device");
+    const auto openings = ds::match_openings(rules, n, fens, moves, move_offsets, out.opening_status);
+    const uint32_t games = ds::match_games(out.opening_status);
+    if (games) {
+        const uint32_t n_slots = std::min(cfg.device_games ? cfg.device_games : max_batch, games);
+        // a wave's root upload: a few history positions per slot on average; a longer run of long histories waits a wave
+        DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e1, e2, cfg, params, n_slots, n_slots * 8u + ds::hist_cap_for<Rules>());
+        ds::match_play(rules, cfg, params, be, openings, out);
+        const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+        const uint64_t waves = be.waves();
+        e1->note_resident(waves, out.evaluations, waves * be.kernels_per_wave(), waves ? secs / static_cast<double>(waves) : 0.0);
+    }
+    out.seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+}
+
+void match_run(cattus_b200_t* ma, cattus_b200_t* mb, const cattus_b200_selfplay_cfg& cfg, const cattus_b200_match_side* side_b, uint32_t n,
+               const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, ds::MatchResult& out) {
+    try {
+        if (!ma) throw Error(CATTUS_B200_EINVAL, "null evaluator handle (there is no CPU fallback)");
+        if (cfg.struct_size != sizeof(cattus_b200_selfplay_cfg)) throw Error(CATTUS_B200_EINVAL, "selfplay cfg struct_size mismatch");
+        Engine* e1 = ma->engine;
+        Engine* e2 = (mb && mb != ma) ? mb->engine : nullptr;
+        if (cfg.game == CATTUS_B200_GAME_HEX) {
+            const int s = static_cast<int>(cfg.board_size);
+            if (s < 2 || s > 11) throw Error(CATTUS_B200_EINVAL, "hex board_size must be 2..11");
+            if (s <= 8) {
+                sp::HexRulesT<uint64_t> rules(s);
+                match_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, side_b, n, fens, moves, move_offsets, out);
+            } else {
+                sp::HexRulesT<sp::u128> rules(s);
+                match_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, side_b, n, fens, moves, move_offsets, out);
+            }
+        } else if (cfg.game == CATTUS_B200_GAME_CHESS) {
+            sp::ChessRules rules;
+            match_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), e1, e2, cfg, side_b, n,
+                        fens, moves, move_offsets, out);
+        } else if (cfg.game == CATTUS_B200_GAME_TTT) {
+            sp::TttRules rules;
+            match_rules(rules, &rules, sizeof(rules), 9u, e1, e2, cfg, side_b, n, fens, moves, move_offsets, out);
         } else {
             throw Error(CATTUS_B200_EINVAL, "unknown game");
         }

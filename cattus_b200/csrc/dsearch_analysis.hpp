@@ -8,8 +8,9 @@
 // MctsPlayer (engine/src/mcts/mod.rs:335-385) searches it with no root noise: no tree is kept between positions, so a
 // result depends neither on the number of slots, the waves in flight, the cache nor where the position falls in the input.
 //
-// `Backend` is the self-play transport (dsearch.cuh's DsCudaBackend, tests/emul's emulation) built with an AnalysisOpts,
-// plus roots_block(wave) / roots_cap(): where a wave's root histories are staged before submit() uploads them.
+// `Backend` is the self-play transport (dsearch.cuh's DsCudaBackend, tests/emul's emulation) built with the analysis
+// result layout and a root upload: roots_block(wave) / roots_cap() is where a wave's root histories are staged before
+// submit() uploads them.
 #pragma once
 
 #include <deque>
@@ -24,8 +25,7 @@
 namespace ds {
 
 struct AnalysisOpts {
-    uint32_t pv_max;     // principal variation plies (<= kPvMax)
-    uint32_t roots_cap;  // positions of root history one wave can carry
+    uint32_t pv_max;  // principal variation plies (<= kPvMax)
 };
 
 inline uint32_t analysis_stride_for(uint32_t max_children) {
@@ -78,14 +78,16 @@ inline sp::Params analysis_params(const cattus_b200_selfplay_cfg& cfg) {
 // Position k = fens[k] (NULL: the game's initial position; chess only otherwise) followed by moves[move_offsets[k],
 // move_offsets[k + 1]).  Returns each position's history as far as the search can need it: for chess the positions
 // since the last pawn move or capture (at most hist_cap_for), for the other games the position alone.  Every position
-// has its status settled.
+// has its status settled.  Errors name the input as `what` k ("position 3: ...").
 template <class Rules>
 std::vector<std::vector<typename Rules::Pos>> analysis_histories(const Rules& R, uint32_t n, const char* const* fens, const uint16_t* moves,
-                                                                 const uint32_t* move_offsets) {
+                                                                 const uint32_t* move_offsets, const char* what = "position") {
     using Pos = typename Rules::Pos;
     using Move = typename Rules::Move;
     std::vector<std::vector<Pos>> out(n);
-    const auto fail = [](uint32_t k, const std::string& what) { return sp::SpError{CATTUS_B200_EINVAL, "position " + std::to_string(k) + ": " + what}; };
+    const auto fail = [what](uint32_t k, const std::string& why) {
+        return sp::SpError{CATTUS_B200_EINVAL, std::string(what) + " " + std::to_string(k) + ": " + why};
+    };
     for (uint32_t k = 0; k < n; ++k) {
         const uint32_t m0 = move_offsets ? move_offsets[k] : 0u, m1 = move_offsets ? move_offsets[k + 1] : 0u;
         if (m1 < m0) throw fail(k, "move_offsets decrease");

@@ -10,9 +10,15 @@
 //
 // `Backend` is the transport: the CUDA one (dsearch.cuh) launches the captured wave graph and reads results from mapped
 // pinned memory; the one in tests/emul runs the same per-slot code on the host for the CPU parity tests.
+//
+// With an opening source (a match between two networks, dsearch_match.hpp) game 2k + c starts from opening k instead of
+// the initial position: a kCmdSetRoot command installs the opening with its history, which the backend uploads with the
+// wave (roots_block / roots_cap).  Everything else is the self-play game loop.
 #pragma once
 
 #include <deque>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "dsearch_core.hpp"
@@ -22,6 +28,12 @@ namespace ds {
 
 inline uint32_t cmd_stride_for(uint32_t max_children) { return (static_cast<uint32_t>(sizeof(Cmd)) + 4u * max_children + 15u) & ~15u; }
 inline uint32_t result_stride_for(uint32_t max_children) { return (static_cast<uint32_t>(sizeof(ResultHdr)) + 6u * max_children + 15u) & ~15u; }
+
+// whether a backend can upload root histories with a wave (kCmdSetRoot)
+template <class B, class = void>
+struct HasRootUpload : std::false_type {};
+template <class B>
+struct HasRootUpload<B, std::void_t<decltype(std::declval<B&>().roots_block(0u))>> : std::true_type {};
 
 template <class Rules, class Backend>
 class Driver {
@@ -34,6 +46,7 @@ class Driver {
         uint32_t game_idx = 0;
         sp::SplitMix64 rng;
         std::vector<Pos> history;
+        size_t hist_base = 0;  // positions of `history` before the game's first position (an opening's history)
         int cur = 0;
         sp::GameRecord rec;
         std::vector<std::pair<Pos, std::vector<std::pair<Move, float>>>> pending_entries;
@@ -44,8 +57,13 @@ class Driver {
     };
 
   public:
-    Driver(const Rules& rules, const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], Backend& be, sp::Shared& sh)
-        : R(rules), cfg_(cfg), be_(be), sh_(sh) {
+    // openings (optional): per opening k, the history kCmdSetRoot loads (oldest first, the opening's position last; at most
+    // the backend's history ring); games 2k and 2k + 1 start there.  An empty history: the opening is not played.
+    // cfg.games_num must be twice the number of openings.  Such games keep records (moves, winner, termination) but write
+    // no training data.
+    Driver(const Rules& rules, const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], Backend& be, sp::Shared& sh,
+           const std::vector<std::vector<Pos>>* openings = nullptr)
+        : R(rules), cfg_(cfg), be_(be), sh_(sh), openings_(openings) {
         params_[0] = params[0];
         params_[1] = params[1];
         games_.resize(be.n_slots());
@@ -70,14 +88,20 @@ class Driver {
             if (pops == 2 && active_pop_[pop] == 0 && cmds_[pop].empty()) pop ^= 1u;  // nothing to do there: give the turn away
             if (active_pop_[pop] > 0 || !cmds_[pop].empty()) {
                 uint8_t* block = be_.cmd_block(wave);
-                const uint32_t n_cmds = static_cast<uint32_t>(cmds_[pop].size() / cmd_stride_);
+                uint32_t n_cmds = static_cast<uint32_t>(cmds_[pop].size() / cmd_stride_);
                 uint32_t* hdr = reinterpret_cast<uint32_t*>(block);
+                if (n_cmds) std::memcpy(block + 16, cmds_[pop].data(), cmds_[pop].size());
+                cmds_[pop].clear();
+                uint32_t n_roots = 0;
+                if constexpr (HasRootUpload<Backend>::value)
+                    n_cmds += stage_roots(pop, wave, block + 16 + static_cast<size_t>(n_cmds) * cmd_stride_, &n_roots);
                 hdr[0] = n_cmds;
                 hdr[1] = wave;
                 hdr[2] = hdr[3] = 0;
-                if (n_cmds) std::memcpy(block + 16, cmds_[pop].data(), cmds_[pop].size());
-                cmds_[pop].clear();
-                be_.submit(wave, pop, n_cmds);
+                if constexpr (HasRootUpload<Backend>::value)
+                    be_.submit(wave, pop, n_cmds, n_roots);
+                else
+                    be_.submit(wave, pop, n_cmds);
                 inflight.push_back(wave++);
                 submitted = true;
                 waves_ += 1;
@@ -122,21 +146,57 @@ class Driver {
     void start_next_game(uint32_t slot) {
         Game& g = games_[slot];
         const uint32_t stride = std::max<uint32_t>(1, cfg_.game_stride);
-        const uint32_t k = sh_.next_game.fetch_add(1);
-        const uint64_t idx = static_cast<uint64_t>(cfg_.first_game) + static_cast<uint64_t>(k) * stride;
-        if (idx >= cfg_.games_num) {
-            g.active = false;
-            return;
-        }
+        uint64_t idx;
+        do {
+            const uint32_t k = sh_.next_game.fetch_add(1);
+            idx = static_cast<uint64_t>(cfg_.first_game) + static_cast<uint64_t>(k) * stride;
+            if (idx >= cfg_.games_num) {
+                g.active = false;
+                return;
+            }
+        } while (openings_ && (*openings_)[idx / 2].empty());
         g = Game();
         g.active = true;
         g.game_idx = static_cast<uint32_t>(idx);
         g.rng = sp::SplitMix64(sp::game_seed(cfg_.seed, g.game_idx));
-        g.history.push_back(R.initial());
         g.rec.game_idx = g.game_idx;
         active_ += 1;
         active_pop_[be_.population_of(slot)] += 1;
-        begin_move(slot, kCmdNewGame, 0);
+        if (openings_) {
+            const std::vector<Pos>& h = (*openings_)[idx / 2];
+            g.history = h;
+            g.hist_base = h.size() - 1;
+            begin_move(slot, kCmdSetRoot, 0);
+        } else {
+            g.history.push_back(R.initial());
+            begin_move(slot, kCmdNewGame, 0);
+        }
+    }
+
+    // Moves the population's waiting kCmdSetRoot commands into the wave's command block at `at` while their histories fit
+    // the wave's root block; the rest wait for a later wave (their slots stay idle on the device until then).
+    uint32_t stage_roots(uint32_t pop, uint32_t wave, uint8_t* at, uint32_t* n_roots) {
+        std::vector<uint8_t>& wait = set_root_[pop];
+        Pos* roots = be_.roots_block(wave);
+        const uint32_t cap = be_.roots_cap();
+        uint32_t staged = 0, n = 0;
+        size_t off = 0;
+        for (; off < wait.size(); off += cmd_stride_, ++n) {
+            Cmd c;
+            std::memcpy(&c, wait.data() + off, sizeof(c));
+            const std::vector<Pos>& h = games_[c.slot].history;
+            const uint32_t len = static_cast<uint32_t>(h.size());
+            if (staged + len > cap) break;
+            std::copy(h.begin(), h.end(), roots + staged);
+            c.root_at = staged;
+            c.root_len = len;
+            std::memcpy(at + off, wait.data() + off, cmd_stride_);
+            std::memcpy(at + off, &c, sizeof(c));
+            staged += len;
+        }
+        wait.erase(wait.begin(), wait.begin() + static_cast<std::ptrdiff_t>(off));
+        *n_roots = staged;
+        return n;
     }
 
     // One step of the game loop at a position that is about to be searched (or ends the game).
@@ -151,7 +211,11 @@ class Driver {
             n_legal = R.status(pos) != 0 ? 0 : sp::popcount128(R.legal_mask(pos));
         }
         int st = g.repetition ? 3 : R.status(pos);  // ChessGame::status: a threefold repetition is a draw
-        if (st == 0 && cfg_.max_moves && g.rec.moves.size() >= cfg_.max_moves) st = 3;  // bounded runs only (not in the reference)
+        g.rec.termination = g.repetition ? sp::kEndRepetition : sp::kEndRules;
+        if (st == 0 && cfg_.max_moves && g.rec.moves.size() >= cfg_.max_moves) {  // bounded runs only (not in the reference)
+            st = 3;
+            g.rec.termination = sp::kEndMaxMoves;
+        }
         if (st != 0) {
             finish_game(g, st);
             active_ -= 1;
@@ -175,7 +239,8 @@ class Driver {
             for (uint32_t i = 0; i < noise_n; ++i) nz_[i] = static_cast<float>(noise_[i] / tot);
         }
         g.search_t0 = sp::Clock::now();
-        std::vector<uint8_t>& cmds = cmds_[be_.population_of(slot)];
+        // kCmdSetRoot waits in its own queue: its history goes with whichever wave has room for it (stage_roots)
+        std::vector<uint8_t>& cmds = (flags == kCmdSetRoot ? set_root_ : cmds_)[be_.population_of(slot)];
         const size_t at = cmds.size();
         cmds.resize(at + cmd_stride_, 0);
         Cmd c;
@@ -210,7 +275,8 @@ class Driver {
         search_duration_ = (1.0 - 0.99) * search_duration_ + 0.99 * secs;  // RunningAverage(0.99), util/metric.rs:1-20
         searches_ += 1;
         if (probs.empty()) throw sp::SpError{CATTUS_B200_EINVAL, "search produced no moves"};
-        const int chosen = sp::choose_move(P, g.history.size(), probs, g.rng, weights_);
+        // the temperature policy counts moves from the game's first position (an opening's history does not count)
+        const int chosen = sp::choose_move(P, g.history.size() - g.hist_base, probs, g.rng, weights_);
         const Move mv = probs[chosen].first;
         g.last_root[g.cur] = g.history.back();
         g.has_last_root[g.cur] = true;
@@ -237,7 +303,7 @@ class Driver {
     void finish_game(Game& g, int status) {
         const uint8_t winner = status == 3 ? 0 : static_cast<uint8_t>(status);
         g.rec.winner = winner;
-        for (size_t pos_idx = 0; pos_idx < g.pending_entries.size(); ++pos_idx) {
+        for (size_t pos_idx = 0; !openings_ && pos_idx < g.pending_entries.size(); ++pos_idx) {
             auto& pe = g.pending_entries[pos_idx];
             std::vector<uint8_t> bytes;
             const int dir = sp::make_entry(R, g.game_idx, pe.first, pe.second, winner, bytes);
@@ -257,7 +323,7 @@ class Driver {
         else
             w2_ += 1;
         games_done_ += 1;
-        if (cfg_.keep_records) {
+        if (cfg_.keep_records || openings_) {
             std::lock_guard<std::mutex> lk(sh_.mu);
             sh_.records.push_back(std::move(g.rec));
         }
@@ -269,8 +335,10 @@ class Driver {
     Backend& be_;
     sp::Shared& sh_;
     sp::Params params_[2];
+    const std::vector<std::vector<Pos>>* openings_;
     std::vector<Game> games_;
-    std::vector<uint8_t> cmds_[2];  // commands for each population's next wave
+    std::vector<uint8_t> cmds_[2];      // commands for each population's next wave
+    std::vector<uint8_t> set_root_[2];  // kCmdSetRoot commands waiting for room in a wave's root block
     uint32_t cmd_stride_ = 0, result_stride_ = 0;
     uint32_t active_ = 0, active_pop_[2] = {0, 0};
     uint64_t waves_ = 0, searches_ = 0;

@@ -2243,6 +2243,36 @@ int cattus_b200_analysis_pv(const cattus_b200_analysis_t* r, uint32_t k, uint16_
 }
 void cattus_b200_analysis_free(cattus_b200_analysis_t* r) { delete r; }
 
+// ---------------------------------------------------------------- match play from openings (include/cattus_b200_match.h)
+struct cattus_b200_match {
+    ds::MatchResult res;
+};
+
+int cattus_b200_match_run(cattus_b200_t* model_a, cattus_b200_t* model_b, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_match_side* side_b,
+                          uint32_t n, const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, cattus_b200_match_t** out) {
+    return guarded([&] {
+        if (!cfg || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        *out = nullptr;
+        std::unique_ptr<cattus_b200_match> r(new cattus_b200_match());
+        cb2::match_run(model_a, model_b, *cfg, side_b, n, fens, moves, move_offsets, r->res);
+        *out = r.release();
+    });
+}
+
+int cattus_b200_match_summary_get(const cattus_b200_match_t* r, cattus_b200_match_summary* out) {
+    return r ? ds::match_summary(r->res, out) : CATTUS_B200_EINVAL;
+}
+int cattus_b200_match_opening_status(const cattus_b200_match_t* r, uint32_t k, uint32_t* status) {
+    return r ? ds::match_opening_status(r->res, k, status) : CATTUS_B200_EINVAL;
+}
+int cattus_b200_match_game_get(const cattus_b200_match_t* r, uint32_t k, cattus_b200_match_game* out) {
+    return r ? ds::match_game(r->res, k, out) : CATTUS_B200_EINVAL;
+}
+int cattus_b200_match_game_moves(const cattus_b200_match_t* r, uint32_t k, uint16_t* moves, uint32_t cap) {
+    return r ? ds::match_game_moves(r->res, k, moves, cap) : CATTUS_B200_EINVAL;
+}
+void cattus_b200_match_free(cattus_b200_match_t* r) { delete r; }
+
 const char* cattus_b200_last_error(void) { return g_last_error.c_str(); }
 uint32_t cattus_b200_abi_version(void) { return CATTUS_B200_ABI_VERSION; }
 

@@ -1328,30 +1328,6 @@ static void run_games(const Rules& rules, const cattus_b200_selfplay_cfg& cfg, c
     workers[0]->run();  // the calling thread does job 0 (self_play.rs:127-137); run() itself never throws
 }
 
-// MctsParams from the config (mcts/mod.rs:72-110; TemperaturePolicy::scheduled, self_play_cmd.rs:68-72)
-static sp::Params parse_params(const cattus_b200_selfplay_cfg* cfg) {
-    if (cfg->sim_num < 2) throw sp::SpError{CATTUS_B200_EINVAL, "sim_num must be > 1 (mcts/mod.rs:157)"};
-    if (!(cfg->explore_factor >= 0.0f) || !(cfg->prior_noise_alpha >= 0.0f) || !(cfg->prior_noise_epsilon >= 0.0f && cfg->prior_noise_epsilon <= 1.0f))
-        throw sp::SpError{CATTUS_B200_EINVAL, "bad mcts parameters (mcts/mod.rs:107-110)"};
-    sp::Params p;
-    p.sim_num = cfg->sim_num;
-    p.explore_factor = cfg->explore_factor;
-    p.noise_alpha = cfg->prior_noise_alpha;
-    p.noise_eps = cfg->prior_noise_epsilon;
-    p.last_temperature = 1.0f;
-    if (cfg->n_temperatures) {
-        if (!cfg->temperature_moves || !cfg->temperature_values) throw sp::SpError{CATTUS_B200_EINVAL, "temperature arrays are NULL"};
-        for (uint32_t i = 0; i + 1 < cfg->n_temperatures; ++i) {
-            if (!(cfg->temperature_values[i] >= 0.0f)) throw sp::SpError{CATTUS_B200_EINVAL, "negative temperature"};
-            if (i > 0 && cfg->temperature_moves[i] <= cfg->temperature_moves[i - 1]) throw sp::SpError{CATTUS_B200_EINVAL, "temperature thresholds must be strictly increasing"};
-            p.temperatures.emplace_back(cfg->temperature_moves[i], cfg->temperature_values[i]);
-        }
-        p.last_temperature = cfg->temperature_values[cfg->n_temperatures - 1];
-        if (!(p.last_temperature >= 0.0f)) throw sp::SpError{CATTUS_B200_EINVAL, "negative temperature"};
-    }
-    return p;
-}
-
 static int selfplay_impl(sp::Evaluator& e1, sp::Evaluator* e2_or_null, const cattus_b200_selfplay_cfg* cfg, cattus_b200_selfplay_t** out) {
     try {
         if (!cfg || !out) throw sp::SpError{CATTUS_B200_EINVAL, "null argument"};
@@ -1359,7 +1335,7 @@ static int selfplay_impl(sp::Evaluator& e1, sp::Evaluator* e2_or_null, const cat
         *out = nullptr;
         if (cfg->games_num % 2 != 0) throw sp::SpError{CATTUS_B200_EINVAL, "Games num should be a multiple of 2 (self_play.rs:100)"};
         if ((cfg->out_dir1 == nullptr) != (cfg->out_dir2 == nullptr)) throw sp::SpError{CATTUS_B200_EINVAL, "out_dir1 and out_dir2 must both be set or both NULL"};
-        const sp::Params p = parse_params(cfg);
+        const sp::Params p = sp::parse_params(cfg);
         sp::Params params[2] = {p, p};
         if (cfg->game == CATTUS_B200_GAME_HEX) {
             if (cfg->board_size < 2 || cfg->board_size > 11) throw sp::SpError{CATTUS_B200_EINVAL, "hex board_size must be 2..11"};
@@ -1556,7 +1532,7 @@ static int chess_search_create_impl(cattus_b200_eval_fn fn, void* ctx, cattus_b2
         if (cfg->struct_size != sizeof(cattus_b200_selfplay_cfg)) throw sp::SpError{CATTUS_B200_EINVAL, "selfplay cfg struct_size mismatch"};
         *out = nullptr;
         std::unique_ptr<cattus_b200_chess_search> s(new cattus_b200_chess_search());
-        s->params[0] = s->params[1] = parse_params(cfg);
+        s->params[0] = s->params[1] = sp::parse_params(cfg);
         s->cfg = *cfg;
         s->cfg.game = CATTUS_B200_GAME_CHESS;
         s->cfg.board_size = 8;

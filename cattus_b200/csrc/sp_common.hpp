@@ -83,9 +83,37 @@ struct Params {
     }
 };
 
+// MctsParams from the config (mcts/mod.rs:72-110; TemperaturePolicy::scheduled, self_play_cmd.rs:68-72)
+inline Params parse_params(const cattus_b200_selfplay_cfg* cfg) {
+    if (cfg->sim_num < 2) throw SpError{CATTUS_B200_EINVAL, "sim_num must be > 1 (mcts/mod.rs:157)"};
+    if (!(cfg->explore_factor >= 0.0f) || !(cfg->prior_noise_alpha >= 0.0f) || !(cfg->prior_noise_epsilon >= 0.0f && cfg->prior_noise_epsilon <= 1.0f))
+        throw SpError{CATTUS_B200_EINVAL, "bad mcts parameters (mcts/mod.rs:107-110)"};
+    Params p;
+    p.sim_num = cfg->sim_num;
+    p.explore_factor = cfg->explore_factor;
+    p.noise_alpha = cfg->prior_noise_alpha;
+    p.noise_eps = cfg->prior_noise_epsilon;
+    p.last_temperature = 1.0f;
+    if (cfg->n_temperatures) {
+        if (!cfg->temperature_moves || !cfg->temperature_values) throw SpError{CATTUS_B200_EINVAL, "temperature arrays are NULL"};
+        for (uint32_t i = 0; i + 1 < cfg->n_temperatures; ++i) {
+            if (!(cfg->temperature_values[i] >= 0.0f)) throw SpError{CATTUS_B200_EINVAL, "negative temperature"};
+            if (i > 0 && cfg->temperature_moves[i] <= cfg->temperature_moves[i - 1]) throw SpError{CATTUS_B200_EINVAL, "temperature thresholds must be strictly increasing"};
+            p.temperatures.emplace_back(cfg->temperature_moves[i], cfg->temperature_values[i]);
+        }
+        p.last_temperature = cfg->temperature_values[cfg->n_temperatures - 1];
+        if (!(p.last_temperature >= 0.0f)) throw SpError{CATTUS_B200_EINVAL, "negative temperature"};
+    }
+    return p;
+}
+
+// How a game of the device-resident driver ended (GameRecord::termination; the host driver leaves it 0)
+enum Termination : uint8_t { kEndRules = 1, kEndRepetition = 2, kEndMaxMoves = 3 };
+
 struct GameRecord {
     uint32_t game_idx = 0;
     uint8_t winner = 0;
+    uint8_t termination = 0;  // Termination
     std::vector<uint16_t> moves;  // hex / ttt: cell index; chess: from | to << 6 | promotion << 12, real board coordinates
     std::vector<std::vector<uint8_t>> entries;
     std::vector<uint8_t> entry_dir;

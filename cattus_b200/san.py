@@ -168,6 +168,52 @@ def _split_ops(s: str) -> List[str]:
     return out
 
 
+_RESULTS = {None: "1/2-1/2", 0: "1/2-1/2", 1: "1-0", 2: "0-1"}
+# PGN's Termination tag has a fixed vocabulary: a game the rules or a repetition ended is "normal", one cut off at
+# max_moves is "adjudication"; a comment after the last move says which
+_TERMINATION_TAG = {"rules": "normal", "repetition": "normal", "max_moves": "adjudication"}
+_TERMINATION_TEXT = {"rules": None, "repetition": "threefold repetition", "max_moves": "draw adjudicated at max_moves"}
+
+
+def pgn_game(fen: Optional[str], opening: Sequence[int], moves: Sequence[int], winner: Optional[int], termination: str, *, white: str = "?",
+             black: str = "?", event: str = "?", round_: str = "?") -> str:
+    """One game in PGN: the Seven Tag Roster, SetUp / FEN for a FEN opening and Termination; the movetext holds the
+    opening's moves, then the game's, numbered from the FEN's fullmove field (1 without one), and ends with the result.
+    winner: None / 0 draw, 1 white, 2 black."""
+    result = _RESULTS[winner]
+    tags = [("Event", event), ("Site", "?"), ("Date", "????.??.??"), ("Round", round_), ("White", white), ("Black", black), ("Result", result)]
+    if fen is not None:
+        tags += [("SetUp", "1"), ("FEN", fen)]
+    tags.append(("Termination", _TERMINATION_TAG[termination]))
+    fields = (fen or START_FEN).split()
+    number = int(fields[5]) if len(fields) > 5 else 1
+    black_to_move = fields[1] == "b"
+    toks, played = [], []
+    for k, m in enumerate(list(opening) + list(moves)):
+        if not black_to_move:
+            toks.append(f"{number}.")
+        elif k == 0:
+            toks.append(f"{number}...")
+        toks.append(move_to_san(fen, played, m))
+        played.append(m)
+        if black_to_move:
+            number += 1
+        black_to_move = not black_to_move
+    note = _TERMINATION_TEXT[termination]
+    if note:
+        toks.append("{" + note + "}")
+    toks.append(result)
+    lines, cur = [], ""
+    for t in toks:  # PGN export format: lines of at most 80 characters
+        if cur and len(cur) + 1 + len(t) > 79:
+            lines.append(cur)
+            cur = t
+        else:
+            cur = f"{cur} {t}" if cur else t
+    lines.append(cur)
+    return "".join(f'[{k} "{v}"]\n' for k, v in tags) + "\n" + "\n".join(lines) + "\n"
+
+
 def parse_fen_line(line: str) -> Tuple[Optional[str], List[str]]:
     """`<FEN> [moves m1 m2 ...]` or `startpos [moves ...]` -> (fen or None, LAN moves)."""
     head, _, tail = line.strip().partition(" moves")
