@@ -92,6 +92,11 @@ class AnalysisPosition(C.Structure):
     ]
 
 
+class AnalysisOpts(C.Structure):
+    """cattus_b200_analysis_opts (include/cattus_b200_analysis.h)."""
+    _fields_ = [("struct_size", C.c_uint32), ("search_batch", C.c_uint32)]
+
+
 class MatchSide(C.Structure):
     """cattus_b200_match_side (include/cattus_b200_match.h)."""
     _fields_ = [("struct_size", C.c_uint32), ("sim_num", C.c_uint32), ("explore_factor", C.c_float)]
@@ -155,6 +160,9 @@ SYMBOLS = {
     "cattus_b200_analysis_get": (C.c_int, [_H, C.c_uint32, C.POINTER(AnalysisPosition)]),
     "cattus_b200_analysis_children": (C.c_int, [_H, C.c_uint32, _u16p, _u32p, _f32p, _f32p, C.c_uint32]),
     "cattus_b200_analysis_pv": (C.c_int, [_H, C.c_uint32, _u16p, C.c_uint32]),
+    "cattus_b200_analyse_opts": (C.c_int, [_H, C.POINTER(SelfPlayCfg), C.POINTER(AnalysisOpts), C.c_uint32, C.POINTER(C.c_char_p), _u16p, _u32p,
+                                           C.POINTER(_H)]),
+    "cattus_b200_analysis_batches": (C.c_int, [_H, C.c_uint32, _u32p, _u32p]),
     "cattus_b200_analysis_free": (None, [_H]),
     # include/cattus_b200_match.h
     "cattus_b200_match_run": (C.c_int, [_H, _H, C.POINTER(SelfPlayCfg), C.POINTER(MatchSide), C.c_uint32, C.POINTER(C.c_char_p), _u16p, _u32p,

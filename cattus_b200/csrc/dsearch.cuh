@@ -52,6 +52,26 @@ __global__ void __launch_bounds__(128, DS_EXPAND_MIN_BLOCKS) ds_expand_kernel(ds
     ds::Core<Rules>::expand_slot(R, p, warp, wave);
 }
 
+// Minibatched analysis (search_batch > 1, DESIGN.md section 15): one warp per searched tree, captured in a wave graph of
+// their own instead of select / expand.
+template <class Rules>
+__global__ void __launch_bounds__(128) ds_select_batch_kernel(ds::Params<Rules> p) {
+    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (warp >= p.n_slots) return;
+    const uint32_t wave = reinterpret_cast<const uint32_t*>(p.cmds)[1];
+    decltype(auto) R = ds::RulesRef<Rules>::get(p.rules);
+    ds::Core<Rules>::batch_select_slot(R, p, warp, wave);
+}
+
+template <class Rules>
+__global__ void __launch_bounds__(128) ds_expand_batch_kernel(ds::Params<Rules> p) {
+    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (warp >= p.n_slots) return;
+    const uint32_t wave = reinterpret_cast<const uint32_t*>(p.cmds)[1];
+    decltype(auto) R = ds::RulesRef<Rules>::get(p.rules);
+    ds::Core<Rules>::batch_expand_slot(R, p, warp, wave);
+}
+
 // One population of slots: its kernel parameters, streams, captured wave graph, command and status blocks, evaluator lanes
 // and evaluation caches.  Two populations alternate waves on two streams (dsearch_host.hpp), so that one population's
 // select / expand kernels run beside the other's evaluator kernels.
@@ -74,7 +94,7 @@ class DsCudaBackend {
     // Without either everything is the self-play arrangement.
     DsCudaBackend(const void* rules_blob, size_t rules_bytes, uint32_t max_children, Engine* e1, Engine* e2, const cattus_b200_selfplay_cfg& cfg,
                   const sp::Params params[2], uint32_t n_slots, uint32_t roots_cap = 0, const ds::AnalysisOpts* analysis = nullptr)
-        : max_children_(max_children), n_slots_(n_slots) {
+        : max_children_(max_children), n_slots_(n_slots), search_batch_(analysis ? std::max<uint32_t>(1, analysis->search_batch) : 1u) {
         eng_[0] = e1;
         eng_[1] = e2;
         n_evals_ = e2 ? 2 : 1;
@@ -88,6 +108,10 @@ class DsCudaBackend {
             // evaluator lanes: one per population and evaluator; a second population needs a second free stream in every evaluator
             for (uint32_t e = 0; e < n_evals_; ++e) {
                 pop_[0].io[e] = eng_[e]->resident_acquire(true);
+                if (search_batch_ > 1 && pop_[0].io[e].max_batch < static_cast<uint64_t>(n_slots) * search_batch_)
+                    throw Error(CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(n_slots) + ") x search_batch (" +
+                                                        std::to_string(search_batch_) + ") exceeds the evaluator's max_batch (" +
+                                                        std::to_string(pop_[0].io[e].max_batch) + ")");
                 if (pop_[0].io[e].max_batch < n_slots)
                     throw Error(CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(n_slots) + ") exceeds the evaluator's max_batch (" +
                                                         std::to_string(pop_[0].io[e].max_batch) + ")");
@@ -98,7 +122,7 @@ class DsCudaBackend {
             // kernels leave no room for the other population's select / expand blocks to run beside them, and half-size batches
             // are less efficient (hex5 64.1 M vs 64.4 M sims/s, hex7 30.0 M vs 37.1 M, chess 10x128 4.7 M vs 5.0 M).  Kept as an
             // experiment knob; the games are the same either way (tests/test_gpu_dsearch.py).
-            if (n_slots >= 64 && depth_ >= 2 && std::getenv("CATTUS_B200_DSEARCH_TWO_POPULATIONS")) {
+            if (n_slots >= 64 && depth_ >= 2 && search_batch_ == 1 && std::getenv("CATTUS_B200_DSEARCH_TWO_POPULATIONS")) {
                 bool ok = true;
                 for (uint32_t e = 0; e < n_evals_; ++e) {
                     pop_[1].io[e] = eng_[e]->resident_acquire(false);
@@ -141,7 +165,13 @@ class DsCudaBackend {
             const uint32_t hist_cap = Rules::kChess ? 128u : 1u;
             alloc(d_hist_, sizeof(typename Rules::Pos) * static_cast<size_t>(n_slots) * hist_cap);
             cmd_stride_ = ds::cmd_stride_for(max_children);
-            result_stride_ = analysis ? ds::analysis_stride_for(max_children) : ds::result_stride_for(max_children);
+            result_stride_ = analysis ? ds::analysis_stride_for(max_children, search_batch_) : ds::result_stride_for(max_children);
+            if (search_batch_ > 1) {  // per-descent records and paths, and a virtual count per child row of each slot's tree
+                alloc(d_descents_, sizeof(ds::BatchDescent) * static_cast<size_t>(n_slots) * search_batch_);
+                alloc(d_bpaths_, sizeof(ds::PathStep) * static_cast<size_t>(n_slots) * search_batch_ * path_cap);
+                alloc(d_vcount_, sizeof(uint32_t) * static_cast<size_t>(n_slots) * (pool_words_ >> 2));
+                CB2_CUDA(cudaMemset(d_vcount_, 0, sizeof(uint32_t) * static_cast<size_t>(n_slots) * (pool_words_ >> 2)));
+            }
             if (roots_cap) {
                 roots_cap_ = roots_cap;
                 CB2_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&h_roots_), sizeof(typename Rules::Pos) * roots_cap_ * n_bufs_, cudaHostAllocDefault));
@@ -236,6 +266,12 @@ class DsCudaBackend {
                 if (analysis) {
                     p.analysis = 1;
                     p.pv_max = std::min<uint32_t>(analysis->pv_max, ds::kPvMax);
+                }
+                if (search_batch_ > 1) {
+                    p.search_batch = search_batch_;
+                    p.descents = static_cast<ds::BatchDescent*>(d_descents_) + static_cast<size_t>(base) * search_batch_;
+                    p.bpaths = static_cast<ds::PathStep*>(d_bpaths_) + static_cast<size_t>(base) * search_batch_ * path_cap;
+                    p.vcount = static_cast<uint32_t*>(d_vcount_) + static_cast<size_t>(base) * (pool_words_ >> 2);
                 }
                 if (begin_lead) {
                     CB2_CUDA(cudaStreamCreateWithFlags(&P.side, cudaStreamNonBlocking));
@@ -333,9 +369,15 @@ class DsCudaBackend {
             } else {
                 ds_begin_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             }
-            ds_select_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
+            if (P.p.search_batch > 1)
+                ds_select_batch_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
+            else
+                ds_select_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             for (uint32_t e = 0; e < n_evals_; ++e) eng_[e]->resident_enqueue(P.io[e].lane, P.stream);
-            ds_expand_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
+            if (P.p.search_batch > 1)
+                ds_expand_batch_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
+            else
+                ds_expand_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             if (P.p.begin_lead) CB2_CUDA(cudaStreamWaitEvent(P.stream, P.join, 0));
             CB2_CUDA(cudaGetLastError());
         } catch (...) {
@@ -375,7 +417,7 @@ class DsCudaBackend {
         for (auto& ev : events_)
             if (ev) cudaEventDestroy(ev);
         events_.clear();
-        for (void** q : {&d_rules_, &d_slots_, &d_pools_, &d_paths_, &d_noise_, &d_hist_}) {
+        for (void** q : {&d_rules_, &d_slots_, &d_pools_, &d_paths_, &d_noise_, &d_hist_, &d_descents_, &d_bpaths_, &d_vcount_}) {
             if (*q) cudaFree(*q);
             *q = nullptr;
         }
@@ -390,9 +432,10 @@ class DsCudaBackend {
     DsPopulation<Rules> pop_[2];
     Engine* eng_[2] = {nullptr, nullptr};
     uint32_t n_evals_ = 1, n_pops_ = 1, split_ = 0, depth_ = 2, n_bufs_ = 3, max_children_ = 0, n_slots_ = 0, pool_words_ = 0, cmd_stride_ = 0,
-             result_stride_ = 0, kernels_per_wave_ = 0, roots_cap_ = 0;
+             result_stride_ = 0, kernels_per_wave_ = 0, roots_cap_ = 0, search_batch_ = 1;
     size_t cmd_bytes_ = 0, result_buf_bytes_ = 0;
     void *d_rules_ = nullptr, *d_slots_ = nullptr, *d_pools_ = nullptr, *d_paths_ = nullptr, *d_noise_ = nullptr, *d_hist_ = nullptr;
+    void *d_descents_ = nullptr, *d_bpaths_ = nullptr, *d_vcount_ = nullptr;
     uint8_t *h_results_ = nullptr, *h_cmds_ = nullptr, *h_status_ = nullptr;
     typename Rules::Pos* h_roots_ = nullptr;
     std::vector<cudaEvent_t> events_;
@@ -428,34 +471,30 @@ static void dsearch_run_rules(const Rules& rules, const void* blob, size_t blob_
 // result layout and kCmdSetRoot's root upload.
 template <class Rules>
 static void analyse_rules(const Rules& rules, const void* blob, size_t blob_bytes, uint32_t max_children, Engine* e, const cattus_b200_selfplay_cfg& cfg,
-                          uint32_t n, const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, std::vector<ds::AnalysisResult>& out) {
+                          uint32_t search_batch, uint32_t n, const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, std::vector<ds::AnalysisResult>& out) {
     const sp::Params params[2] = {ds::analysis_params(cfg), ds::analysis_params(cfg)};
     const auto hist = ds::analysis_histories(rules, n, fens, moves, move_offsets);
     cattus_b200_info info;
     e->get_info(&info);
     if (info.game != cfg.game || (cfg.game == CATTUS_B200_GAME_HEX && info.board_size != cfg.board_size))
         throw Error(CATTUS_B200_EINVAL, "analysis: the model was made for another game or board size than cfg");
-    if (cfg.device_games > info.max_batch)
-        throw Error(CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(cfg.device_games) + ") exceeds the evaluator's max_batch (" +
-                                            std::to_string(info.max_batch) + ")");
-    const uint32_t want = cfg.device_games ? cfg.device_games : info.max_batch;
-    const uint32_t n_slots = std::max<uint32_t>(1, std::min<uint32_t>(want, n));
+    const uint32_t n_slots = ds::analysis_slots(cfg.device_games, n, info.max_batch, search_batch);
     if (n == 0) {
         out.clear();
         return;
     }
     // a wave's root upload: a few history positions per slot on average; a longer run of long histories waits a wave
-    const ds::AnalysisOpts opts{ds::kPvMax};
+    const ds::AnalysisOpts opts{ds::kPvMax, search_batch};
     const auto t0 = std::chrono::steady_clock::now();
     DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e, nullptr, cfg, params, n_slots, n_slots * 8u + ds::hist_cap_for<Rules>(), &opts);
-    ds::AnalysisDriver<Rules, DsCudaBackend<Rules>> drv(rules, params[0], be, hist, out);
+    ds::AnalysisDriver<Rules, DsCudaBackend<Rules>> drv(rules, params[0], be, hist, out, search_batch);
     drv.run();
     const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     const uint64_t waves = be.waves();
     e->note_resident(waves, drv.counters()[1], waves * be.kernels_per_wave(), waves ? secs / static_cast<double>(waves) : 0.0);
 }
 
-void analyse_run(cattus_b200_t* m, const cattus_b200_selfplay_cfg& cfg, uint32_t n, const char* const* fens, const uint16_t* moves,
+void analyse_run(cattus_b200_t* m, const cattus_b200_selfplay_cfg& cfg, uint32_t search_batch, uint32_t n, const char* const* fens, const uint16_t* moves,
                  const uint32_t* move_offsets, std::vector<ds::AnalysisResult>& out) {
     try {
         if (!m) throw Error(CATTUS_B200_EINVAL, "null evaluator handle (there is no CPU fallback)");
@@ -465,18 +504,18 @@ void analyse_run(cattus_b200_t* m, const cattus_b200_selfplay_cfg& cfg, uint32_t
             if (s < 2 || s > 11) throw Error(CATTUS_B200_EINVAL, "hex board_size must be 2..11");
             if (s <= 8) {
                 sp::HexRulesT<uint64_t> rules(s);
-                analyse_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, n, fens, moves, move_offsets, out);
+                analyse_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, search_batch, n, fens, moves, move_offsets, out);
             } else {
                 sp::HexRulesT<sp::u128> rules(s);
-                analyse_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, n, fens, moves, move_offsets, out);
+                analyse_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, search_batch, n, fens, moves, move_offsets, out);
             }
         } else if (cfg.game == CATTUS_B200_GAME_CHESS) {
             sp::ChessRules rules;
-            analyse_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), m->engine, cfg, n, fens,
-                          moves, move_offsets, out);
+            analyse_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), m->engine, cfg, search_batch,
+                          n, fens, moves, move_offsets, out);
         } else if (cfg.game == CATTUS_B200_GAME_TTT) {
             sp::TttRules rules;
-            analyse_rules(rules, &rules, sizeof(rules), 9u, m->engine, cfg, n, fens, moves, move_offsets, out);
+            analyse_rules(rules, &rules, sizeof(rules), 9u, m->engine, cfg, search_batch, n, fens, moves, move_offsets, out);
         } else {
             throw Error(CATTUS_B200_EINVAL, "unknown game");
         }

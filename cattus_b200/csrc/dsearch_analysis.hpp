@@ -25,11 +25,33 @@
 namespace ds {
 
 struct AnalysisOpts {
-    uint32_t pv_max;  // principal variation plies (<= kPvMax)
+    uint32_t pv_max;             // principal variation plies (<= kPvMax)
+    uint32_t search_batch = 1;   // descents per minibatch under virtual loss (DESIGN.md section 15); 1: one leaf in flight
 };
 
-inline uint32_t analysis_stride_for(uint32_t max_children) {
-    return (static_cast<uint32_t>(sizeof(AnalysisHdr)) + 2u * kPvMax + 14u * max_children + 15u) & ~15u;
+// A minibatched search's entry ends in 16 more bytes: u32 minibatches, u32 collisions (batch_expand_slot).
+inline uint32_t analysis_stride_for(uint32_t max_children, uint32_t search_batch = 1) {
+    return ((static_cast<uint32_t>(sizeof(AnalysisHdr)) + 2u * kPvMax + 14u * max_children + 15u) & ~15u) + (search_batch > 1 ? 16u : 0u);
+}
+
+// search_batch of the C ABI's options: NULL, 0 or 1 is one leaf in flight.
+inline uint32_t analysis_search_batch(const cattus_b200_analysis_opts* opts) {
+    if (!opts) return 1;
+    if (opts->struct_size != sizeof(cattus_b200_analysis_opts)) throw sp::SpError{CATTUS_B200_EINVAL, "analysis opts struct_size mismatch"};
+    return opts->search_batch ? opts->search_batch : 1u;
+}
+
+// Concurrent searches of an analysis of n positions: device_games, 0 = min(n, max_batch / search_batch).  Every slot
+// writes up to search_batch evaluator rows per wave, so device_games x search_batch above max_batch is ERANGE.
+inline uint32_t analysis_slots(uint32_t device_games, uint32_t n, uint32_t max_batch, uint32_t search_batch) {
+    if (search_batch > 1 && static_cast<uint64_t>(device_games ? device_games : 1u) * search_batch > max_batch)
+        throw sp::SpError{CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(device_games) + ") x search_batch (" +
+                                                  std::to_string(search_batch) + ") exceeds the evaluator's max_batch (" + std::to_string(max_batch) + ")"};
+    if (device_games > max_batch)
+        throw sp::SpError{CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(device_games) + ") exceeds the evaluator's max_batch (" +
+                                                  std::to_string(max_batch) + ")"};
+    const uint32_t want = device_games ? device_games : max_batch / search_batch;
+    return std::max<uint32_t>(1, std::min<uint32_t>(want, n));
 }
 
 // The history ring of a slot (dsearch.cuh allocates it): chess keeps what detect_repetition can look back into, the
@@ -51,6 +73,8 @@ struct AnalysisResult {
     std::vector<uint32_t> visits;
     std::vector<float> w, prior;
     std::vector<uint16_t> pv;
+    uint32_t minibatches = 0;  // rounds of descents (one leaf in flight: one per simulation)
+    uint32_t collisions = 0;   // descents that ended on a leaf an earlier descent of their minibatch had claimed
 };
 
 // MctsParams of an analysis: the mcts.* fields without root noise (a noisy search would not be an analysis of the
@@ -156,13 +180,14 @@ class AnalysisDriver {
     static constexpr bool kChess = Rules::kChess;
 
   public:
+    // search_batch: the backend's (descents per minibatch; its result entries carry the minibatch counts when > 1)
     AnalysisDriver(const Rules& rules, const sp::Params& params, Backend& be, const std::vector<std::vector<Pos>>& histories,
-                   std::vector<AnalysisResult>& out)
-        : R(rules), params_(params), be_(be), hist_(histories), out_(out) {
+                   std::vector<AnalysisResult>& out, uint32_t search_batch = 1)
+        : R(rules), params_(params), be_(be), hist_(histories), out_(out), search_batch_(search_batch) {
         out_.assign(hist_.size(), AnalysisResult());
         job_of_slot_.assign(be.n_slots(), -1);
         cmd_stride_ = cmd_stride_for(be.max_children());
-        result_stride_ = analysis_stride_for(be.max_children());
+        result_stride_ = analysis_stride_for(be.max_children(), search_batch);
     }
 
     void run() {
@@ -262,6 +287,13 @@ class AnalysisDriver {
         AnalysisResult& r = out_[k];
         r.status = 0;
         r.simulations = params_.sim_num;
+        r.minibatches = params_.sim_num;
+        r.collisions = 0;
+        if (search_batch_ > 1) {
+            const uint32_t* counts = reinterpret_cast<const uint32_t*>(e + result_stride_ - 16u);
+            r.minibatches = counts[0];
+            r.collisions = counts[1];
+        }
         uint32_t total = 0;
         double sw = 0.0;
         for (uint32_t i = 0; i < count; ++i) {
@@ -307,7 +339,7 @@ class AnalysisDriver {
     std::deque<uint32_t> free_[2];
     size_t next_ = 0;
     uint32_t active_ = 0, active_pop_[2] = {0, 0};
-    uint32_t cmd_stride_ = 0, result_stride_ = 0;
+    uint32_t search_batch_ = 1, cmd_stride_ = 0, result_stride_ = 0;
     unsigned long long counters_[4] = {0, 0, 0, 0};
     std::vector<std::pair<Move, float>> probs_;
     std::vector<float> weights_;
@@ -339,6 +371,13 @@ inline int analysis_children(const std::vector<AnalysisResult>& r, uint32_t k, u
         if (w) w[i] = a.w[i];
         if (priors) priors[i] = a.prior[i];
     }
+    return CATTUS_B200_OK;
+}
+
+inline int analysis_batches(const std::vector<AnalysisResult>& r, uint32_t k, uint32_t* minibatches, uint32_t* collisions) {
+    if (k >= r.size()) return CATTUS_B200_ERANGE;
+    if (minibatches) *minibatches = r[k].minibatches;
+    if (collisions) *collisions = r[k].collisions;
     return CATTUS_B200_OK;
 }
 

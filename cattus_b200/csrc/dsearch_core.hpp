@@ -256,6 +256,17 @@ struct AnalysisHdr {
     uint32_t slot, count, pv_len, pad;
 };
 
+// One descent of a minibatch (Params::search_batch > 1, DESIGN.md section 15), written by batch_select_slot and backed up
+// by batch_expand_slot.  Its path is Params::bpaths[slot][descent][0, depth).
+enum DescentKind : uint32_t { kDescentCollision = 0, kDescentLeaf = 1, kDescentScored = 2 };
+struct BatchDescent {
+    int32_t leaf;    // block of the node the descent ended on
+    uint32_t depth;  // edges on its path
+    uint32_t kind;   // DescentKind
+    uint32_t row;    // kDescentLeaf: the leaf's evaluator row
+    float value;     // kDescentScored: repetition 0, finished position the winner's +-1 (player 1's view)
+};
+
 template <class Rules>
 struct Params {
     const void* rules;  // device copy of the rule tables (HexRulesT / ChessTables; unused for tic-tac-toe)
@@ -290,6 +301,11 @@ struct Params {
     const typename Rules::Pos* roots;  // root histories of this wave's kCmdSetRoot commands
     uint32_t analysis;                 // 1: finished searches post the AnalysisHdr layout instead of ResultHdr
     uint32_t pv_max;                   // principal variation plies to post (<= kPvMax)
+    // minibatched analysis (batch_select_slot / batch_expand_slot); all zero with one leaf in flight
+    uint32_t search_batch;      // descents per minibatch (> 1)
+    BatchDescent* descents;     // [n_slots][search_batch]
+    PathStep* bpaths;           // [n_slots][search_batch][path_cap]
+    uint32_t* vcount;           // [n_slots][pool_words / 4]: virtual count of each child row (16-byte pool unit) of the tree
 };
 
 template <class Pos>
@@ -465,7 +481,8 @@ struct Core {
     // Analysis result: every root row, and the principal variation -- from the root, repeatedly the child with the most
     // visits, equal counts going to the smallest insertion index (the last maximum in edges() order, as
     // choose_move_from_probabilities at temperature 0 picks), until a node that was never expanded or pv_max plies.
-    CB2_HD static void post_analysis(const P& p, uint32_t wave, uint32_t si, uint32_t* pool, int32_t root) {
+    // Returns the posted entry.
+    CB2_HD static uint8_t* post_analysis(const P& p, uint32_t wave, uint32_t si, uint32_t* pool, int32_t root) {
         const int ln = lane();
         const int count = T::hdr(pool, root)->count;
         uint32_t k = 0;
@@ -516,6 +533,7 @@ struct Core {
             ah->pv_len = len;
             ah->pad = 0;
         }
+        return e;
     }
 
     // MctsPlayer::detect_repetition (mod.rs:133-154), as the host driver does it: each path position is counted
@@ -937,6 +955,224 @@ struct Core {
             S.sims_left = sims_left;
             S.noise_n = noise_n;
             atomic_add_u64(p.counters + 0, 1ull);
+        }
+    }
+
+    // ---------------------------------------------------------------- minibatches under virtual loss (DESIGN.md section 15)
+    // Analysis with search_batch = L > 1.  One wave runs one minibatch of a slot: batch_select_slot makes its
+    // k = min(L, sims_left) descents, batch_expand_slot backs them up once the evaluator has run.  The slot keeps
+    // the number of descents in flight in path_len and its minibatch / collision counts in pad[0] / pad[1].
+    //
+    // Phase 1: descents j = 0 .. k-1 in order on a FROZEN tree (no n, w or children change; first visits of an edge are
+    // linked as select links them).  Every child row is seen with its virtual count v, the descents of this minibatch
+    // that took it so far: n' = n + v, w' = w - v, then select's heuristic and tie rule; with every v = 0 this is select
+    // bit for bit.  A descent ends where select ends and is a repetition (value 0), a finished position (the winner's
+    // +-1), a new leaf (the first to end on that unexpanded node: claimed with expanded = 2, its record written to the
+    // evaluator batch) or a collision (a later one), then adds 1 to v along its path.  No cache probe: a hit would have
+    // to be copied out before the expand kernel's inserts could evict it, and the tree's own leaves fill the batch.
+    CB2_HD static void batch_select_slot(const Rules& R, const P& p, uint32_t si, uint32_t wave) {
+        SlotState& S = p.slots[si];
+        const uint32_t pw = S.phase;
+        const uint32_t phase0 = pw & 3u, start_wave = pw >> 2;
+        const uint32_t cur = S.cur;
+        const uint32_t sims_left = S.sims_left;
+        Tree t;
+        t.pool = p.pools + (static_cast<size_t>(si) * 3u + S.buf[cur & 1u]) * p.pool_words;
+        t.used = S.used[cur & 1u];
+        t.root = S.root[cur & 1u];
+        const uint32_t hist_len = S.hist_len;
+        wsync();
+        if (phase0 != kRun || start_wave > wave) return;
+        const int ln = lane();
+        const uint32_t e = p.n_evals > 1 ? cur : 0u;
+        const float ef = p.explore[cur];
+        const uint32_t L = p.search_batch;
+        const uint32_t k = sims_left < L ? sims_left : L;
+        uint32_t* vc = p.vcount + static_cast<size_t>(si) * (p.pool_words >> 2);
+        BatchDescent* bd = p.descents + static_cast<size_t>(si) * L;
+        uint32_t err = 0, rows = 0;
+        for (uint32_t j = 0; j < k && !err; ++j) {
+            PathStep* path = p.bpaths + (static_cast<size_t>(si) * L + j) * p.path_cap;
+            int32_t node = t.root;
+            uint32_t depth = 0;
+            for (;;) {
+                const Hdr* h = T::hdr(t.pool, node);
+                if (h->expanded != 1 || R.status(h->pos) != 0) break;
+                const int count = h->count;
+                const Child* ch = T::child(t.pool, node);
+                const uint32_t* vn = vc + ((static_cast<uint32_t>(node) + T::kHdrWords) >> 2);
+                int part = 0;
+                for (int i = ln; i < count; i += DS_LANES) part += ch[i].n + static_cast<int>(vn[i]);
+                const int simcount = 1 + wsum(part);
+                const float sq = fsqrt(static_cast<float>(simcount));
+                float bv = -__builtin_inff();
+                int bi = 0x7FFFFFFF;
+                uint32_t be = 0;
+                for (int i = ln; i < count; i += DS_LANES) {
+                    const Child c = ch[i];
+                    const uint32_t v = vn[i];
+                    const int n = c.n + static_cast<int>(v);
+                    const float w = fadd(c.w, -static_cast<float>(v));
+                    const float exploit = n == 0 ? 0.0f : fdiv(w, static_cast<float>(n));
+                    const float explore = fmul(fmul(ef, c.init), fdiv(sq, static_cast<float>(1 + n)));
+                    const float s = fadd(exploit, explore);
+                    if (s == s && (bi == 0x7FFFFFFF || s > bv)) {
+                        bv = s;
+                        bi = i;
+                        be = c.edge;
+                    }
+                }
+                wargmax(bv, bi, be);
+                if (bi == 0x7FFFFFFF) {
+                    bi = count - 1;
+                    be = ch[bi].edge;
+                }
+                int32_t c = T::edge_child(be);
+                if (c < 0) {
+                    c = materialise(R, p, t, node, count, bi);
+                    if (c < 0) {
+                        err = kErrPool;
+                        break;
+                    }
+                }
+                if (depth >= p.path_cap) {
+                    err = kErrPath;
+                    break;
+                }
+                if (ln == 0) {
+                    PathStep ps;
+                    ps.c_idx = node + T::kHdrWords + 4 * bi;
+                    ps.pad = 0;
+                    ps.child = c;
+                    path[depth] = ps;
+                }
+                depth += 1;
+                node = c;
+            }
+            if (err) break;
+            wsync();
+            Hdr* lh = T::hdr(t.pool, node);
+            BatchDescent d;
+            d.leaf = node;
+            d.depth = depth;
+            d.row = 0;
+            d.value = 0.0f;
+            const bool repeated = detect_repetition(R, p, t.pool, path, depth, si, hist_len);
+            const int st = R.status(lh->pos);
+            if (repeated || st != 0) {
+                d.kind = kDescentScored;
+                d.value = repeated ? 0.0f : (st == 3 ? 0.0f : (st == 1 ? 1.0f : -1.0f));
+            } else if (lh->expanded == 2) {
+                d.kind = kDescentCollision;
+            } else {
+                d.kind = kDescentLeaf;
+                d.row = emit_record(R, p, e, t.pool, node);
+                if (d.row == 0xFFFFFFFFu) {
+                    err = kErrRows;
+                    break;
+                }
+                rows += 1;
+                if (ln == 0) lh->expanded = 2;
+            }
+            for (uint32_t s = static_cast<uint32_t>(ln); s < depth; s += DS_LANES) vc[static_cast<uint32_t>(path[s].c_idx) >> 2] += 1u;
+            if (ln == 0) bd[j] = d;
+            wsync();
+        }
+        if (ln == 0) {  // the slot's scalars are read again rather than kept live across the descents
+            SlotState& Q = p.slots[si];
+            const uint32_t qc = Q.cur, left = Q.sims_left;
+            uint32_t phase = kWaitEval;
+            if (err) {
+                atomic_or_u32(p.error, err);
+                Q.error = err;
+                phase = kIdle;
+            }
+            Q.phase = phase;
+            Q.path_len = left < L ? left : L;
+            Q.used[qc & 1u] = t.used;
+            if (t.used > Q.pad0) {
+                Q.pad0 = t.used;
+                atomic_max_u32(p.max_used, t.used);
+            }
+            if (left == p.sim_num[qc]) {  // the search's first minibatch
+                Q.pad[0] = 0;
+                Q.pad[1] = 0;
+            }
+            if (rows) atomic_add_u64(p.counters + 1, rows);
+        }
+    }
+
+    // Phase 3: in descent order, a new leaf gets create_children from its evaluation, then it and every scored descent is
+    // backpropagated as expand_slot / select do; a collision does nothing.  Per edge that is a sum in ascending descent
+    // order, as the sequential definition adds.  Then every virtual count of the minibatch is dropped.
+    CB2_HD static void batch_expand_slot(const Rules& R, const P& p, uint32_t si, uint32_t wave) {
+        SlotState& S = p.slots[si];
+        const uint32_t phase0 = S.phase & 3u, cur = S.cur, k = S.path_len;
+        uint32_t* pool = p.pools + (static_cast<size_t>(si) * 3u + S.buf[cur & 1u]) * p.pool_words;
+        const int32_t root = S.root[cur & 1u];
+        wsync();
+        if (phase0 != kWaitEval) return;
+        const int ln = lane();
+        const uint32_t e = p.n_evals > 1 ? cur : 0u;
+        const EvalIo& io = p.eval[e];
+        const uint32_t L = p.search_batch;
+        const uint8_t root_turn = T::hdr(pool, root)->pos.turn;
+        uint32_t* vc = p.vcount + static_cast<size_t>(si) * (p.pool_words >> 2);
+        const BatchDescent* bd = p.descents + static_cast<size_t>(si) * L;
+        uint32_t n_sims = 0, n_scored = 0, n_coll = 0, noise_n = 0;
+        for (uint32_t j = 0; j < k; ++j) {
+            const BatchDescent d = bd[j];
+            const PathStep* path = p.bpaths + (static_cast<size_t>(si) * L + j) * p.path_cap;
+            if (d.kind == kDescentCollision) {
+                n_coll += 1;
+                continue;
+            }
+            float v = d.value;
+            if (d.kind == kDescentLeaf) {
+                const float* probs = io.probs + static_cast<size_t>(d.row) * io.prob_stride;
+                const float value = io.values[d.row];
+                if (p.cache[e].enabled) {
+                    uint64_t key[4];
+                    const uint64_t kh = position_key(R, T::hdr(pool, d.leaf)->pos, key);
+                    cache_insert(p.cache[e], key, kh, T::hdr(pool, d.leaf)->count, probs, value);
+                }
+                apply_evaluation(R, p, si, cur, pool, d.leaf, root, probs, value, noise_n, 0u);  // children only: depth 0
+                v = T::hdr(pool, d.leaf)->pos.turn != 1 ? -value : value;
+            } else {
+                n_scored += 1;
+            }
+            wsync();
+            backpropagate(pool, path, d.depth, root_turn, v);
+            n_sims += 1;
+            wsync();
+        }
+        for (uint32_t j = 0; j < k; ++j) {
+            const uint32_t depth = bd[j].depth;
+            const PathStep* path = p.bpaths + (static_cast<size_t>(si) * L + j) * p.path_cap;
+            for (uint32_t s = static_cast<uint32_t>(ln); s < depth; s += DS_LANES) vc[static_cast<uint32_t>(path[s].c_idx) >> 2] = 0u;
+        }
+        wsync();
+        // the slot's counts are read here rather than kept live across the backups
+        SlotState& Q = p.slots[si];
+        const uint32_t left = Q.sims_left - n_sims, minibatches = Q.pad[0] + 1u, collisions = Q.pad[1] + n_coll;
+        wsync();
+        uint32_t phase = kRun;
+        if (left == 0) {
+            uint8_t* entry = post_analysis(p, wave, si, pool, root);
+            if (ln == 0) {
+                uint32_t* counts = reinterpret_cast<uint32_t*>(entry + p.result_stride - 16u);
+                counts[0] = minibatches;
+                counts[1] = collisions;
+            }
+            phase = kDone;
+        }
+        if (ln == 0) {
+            Q.phase = phase;
+            Q.sims_left = left;
+            Q.pad[0] = minibatches;
+            Q.pad[1] = collisions;
+            if (n_sims) atomic_add_u64(p.counters + 0, n_sims);
+            if (n_scored) atomic_add_u64(p.counters + 2, n_scored);
         }
     }
 

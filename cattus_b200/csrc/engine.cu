@@ -2221,7 +2221,24 @@ int cattus_b200_analyse(cattus_b200_t* model, const cattus_b200_selfplay_cfg* cf
         if (!cfg || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
         *out = nullptr;
         std::unique_ptr<cattus_b200_analysis> r(new cattus_b200_analysis());
-        cb2::analyse_run(model, *cfg, n, fens, moves, move_offsets, r->res);
+        cb2::analyse_run(model, *cfg, 1, n, fens, moves, move_offsets, r->res);
+        *out = r.release();
+    });
+}
+
+int cattus_b200_analyse_opts(cattus_b200_t* model, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_analysis_opts* opts, uint32_t n,
+                             const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, cattus_b200_analysis_t** out) {
+    return guarded([&] {
+        if (!cfg || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        *out = nullptr;
+        uint32_t search_batch = 1;
+        try {
+            search_batch = ds::analysis_search_batch(opts);
+        } catch (const sp::SpError& e) {
+            throw cb2::Error(e.code, e.msg);
+        }
+        std::unique_ptr<cattus_b200_analysis> r(new cattus_b200_analysis());
+        cb2::analyse_run(model, *cfg, search_batch, n, fens, moves, move_offsets, r->res);
         *out = r.release();
     });
 }
@@ -2240,6 +2257,9 @@ int cattus_b200_analysis_children(const cattus_b200_analysis_t* r, uint32_t k, u
 }
 int cattus_b200_analysis_pv(const cattus_b200_analysis_t* r, uint32_t k, uint16_t* pv, uint32_t cap) {
     return r ? ds::analysis_pv(r->res, k, pv, cap) : CATTUS_B200_EINVAL;
+}
+int cattus_b200_analysis_batches(const cattus_b200_analysis_t* r, uint32_t k, uint32_t* minibatches, uint32_t* collisions) {
+    return r ? ds::analysis_batches(r->res, k, minibatches, collisions) : CATTUS_B200_EINVAL;
 }
 void cattus_b200_analysis_free(cattus_b200_analysis_t* r) { delete r; }
 

@@ -14,6 +14,13 @@ with 64 / 128 / 256 filters).
 with the leaf the search is waiting for; they only land in the value-function cache, so the moves played are unchanged
 and a `go` needs about an eighth of the evaluator round trips.
 
+`search_batch` (top-level key, default 1) L > 1 runs every `go` as a one-position analysis on the device-resident search
+(cattus_b200.analysis) in minibatches of L descents under virtual loss (DESIGN.md section 15): the evaluator sees up to L
+leaves of the tree at once instead of one.  Each `go` then starts from a FRESH tree with the position's history (no tree
+is kept between `go`s), searches without root noise, and its result is that of the minibatched search, not the one-leaf
+search's.  It prints `info depth <PV plies> nodes <sim_num> nps <n> score cp <cp> pv <moves>` before `bestmove`, where
+cp = round(90 * tan(1.5637541897 * q)) of the side to move's mean score q in [-1, 1] (clamped to +-0.99), a monotone map.
+
 Commands handled as in uci.rs:27-73: uci, isready, setoption, ucinewgame, position [fen <FEN> | startpos] [moves ...],
 go (its arguments are parsed and ignored, as there), stop, quit.  One MctsPlayer per game: the tree of the previous
 `go` is reused when the new position is in it; every search runs `mcts.sim_num` simulations with one leaf in flight.
@@ -22,7 +29,9 @@ from __future__ import annotations
 
 import argparse
 import json
+import math
 import sys
+import time
 from pathlib import Path
 from typing import List, Optional, TextIO
 
@@ -30,6 +39,13 @@ from .network import CudaNetwork
 from .selfplay import ChessSearch
 
 GO_KEYS = ("searchmoves", "ponder", "wtime", "btime", "winc", "binc", "movestogo", "depth", "nodes", "mate", "movetime", "infinite")
+
+
+def q_to_cp(q: float) -> int:
+    """The side to move's mean score q in [-1, 1] as centipawns: round(90 * tan(1.5637541897 * q)), q clamped to +-0.99
+    (monotone; 0 -> 0, +-0.5 -> +-90, +-0.99 -> +-2720)."""
+    q = max(-0.99, min(0.99, float(q)))
+    return int(round(90.0 * math.tan(1.5637541897 * q)))
 
 
 def parse_args(args: List[str], keys) -> dict:
@@ -54,6 +70,9 @@ class UCI:
         cfg = dict(cfg)
         cfg.setdefault("speculate", 31 if (cfg.get("mcts") or {}).get("cache_size") else 0)
         self.cfg = cfg
+        self.search_batch = int(cfg.get("search_batch", 1))
+        if self.search_batch < 1:
+            raise ValueError("search_batch must be >= 1")
         self.model = model
         self.eval_fn = eval_fn
         self.out = out
@@ -93,6 +112,11 @@ class UCI:
             self.moves = list(a.get("moves", []))
         elif command == "go":
             parse_args(args, GO_KEYS)
+            if self.search_batch > 1:
+                if self.moves is None:
+                    raise ValueError("go before position")
+                self.go_batched()
+                return True
             if self.player is None:  # the reference unwraps None here; a GUI that skips ucinewgame still gets a player
                 self.player = ChessSearch(self.cfg, self.model, self.eval_fn)
             if self.moves is None:
@@ -110,6 +134,29 @@ class UCI:
         else:
             print(f"unknown command {command}", file=sys.stderr)
         return True
+
+    def go_batched(self) -> None:
+        """One minibatched device analysis of the current position and history, from a fresh tree."""
+        from .analysis import analyse
+        from .selfplay import move_to_lan
+
+        mc = dict(self.cfg.get("mcts") or {})
+        mc["prior_noise_epsilon"] = 0.0  # an analysis has no root noise
+        cfg = {"mcts": mc, "device_games": 1}
+        for key in ("device_tree_kwords",):
+            if key in self.cfg:
+                cfg[key] = self.cfg[key]
+        t0 = time.perf_counter()
+        a = analyse(self.model, "chess", [(self.fen, list(self.moves))], cfg, search_batch=self.search_batch)[0]
+        secs = time.perf_counter() - t0
+        self.last_stats = {"simulations": a.simulations, "seconds": secs, "minibatches": a.minibatches, "collisions": a.collisions, "q": a.q,
+                           "analysis": a}
+        if a.status != 0:  # the game is over: there is no move to search
+            self.send("bestmove 0000")
+            return
+        pv = " ".join(move_to_lan(m) for m in a.pv)
+        self.send(f"info depth {len(a.pv)} nodes {a.simulations} nps {int(a.simulations / max(secs, 1e-9))} score cp {q_to_cp(a.q)} pv {pv}")
+        self.send(f"bestmove {move_to_lan(a.best_move)}")
 
     def run(self, inp: TextIO = sys.stdin) -> None:
         for line in inp:
@@ -131,8 +178,10 @@ def main(argv=None) -> int:
     inference = model_cfg.get("inference") or {}
     if inference.get("engine", "cuda-b200") != "cuda-b200":
         raise SystemExit(f"this executable is the cuda-b200 engine; config.model.inference.engine is {inference.get('engine')!r} (there is no CPU fallback)")
-    # room for the speculative rows: a device batch of up to 64 positions costs what one position costs
-    with CudaNetwork(Path(model_cfg["model_path"]), "chess", device=int(inference.get("device", 0)), batch_size=max(64, int(model_cfg.get("batch_size", 1))),
+    # room for the speculative rows: a device batch of up to 64 positions costs what one position costs; a minibatched
+    # search writes up to search_batch rows per round
+    batch = max(64, int(model_cfg.get("batch_size", 1)), int(cfg.get("search_batch", 1)))
+    with CudaNetwork(Path(model_cfg["model_path"]), "chess", device=int(inference.get("device", 0)), batch_size=batch,
                      n_streams=1, precision=inference.get("precision", "bf16")) as nw:
         UCI(cfg, model=nw).run()
     return 0

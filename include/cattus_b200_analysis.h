@@ -50,6 +50,21 @@ typedef struct cattus_b200_analysis_position {
 int cattus_b200_analyse(cattus_b200_t* model, const cattus_b200_selfplay_cfg* cfg, uint32_t n, const char* const* fens, const uint16_t* moves,
                         const uint32_t* move_offsets, cattus_b200_analysis_t** out);
 
+/* Options of cattus_b200_analyse_opts.  struct_size must be sizeof(cattus_b200_analysis_opts). */
+typedef struct cattus_b200_analysis_opts {
+    uint32_t struct_size;
+    uint32_t search_batch; /* descents per minibatch under virtual loss (DESIGN.md section 15); 0 or 1: one leaf in flight */
+} cattus_b200_analysis_opts;
+
+/* cattus_b200_analyse with options; opts NULL is cattus_b200_analyse.  With search_batch L > 1 every search runs
+ * minibatches of L descents of its tree under virtual loss, so that the evaluator sees up to L leaves of one tree at
+ * once: the mode for searching one position, or a few, deeply.  Its results are deterministic -- they depend on the
+ * position, its history, the network, sim_num, explore_factor and L alone -- but are not those of one leaf in flight.
+ * device_games 0 means min(n, max_batch / L); device_games x L above the model's max_batch is ERANGE, a bad
+ * opts->struct_size EINVAL. */
+int cattus_b200_analyse_opts(cattus_b200_t* model, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_analysis_opts* opts, uint32_t n,
+                             const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, cattus_b200_analysis_t** out);
+
 int cattus_b200_analysis_count(const cattus_b200_analysis_t* r, uint32_t* n);
 int cattus_b200_analysis_get(const cattus_b200_analysis_t* r, uint32_t k, cattus_b200_analysis_position* out);
 /* The root's children in edges() order (newest first, the order calc_moves_probabilities lists them): move, visits
@@ -60,6 +75,10 @@ int cattus_b200_analysis_children(const cattus_b200_analysis_t* r, uint32_t k, u
 /* The principal variation: from the root, repeatedly the most visited child (equal counts: the one best_move's rule
  * picks), until a node that was never expanded or 16 plies. */
 int cattus_b200_analysis_pv(const cattus_b200_analysis_t* r, uint32_t k, uint16_t* pv, uint32_t cap);
+/* Minibatches the search of position k ran and its descents that were collisions (ended on a leaf an earlier descent
+ * of the same minibatch had claimed).  One leaf in flight: minibatches = simulations, collisions 0.  Not searched: 0, 0.
+ * Either output may be NULL. */
+int cattus_b200_analysis_batches(const cattus_b200_analysis_t* r, uint32_t k, uint32_t* minibatches, uint32_t* collisions);
 void cattus_b200_analysis_free(cattus_b200_analysis_t* r);
 
 #ifdef __cplusplus
