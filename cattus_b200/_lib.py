@@ -97,6 +97,16 @@ class AnalysisOpts(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("search_batch", C.c_uint32)]
 
 
+class SelfPlayOpts(C.Structure):
+    """cattus_b200_selfplay_opts (include/cattus_b200_selfplay.h)."""
+    _fields_ = [("struct_size", C.c_uint32), ("search_batch", C.c_uint32)]
+
+
+class MatchOpts(C.Structure):
+    """cattus_b200_match_opts (include/cattus_b200_match.h)."""
+    _fields_ = [("struct_size", C.c_uint32), ("search_batch_a", C.c_uint32), ("search_batch_b", C.c_uint32)]
+
+
 class MatchSide(C.Structure):
     """cattus_b200_match_side (include/cattus_b200_match.h)."""
     _fields_ = [("struct_size", C.c_uint32), ("sim_num", C.c_uint32), ("explore_factor", C.c_float)]
@@ -142,7 +152,9 @@ SYMBOLS = {
     # include/cattus_b200_selfplay.h
     "cattus_b200_selfplay_run": (C.c_int, [_H, _H, C.POINTER(SelfPlayCfg), C.POINTER(_H)]),
     "cattus_b200_selfplay_run_with": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(SelfPlayCfg), C.POINTER(_H)]),
+    "cattus_b200_selfplay_run_opts": (C.c_int, [_H, _H, C.POINTER(SelfPlayCfg), C.POINTER(SelfPlayOpts), C.POINTER(_H)]),
     "cattus_b200_selfplay_summary_get": (C.c_int, [_H, C.POINTER(SelfPlaySummary)]),
+    "cattus_b200_selfplay_batches": (C.c_int, [_H, _u64p, _u64p]),
     "cattus_b200_selfplay_game_count": (C.c_int, [_H, _u32p]),
     "cattus_b200_selfplay_game_info": (C.c_int, [_H, C.c_uint32, _u32p, _u32p, _u32p]),
     "cattus_b200_selfplay_game_moves": (C.c_int, [_H, C.c_uint32, _u8p, C.c_uint32]),
@@ -167,7 +179,10 @@ SYMBOLS = {
     # include/cattus_b200_match.h
     "cattus_b200_match_run": (C.c_int, [_H, _H, C.POINTER(SelfPlayCfg), C.POINTER(MatchSide), C.c_uint32, C.POINTER(C.c_char_p), _u16p, _u32p,
                                         C.POINTER(_H)]),
+    "cattus_b200_match_run_opts": (C.c_int, [_H, _H, C.POINTER(SelfPlayCfg), C.POINTER(MatchSide), C.POINTER(MatchOpts), C.c_uint32,
+                                             C.POINTER(C.c_char_p), _u16p, _u32p, C.POINTER(_H)]),
     "cattus_b200_match_summary_get": (C.c_int, [_H, C.POINTER(MatchSummary)]),
+    "cattus_b200_match_batches": (C.c_int, [_H, C.c_uint32, _u64p, _u64p]),
     "cattus_b200_match_opening_status": (C.c_int, [_H, C.c_uint32, _u32p]),
     "cattus_b200_match_game_get": (C.c_int, [_H, C.c_uint32, C.POINTER(MatchGame)]),
     "cattus_b200_match_game_moves": (C.c_int, [_H, C.c_uint32, _u16p, C.c_uint32]),

@@ -52,10 +52,11 @@ __global__ void __launch_bounds__(128, DS_EXPAND_MIN_BLOCKS) ds_expand_kernel(ds
     ds::Core<Rules>::expand_slot(R, p, warp, wave);
 }
 
-// Minibatched analysis (search_batch > 1, DESIGN.md section 15): one warp per searched tree, captured in a wave graph of
-// their own instead of select / expand.
+// Minibatched search (a side with search_batch > 1, DESIGN.md sections 15 and 16): one warp per searched tree, captured
+// in a wave graph of their own instead of select / expand.  The select kernel states its one block per SM: without it
+// ptxas caps tic-tac-toe at 64 registers and spills, and hex 9-11 spill more.
 template <class Rules>
-__global__ void __launch_bounds__(128) ds_select_batch_kernel(ds::Params<Rules> p) {
+__global__ void __launch_bounds__(128, 1) ds_select_batch_kernel(ds::Params<Rules> p) {
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (warp >= p.n_slots) return;
     const uint32_t wave = reinterpret_cast<const uint32_t*>(p.cmds)[1];
@@ -90,11 +91,18 @@ template <class Rules>
 class DsCudaBackend {
   public:
     // `roots_cap` > 0 adds the per-wave root upload of kCmdSetRoot (analysis, matches from openings): up to that many
-    // history positions per wave.  `analysis` (optional) switches the finished searches to the analysis result layout.
-    // Without either everything is the self-play arrangement.
+    // history positions per wave.  `search_batch` (optional) is each side's descents per minibatch: when one of them is
+    // above 1 the waves run the minibatch kernels.  `analysis` (optional) switches the finished searches to the analysis
+    // result layout.  Without them everything is the self-play arrangement.
     DsCudaBackend(const void* rules_blob, size_t rules_bytes, uint32_t max_children, Engine* e1, Engine* e2, const cattus_b200_selfplay_cfg& cfg,
-                  const sp::Params params[2], uint32_t n_slots, uint32_t roots_cap = 0, const ds::AnalysisOpts* analysis = nullptr)
-        : max_children_(max_children), n_slots_(n_slots), search_batch_(analysis ? std::max<uint32_t>(1, analysis->search_batch) : 1u) {
+                  const sp::Params params[2], uint32_t n_slots, uint32_t roots_cap = 0, const uint32_t* search_batch = nullptr,
+                  const ds::AnalysisOpts* analysis = nullptr)
+        : max_children_(max_children), n_slots_(n_slots) {
+        if (search_batch) {
+            side_batch_[0] = std::max<uint32_t>(1, search_batch[0]);
+            side_batch_[1] = std::max<uint32_t>(1, search_batch[1]);
+            search_batch_ = std::max(side_batch_[0], side_batch_[1]);
+        }
         eng_[0] = e1;
         eng_[1] = e2;
         n_evals_ = e2 ? 2 : 1;
@@ -268,7 +276,9 @@ class DsCudaBackend {
                     p.pv_max = std::min<uint32_t>(analysis->pv_max, ds::kPvMax);
                 }
                 if (search_batch_ > 1) {
-                    p.search_batch = search_batch_;
+                    p.search_batch.side[0] = side_batch_[0];
+                    p.search_batch.side[1] = side_batch_[1];
+                    p.search_batch.max = search_batch_;
                     p.descents = static_cast<ds::BatchDescent*>(d_descents_) + static_cast<size_t>(base) * search_batch_;
                     p.bpaths = static_cast<ds::PathStep*>(d_bpaths_) + static_cast<size_t>(base) * search_batch_ * path_cap;
                     p.vcount = static_cast<uint32_t*>(d_vcount_) + static_cast<size_t>(base) * (pool_words_ >> 2);
@@ -369,12 +379,12 @@ class DsCudaBackend {
             } else {
                 ds_begin_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             }
-            if (P.p.search_batch > 1)
+            if (search_batch_ > 1)
                 ds_select_batch_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             else
                 ds_select_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             for (uint32_t e = 0; e < n_evals_; ++e) eng_[e]->resident_enqueue(P.io[e].lane, P.stream);
-            if (P.p.search_batch > 1)
+            if (search_batch_ > 1)
                 ds_expand_batch_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             else
                 ds_expand_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
@@ -433,6 +443,7 @@ class DsCudaBackend {
     Engine* eng_[2] = {nullptr, nullptr};
     uint32_t n_evals_ = 1, n_pops_ = 1, split_ = 0, depth_ = 2, n_bufs_ = 3, max_children_ = 0, n_slots_ = 0, pool_words_ = 0, cmd_stride_ = 0,
              result_stride_ = 0, kernels_per_wave_ = 0, roots_cap_ = 0, search_batch_ = 1;
+    uint32_t side_batch_[2] = {1, 1};  // search_batch_ is the larger
     size_t cmd_bytes_ = 0, result_buf_bytes_ = 0;
     void *d_rules_ = nullptr, *d_slots_ = nullptr, *d_pools_ = nullptr, *d_paths_ = nullptr, *d_noise_ = nullptr, *d_hist_ = nullptr;
     void *d_descents_ = nullptr, *d_bpaths_ = nullptr, *d_vcount_ = nullptr;
@@ -447,17 +458,24 @@ class DsCudaBackend {
 
 template <class Rules>
 static void dsearch_run_rules(const Rules& rules, const void* blob, size_t blob_bytes, uint32_t max_children, Engine* e1, Engine* e2,
-                              const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], sp::Shared& sh) {
+                              const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], const uint32_t search_batch[2], sp::Shared& sh) {
     const uint32_t stride = std::max<uint32_t>(1, cfg.game_stride);
     const uint32_t my_games = cfg.games_num > cfg.first_game ? (cfg.games_num - cfg.first_game + stride - 1) / stride : 0;
     if (my_games == 0) return;
-    const uint32_t n_slots = std::max<uint32_t>(1, std::min<uint32_t>(cfg.device_games, my_games));
+    uint32_t max_batch = 0xFFFFFFFFu;
+    for (Engine* e : {e1, e2}) {
+        if (!e) continue;
+        cattus_b200_info info;
+        e->get_info(&info);
+        max_batch = std::min(max_batch, info.max_batch);
+    }
+    const uint32_t n_slots = ds::selfplay_slots(cfg.device_games, my_games, max_batch, std::max(search_batch[0], search_batch[1]));
     const auto t0 = std::chrono::steady_clock::now();
-    DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e1, e2, cfg, params, n_slots);
+    DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e1, e2, cfg, params, n_slots, 0, search_batch);
     if (std::getenv("CATTUS_B200_DSEARCH_PROFILE"))
         std::fprintf(stderr, "device search: %u slots in %u population(s), %u words per tree buffer, set up in %.3f s\n", n_slots, be.populations(),
                      be.pool_words(), be.setup_seconds());
-    ds::Driver<Rules, DsCudaBackend<Rules>> drv(rules, cfg, params, be, sh);
+    ds::Driver<Rules, DsCudaBackend<Rules>> drv(rules, cfg, params, be, sh, nullptr, search_batch);
     drv.run();
     const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     const uint64_t waves = be.waves();
@@ -484,9 +502,10 @@ static void analyse_rules(const Rules& rules, const void* blob, size_t blob_byte
         return;
     }
     // a wave's root upload: a few history positions per slot on average; a longer run of long histories waits a wave
-    const ds::AnalysisOpts opts{ds::kPvMax, search_batch};
+    const ds::AnalysisOpts opts{ds::kPvMax};
+    const uint32_t sides[2] = {search_batch, search_batch};
     const auto t0 = std::chrono::steady_clock::now();
-    DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e, nullptr, cfg, params, n_slots, n_slots * 8u + ds::hist_cap_for<Rules>(), &opts);
+    DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e, nullptr, cfg, params, n_slots, n_slots * 8u + ds::hist_cap_for<Rules>(), sides, &opts);
     ds::AnalysisDriver<Rules, DsCudaBackend<Rules>> drv(rules, params[0], be, hist, out, search_batch);
     drv.run();
     const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
@@ -528,8 +547,8 @@ void analyse_run(cattus_b200_t* m, const cattus_b200_selfplay_cfg& cfg, uint32_t
 // and result layout with kCmdSetRoot's root upload.
 template <class Rules>
 static void match_rules(const Rules& rules, const void* blob, size_t blob_bytes, uint32_t max_children, Engine* e1, Engine* e2,
-                        const cattus_b200_selfplay_cfg& cfg, const cattus_b200_match_side* side_b, uint32_t n, const char* const* fens,
-                        const uint16_t* moves, const uint32_t* move_offsets, ds::MatchResult& out) {
+                        const cattus_b200_selfplay_cfg& cfg, const cattus_b200_match_side* side_b, const uint32_t search_batch[2], uint32_t n,
+                        const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, ds::MatchResult& out) {
     const auto t0 = std::chrono::steady_clock::now();
     sp::Params params[2];
     ds::match_params(cfg, side_b, params);
@@ -549,10 +568,10 @@ static void match_rules(const Rules& rules, const void* blob, size_t blob_bytes,
     const auto openings = ds::match_openings(rules, n, fens, moves, move_offsets, out.opening_status);
     const uint32_t games = ds::match_games(out.opening_status);
     if (games) {
-        const uint32_t n_slots = std::min(cfg.device_games ? cfg.device_games : max_batch, games);
+        const uint32_t n_slots = ds::analysis_slots(cfg.device_games, games, max_batch, std::max(search_batch[0], search_batch[1]));
         // a wave's root upload: a few history positions per slot on average; a longer run of long histories waits a wave
-        DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e1, e2, cfg, params, n_slots, n_slots * 8u + ds::hist_cap_for<Rules>());
-        ds::match_play(rules, cfg, params, be, openings, out);
+        DsCudaBackend<Rules> be(blob, blob_bytes, max_children, e1, e2, cfg, params, n_slots, n_slots * 8u + ds::hist_cap_for<Rules>(), search_batch);
+        ds::match_play(rules, cfg, params, be, openings, out, search_batch);
         const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         const uint64_t waves = be.waves();
         e1->note_resident(waves, out.evaluations, waves * be.kernels_per_wave(), waves ? secs / static_cast<double>(waves) : 0.0);
@@ -560,8 +579,9 @@ static void match_rules(const Rules& rules, const void* blob, size_t blob_bytes,
     out.seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 }
 
-void match_run(cattus_b200_t* ma, cattus_b200_t* mb, const cattus_b200_selfplay_cfg& cfg, const cattus_b200_match_side* side_b, uint32_t n,
-               const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, ds::MatchResult& out) {
+void match_run(cattus_b200_t* ma, cattus_b200_t* mb, const cattus_b200_selfplay_cfg& cfg, const cattus_b200_match_side* side_b,
+               const uint32_t search_batch[2], uint32_t n, const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets,
+               ds::MatchResult& out) {
     try {
         if (!ma) throw Error(CATTUS_B200_EINVAL, "null evaluator handle (there is no CPU fallback)");
         if (cfg.struct_size != sizeof(cattus_b200_selfplay_cfg)) throw Error(CATTUS_B200_EINVAL, "selfplay cfg struct_size mismatch");
@@ -572,18 +592,18 @@ void match_run(cattus_b200_t* ma, cattus_b200_t* mb, const cattus_b200_selfplay_
             if (s < 2 || s > 11) throw Error(CATTUS_B200_EINVAL, "hex board_size must be 2..11");
             if (s <= 8) {
                 sp::HexRulesT<uint64_t> rules(s);
-                match_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, side_b, n, fens, moves, move_offsets, out);
+                match_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, side_b, search_batch, n, fens, moves, move_offsets, out);
             } else {
                 sp::HexRulesT<sp::u128> rules(s);
-                match_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, side_b, n, fens, moves, move_offsets, out);
+                match_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, side_b, search_batch, n, fens, moves, move_offsets, out);
             }
         } else if (cfg.game == CATTUS_B200_GAME_CHESS) {
             sp::ChessRules rules;
-            match_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), e1, e2, cfg, side_b, n,
-                        fens, moves, move_offsets, out);
+            match_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), e1, e2, cfg, side_b,
+                        search_batch, n, fens, moves, move_offsets, out);
         } else if (cfg.game == CATTUS_B200_GAME_TTT) {
             sp::TttRules rules;
-            match_rules(rules, &rules, sizeof(rules), 9u, e1, e2, cfg, side_b, n, fens, moves, move_offsets, out);
+            match_rules(rules, &rules, sizeof(rules), 9u, e1, e2, cfg, side_b, search_batch, n, fens, moves, move_offsets, out);
         } else {
             throw Error(CATTUS_B200_EINVAL, "unknown game");
         }
@@ -592,7 +612,8 @@ void match_run(cattus_b200_t* ma, cattus_b200_t* mb, const cattus_b200_selfplay_
     }
 }
 
-void dsearch_run(cattus_b200_t* m1, cattus_b200_t* m2, const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], sp::Shared& sh) {
+void dsearch_run(cattus_b200_t* m1, cattus_b200_t* m2, const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], const uint32_t search_batch[2],
+                 sp::Shared& sh) {
     try {
         if (!m1) throw Error(CATTUS_B200_EINVAL, "null evaluator handle (there is no CPU fallback)");
         Engine* e1 = m1->engine;
@@ -601,17 +622,17 @@ void dsearch_run(cattus_b200_t* m1, cattus_b200_t* m2, const cattus_b200_selfpla
             const int s = static_cast<int>(cfg.board_size);
             if (s <= 8) {
                 sp::HexRulesT<uint64_t> rules(s);
-                dsearch_run_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, params, sh);
+                dsearch_run_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, params, search_batch, sh);
             } else {
                 sp::HexRulesT<sp::u128> rules(s);
-                dsearch_run_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, params, sh);
+                dsearch_run_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), e1, e2, cfg, params, search_batch, sh);
             }
         } else if (cfg.game == CATTUS_B200_GAME_CHESS) {
             sp::ChessRules rules;
-            dsearch_run_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), e1, e2, cfg, params, sh);
+            dsearch_run_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), e1, e2, cfg, params, search_batch, sh);
         } else {
             sp::TttRules rules;
-            dsearch_run_rules(rules, &rules, sizeof(rules), 9u, e1, e2, cfg, params, sh);
+            dsearch_run_rules(rules, &rules, sizeof(rules), 9u, e1, e2, cfg, params, search_batch, sh);
         }
     } catch (const Error& e) {
         throw sp::SpError{e.code, e.what()};

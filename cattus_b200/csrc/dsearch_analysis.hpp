@@ -25,8 +25,7 @@
 namespace ds {
 
 struct AnalysisOpts {
-    uint32_t pv_max;             // principal variation plies (<= kPvMax)
-    uint32_t search_batch = 1;   // descents per minibatch under virtual loss (DESIGN.md section 15); 1: one leaf in flight
+    uint32_t pv_max;  // principal variation plies (<= kPvMax)
 };
 
 // A minibatched search's entry ends in 16 more bytes: u32 minibatches, u32 collisions (batch_expand_slot).
@@ -41,8 +40,9 @@ inline uint32_t analysis_search_batch(const cattus_b200_analysis_opts* opts) {
     return opts->search_batch ? opts->search_batch : 1u;
 }
 
-// Concurrent searches of an analysis of n positions: device_games, 0 = min(n, max_batch / search_batch).  Every slot
-// writes up to search_batch evaluator rows per wave, so device_games x search_batch above max_batch is ERANGE.
+// Concurrent searches of an analysis of n positions, or of a match of n games: device_games, 0 = min(n, max_batch /
+// search_batch).  Every slot writes up to search_batch evaluator rows per wave (a match: the larger side's), so
+// device_games x search_batch above max_batch is ERANGE.
 inline uint32_t analysis_slots(uint32_t device_games, uint32_t n, uint32_t max_batch, uint32_t search_batch) {
     if (search_batch > 1 && static_cast<uint64_t>(device_games ? device_games : 1u) * search_batch > max_batch)
         throw sp::SpError{CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(device_games) + ") x search_batch (" +
@@ -52,6 +52,13 @@ inline uint32_t analysis_slots(uint32_t device_games, uint32_t n, uint32_t max_b
                                                   std::to_string(max_batch) + ")"};
     const uint32_t want = device_games ? device_games : max_batch / search_batch;
     return std::max<uint32_t>(1, std::min<uint32_t>(want, n));
+}
+
+// Concurrent games of a self-play partition of `games` games (device_games > 0): with minibatches (search_batch > 1)
+// checked as analysis_slots checks them; with one leaf in flight the backend checks the slots against max_batch.
+inline uint32_t selfplay_slots(uint32_t device_games, uint32_t games, uint32_t max_batch, uint32_t search_batch) {
+    if (search_batch > 1) return analysis_slots(device_games, games, max_batch, search_batch);
+    return std::max<uint32_t>(1, std::min<uint32_t>(device_games, games));
 }
 
 // The history ring of a slot (dsearch.cuh allocates it): chess keeps what detect_repetition can look back into, the

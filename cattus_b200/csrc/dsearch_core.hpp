@@ -245,7 +245,8 @@ struct Cmd {
     uint32_t slot, flags, move, cur, noise_n, root_at, root_len, pad;
 };
 // Result of one finished search, written by the device into mapped host memory: header + n[max_children] u32 +
-// move[max_children] u16 (in insertion order; the host turns them into edges() order).
+// move[max_children] u16 (in insertion order; the host turns them into edges() order).  A search run in minibatches
+// (batch_expand_slot) puts its minibatch and collision counts in pad[0] / pad[1]; the one-leaf kernels leave them unset.
 struct ResultHdr {
     uint32_t slot, count, pad[2];
 };
@@ -256,8 +257,8 @@ struct AnalysisHdr {
     uint32_t slot, count, pv_len, pad;
 };
 
-// One descent of a minibatch (Params::search_batch > 1, DESIGN.md section 15), written by batch_select_slot and backed up
-// by batch_expand_slot.  Its path is Params::bpaths[slot][descent][0, depth).
+// One descent of a minibatch (Params::search_batch, DESIGN.md sections 15 and 16), written by batch_select_slot and
+// backed up by batch_expand_slot.  Its path is Params::bpaths[slot][descent][0, depth).
 enum DescentKind : uint32_t { kDescentCollision = 0, kDescentLeaf = 1, kDescentScored = 2 };
 struct BatchDescent {
     int32_t leaf;    // block of the node the descent ended on
@@ -265,6 +266,17 @@ struct BatchDescent {
     uint32_t kind;   // DescentKind
     uint32_t row;    // kDescentLeaf: the leaf's evaluator row
     float value;     // kDescentScored: repetition 0, finished position the winner's +-1 (player 1's view)
+};
+
+// Descents per minibatch of each side (indexed by SlotState::cur) and the larger of the two, which sizes each slot's
+// descent records and paths.  Assigning one L gives both sides L (analysis searches one way throughout).
+struct SearchBatch {
+    uint32_t side[2];
+    uint32_t max;
+    CB2_HD SearchBatch& operator=(uint32_t L) {
+        side[0] = side[1] = max = L;
+        return *this;
+    }
 };
 
 template <class Rules>
@@ -301,10 +313,10 @@ struct Params {
     const typename Rules::Pos* roots;  // root histories of this wave's kCmdSetRoot commands
     uint32_t analysis;                 // 1: finished searches post the AnalysisHdr layout instead of ResultHdr
     uint32_t pv_max;                   // principal variation plies to post (<= kPvMax)
-    // minibatched analysis (batch_select_slot / batch_expand_slot); all zero with one leaf in flight
-    uint32_t search_batch;      // descents per minibatch (> 1)
-    BatchDescent* descents;     // [n_slots][search_batch]
-    PathStep* bpaths;           // [n_slots][search_batch][path_cap]
+    // minibatched search (batch_select_slot / batch_expand_slot); all zero with one leaf in flight
+    SearchBatch search_batch;   // each side >= 1, max > 1
+    BatchDescent* descents;     // [n_slots][search_batch.max]
+    PathStep* bpaths;           // [n_slots][search_batch.max][path_cap]
     uint32_t* vcount;           // [n_slots][pool_words / 4]: virtual count of each child row (16-byte pool unit) of the tree
 };
 
@@ -453,11 +465,9 @@ struct Core {
     }
 
     // The finished search's root rows, for the host: calc_moves_probabilities' tail and the move choice run there.
-    CB2_HD static void post_results(const P& p, uint32_t wave, uint32_t si, uint32_t* pool, int32_t root) {
-        if (p.analysis) {
-            post_analysis(p, wave, si, pool, root);
-            return;
-        }
+    // Returns the posted entry.
+    CB2_HD static uint8_t* post_results(const P& p, uint32_t wave, uint32_t si, uint32_t* pool, int32_t root) {
+        if (p.analysis) return post_analysis(p, wave, si, pool, root);
         const int ln = lane();
         const int count = T::hdr(pool, root)->count;
         uint32_t k = 0;
@@ -476,6 +486,7 @@ struct Core {
             rn[i] = static_cast<uint32_t>(ch[i].n);
             rm[i] = static_cast<uint16_t>(move_at(pool, root, count, i));
         }
+        return e;
     }
 
     // Analysis result: every root row, and the principal variation -- from the root, repeatedly the child with the most
@@ -959,7 +970,8 @@ struct Core {
     }
 
     // ---------------------------------------------------------------- minibatches under virtual loss (DESIGN.md section 15)
-    // Analysis with search_batch = L > 1.  One wave runs one minibatch of a slot: batch_select_slot makes its
+    // Any search with search_batch[cur] = L (analysis, and self-play / match play when a side has L > 1; a side with
+    // L = 1 gets develop_tree's result).  One wave runs one minibatch of a slot: batch_select_slot makes its
     // k = min(L, sims_left) descents, batch_expand_slot backs them up once the evaluator has run.  The slot keeps
     // the number of descents in flight in path_len and its minibatch / collision counts in pad[0] / pad[1].
     //
@@ -986,13 +998,14 @@ struct Core {
         const int ln = lane();
         const uint32_t e = p.n_evals > 1 ? cur : 0u;
         const float ef = p.explore[cur];
-        const uint32_t L = p.search_batch;
+        const uint32_t L = (cur & 1u) ? p.search_batch.side[1] : p.search_batch.side[0];
+        const uint32_t stride = p.search_batch.max;
         const uint32_t k = sims_left < L ? sims_left : L;
         uint32_t* vc = p.vcount + static_cast<size_t>(si) * (p.pool_words >> 2);
-        BatchDescent* bd = p.descents + static_cast<size_t>(si) * L;
+        BatchDescent* bd = p.descents + static_cast<size_t>(si) * stride;
         uint32_t err = 0, rows = 0;
         for (uint32_t j = 0; j < k && !err; ++j) {
-            PathStep* path = p.bpaths + (static_cast<size_t>(si) * L + j) * p.path_cap;
+            PathStep* path = p.bpaths + (static_cast<size_t>(si) * stride + j) * p.path_cap;
             int32_t node = t.root;
             uint32_t depth = 0;
             for (;;) {
@@ -1088,6 +1101,7 @@ struct Core {
                 phase = kIdle;
             }
             Q.phase = phase;
+            const uint32_t L = (qc & 1u) ? p.search_batch.side[1] : p.search_batch.side[0];
             Q.path_len = left < L ? left : L;
             Q.used[qc & 1u] = t.used;
             if (t.used > Q.pad0) {
@@ -1104,7 +1118,8 @@ struct Core {
 
     // Phase 3: in descent order, a new leaf gets create_children from its evaluation, then it and every scored descent is
     // backpropagated as expand_slot / select do; a collision does nothing.  Per edge that is a sum in ascending descent
-    // order, as the sequential definition adds.  Then every virtual count of the minibatch is dropped.
+    // order, as the sequential definition adds.  Then every virtual count of the minibatch is dropped.  A root that a
+    // minibatch expands takes the host's noise sample as expand_slot's does.
     CB2_HD static void batch_expand_slot(const Rules& R, const P& p, uint32_t si, uint32_t wave) {
         SlotState& S = p.slots[si];
         const uint32_t phase0 = S.phase & 3u, cur = S.cur, k = S.path_len;
@@ -1115,14 +1130,14 @@ struct Core {
         const int ln = lane();
         const uint32_t e = p.n_evals > 1 ? cur : 0u;
         const EvalIo& io = p.eval[e];
-        const uint32_t L = p.search_batch;
+        const uint32_t stride = p.search_batch.max;
         const uint8_t root_turn = T::hdr(pool, root)->pos.turn;
         uint32_t* vc = p.vcount + static_cast<size_t>(si) * (p.pool_words >> 2);
-        const BatchDescent* bd = p.descents + static_cast<size_t>(si) * L;
-        uint32_t n_sims = 0, n_scored = 0, n_coll = 0, noise_n = 0;
+        const BatchDescent* bd = p.descents + static_cast<size_t>(si) * stride;
+        uint32_t n_sims = 0, n_scored = 0, n_coll = 0;
         for (uint32_t j = 0; j < k; ++j) {
             const BatchDescent d = bd[j];
-            const PathStep* path = p.bpaths + (static_cast<size_t>(si) * L + j) * p.path_cap;
+            const PathStep* path = p.bpaths + (static_cast<size_t>(si) * stride + j) * p.path_cap;
             if (d.kind == kDescentCollision) {
                 n_coll += 1;
                 continue;
@@ -1136,7 +1151,11 @@ struct Core {
                     const uint64_t kh = position_key(R, T::hdr(pool, d.leaf)->pos, key);
                     cache_insert(p.cache[e], key, kh, T::hdr(pool, d.leaf)->count, probs, value);
                 }
+                // the root's noise count is read only where a minibatch expands the root, rather than kept live
+                uint32_t noise_n = d.leaf == root ? p.slots[si].noise_n : 0u;
+                wsync();
                 apply_evaluation(R, p, si, cur, pool, d.leaf, root, probs, value, noise_n, 0u);  // children only: depth 0
+                if (d.leaf == root && ln == 0) p.slots[si].noise_n = noise_n;
                 v = T::hdr(pool, d.leaf)->pos.turn != 1 ? -value : value;
             } else {
                 n_scored += 1;
@@ -1148,7 +1167,7 @@ struct Core {
         }
         for (uint32_t j = 0; j < k; ++j) {
             const uint32_t depth = bd[j].depth;
-            const PathStep* path = p.bpaths + (static_cast<size_t>(si) * L + j) * p.path_cap;
+            const PathStep* path = p.bpaths + (static_cast<size_t>(si) * stride + j) * p.path_cap;
             for (uint32_t s = static_cast<uint32_t>(ln); s < depth; s += DS_LANES) vc[static_cast<uint32_t>(path[s].c_idx) >> 2] = 0u;
         }
         wsync();
@@ -1158,9 +1177,9 @@ struct Core {
         wsync();
         uint32_t phase = kRun;
         if (left == 0) {
-            uint8_t* entry = post_analysis(p, wave, si, pool, root);
-            if (ln == 0) {
-                uint32_t* counts = reinterpret_cast<uint32_t*>(entry + p.result_stride - 16u);
+            uint8_t* entry = post_results(p, wave, si, pool, root);
+            if (ln == 0) {  // the analysis entry ends in the two counts; the self-play one has them in ResultHdr::pad
+                uint32_t* counts = p.analysis ? reinterpret_cast<uint32_t*>(entry + p.result_stride - 16u) : reinterpret_cast<ResultHdr*>(entry)->pad;
                 counts[0] = minibatches;
                 counts[1] = collisions;
             }

@@ -14,6 +14,9 @@
 // With an opening source (a match between two networks, dsearch_match.hpp) game 2k + c starts from opening k instead of
 // the initial position: a kCmdSetRoot command installs the opening with its history, which the backend uploads with the
 // wave (roots_block / roots_cap).  Everything else is the self-play game loop.
+//
+// With minibatches (a side's search_batch > 1, DESIGN.md section 16) the backend runs the minibatch kernels, and each
+// finished search posts its minibatch and collision counts in ResultHdr::pad; the driver sums them per side.
 #pragma once
 
 #include <deque>
@@ -60,10 +63,10 @@ class Driver {
     // openings (optional): per opening k, the history kCmdSetRoot loads (oldest first, the opening's position last; at most
     // the backend's history ring); games 2k and 2k + 1 start there.  An empty history: the opening is not played.
     // cfg.games_num must be twice the number of openings.  Such games keep records (moves, winner, termination) but write
-    // no training data.
+    // no training data.  search_batch (optional): the backend's descents per minibatch of model 1's and model 2's searches.
     Driver(const Rules& rules, const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], Backend& be, sp::Shared& sh,
-           const std::vector<std::vector<Pos>>* openings = nullptr)
-        : R(rules), cfg_(cfg), be_(be), sh_(sh), openings_(openings) {
+           const std::vector<std::vector<Pos>>* openings = nullptr, const uint32_t* search_batch = nullptr)
+        : R(rules), cfg_(cfg), be_(be), sh_(sh), openings_(openings), batched_(search_batch && (search_batch[0] > 1 || search_batch[1] > 1)) {
         params_[0] = params[0];
         params_[1] = params[1];
         games_.resize(be.n_slots());
@@ -138,6 +141,10 @@ class Driver {
         sh_.w2 += w2_;
         sh_.d += d_;
         sh_.games += games_done_;
+        for (int s = 0; s < 2; ++s) {
+            sh_.minibatches[s] += minibatches_[s];
+            sh_.collisions[s] += collisions_[s];
+        }
         sh_.search_duration = search_duration_;
     }
 
@@ -265,6 +272,9 @@ class Driver {
         const uint32_t* rn = reinterpret_cast<const uint32_t*>(e + sizeof(ResultHdr));
         const uint16_t* rm = reinterpret_cast<const uint16_t*>(e + sizeof(ResultHdr) + 4u * be_.max_children());
         const sp::Params& P = params_[g.cur];
+        // the one-leaf kernels run a search as sim_num rounds of one descent each and post no counts
+        minibatches_[g.cur] += batched_ ? rh->pad[0] : P.sim_num;
+        collisions_[g.cur] += batched_ ? rh->pad[1] : 0u;
         std::vector<std::pair<Move, float>> probs;
         probs.reserve(count);
         uint32_t total = 0;
@@ -336,12 +346,13 @@ class Driver {
     sp::Shared& sh_;
     sp::Params params_[2];
     const std::vector<std::vector<Pos>>* openings_;
+    const bool batched_;
     std::vector<Game> games_;
     std::vector<uint8_t> cmds_[2];      // commands for each population's next wave
     std::vector<uint8_t> set_root_[2];  // kCmdSetRoot commands waiting for room in a wave's root block
     uint32_t cmd_stride_ = 0, result_stride_ = 0;
     uint32_t active_ = 0, active_pop_[2] = {0, 0};
-    uint64_t waves_ = 0, searches_ = 0;
+    uint64_t waves_ = 0, searches_ = 0, minibatches_[2] = {0, 0}, collisions_[2] = {0, 0};
     uint32_t w1_ = 0, w2_ = 0, d_ = 0, games_done_ = 0;
     double search_duration_ = 0.0, t_submit_ = 0.0, t_wait_ = 0.0, t_process_ = 0.0;
     std::vector<double> noise_;

@@ -24,8 +24,18 @@ struct MatchResult {
     std::vector<sp::GameRecord> games;     // by game index 2k + c
     uint32_t a_wins = 0, b_wins = 0, draws = 0;
     uint64_t simulations = 0, evaluations = 0;
+    uint64_t minibatches[2] = {0, 0}, collisions[2] = {0, 0};  // per side (A, B)
     double seconds = 0.0;
 };
+
+// Each side's descents per minibatch from the C ABI's options: NULL, or 0 or 1 for a side, is one leaf in flight.
+inline void match_search_batch(const cattus_b200_match_opts* opts, uint32_t out[2]) {
+    out[0] = out[1] = 1;
+    if (!opts) return;
+    if (opts->struct_size != sizeof(cattus_b200_match_opts)) throw sp::SpError{CATTUS_B200_EINVAL, "match opts struct_size mismatch"};
+    out[0] = opts->search_batch_a ? opts->search_batch_a : 1u;
+    out[1] = opts->search_batch_b ? opts->search_batch_b : 1u;
+}
 
 // The two sides' MctsParams: cfg's, with side B's sim_num / explore_factor where side_b gives them.
 inline void match_params(const cattus_b200_selfplay_cfg& cfg, const cattus_b200_match_side* side_b, sp::Params out[2]) {
@@ -81,10 +91,10 @@ std::vector<std::vector<typename Rules::Pos>> match_openings(const Rules& R, uin
 // Plays the openings' games on `be` (its slots: at most the number of games) and fills out's games and counts.
 template <class Rules, class Backend>
 void match_play(const Rules& R, const cattus_b200_selfplay_cfg& cfg, const sp::Params params[2], Backend& be,
-                const std::vector<std::vector<typename Rules::Pos>>& openings, MatchResult& out) {
+                const std::vector<std::vector<typename Rules::Pos>>& openings, MatchResult& out, const uint32_t* search_batch = nullptr) {
     const cattus_b200_selfplay_cfg mc = match_cfg(cfg, static_cast<uint32_t>(openings.size()));
     sp::Shared sh;
-    Driver<Rules, Backend> drv(R, mc, params, be, sh, &openings);
+    Driver<Rules, Backend> drv(R, mc, params, be, sh, &openings, search_batch);
     drv.run();
     out.games = std::move(sh.records);
     std::sort(out.games.begin(), out.games.end(), [](const sp::GameRecord& a, const sp::GameRecord& b) { return a.game_idx < b.game_idx; });
@@ -93,6 +103,10 @@ void match_play(const Rules& R, const cattus_b200_selfplay_cfg& cfg, const sp::P
     out.draws = sh.d;
     out.simulations = sh.simulations;
     out.evaluations = sh.evaluations;
+    for (int s = 0; s < 2; ++s) {
+        out.minibatches[s] = sh.minibatches[s];
+        out.collisions[s] = sh.collisions[s];
+    }
 }
 
 // The games a match needs slots for: two per opening that is played.
@@ -147,6 +161,13 @@ inline int match_game(const MatchResult& r, uint32_t k, cattus_b200_match_game* 
     out->winner = g.winner;
     out->termination = g.termination;
     out->n_moves = static_cast<uint32_t>(g.moves.size());
+    return CATTUS_B200_OK;
+}
+
+inline int match_batches(const MatchResult& r, uint32_t side, uint64_t* minibatches, uint64_t* collisions) {
+    if (side > 1) return CATTUS_B200_ERANGE;
+    if (minibatches) *minibatches = r.minibatches[side];
+    if (collisions) *collisions = r.collisions[side];
     return CATTUS_B200_OK;
 }
 

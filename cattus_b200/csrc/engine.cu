@@ -2273,10 +2273,32 @@ int cattus_b200_match_run(cattus_b200_t* model_a, cattus_b200_t* model_b, const 
     return guarded([&] {
         if (!cfg || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
         *out = nullptr;
+        const uint32_t one[2] = {1, 1};
         std::unique_ptr<cattus_b200_match> r(new cattus_b200_match());
-        cb2::match_run(model_a, model_b, *cfg, side_b, n, fens, moves, move_offsets, r->res);
+        cb2::match_run(model_a, model_b, *cfg, side_b, one, n, fens, moves, move_offsets, r->res);
         *out = r.release();
     });
+}
+
+int cattus_b200_match_run_opts(cattus_b200_t* model_a, cattus_b200_t* model_b, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_match_side* side_b,
+                               const cattus_b200_match_opts* opts, uint32_t n, const char* const* fens, const uint16_t* moves,
+                               const uint32_t* move_offsets, cattus_b200_match_t** out) {
+    return guarded([&] {
+        if (!cfg || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        *out = nullptr;
+        uint32_t search_batch[2];
+        try {
+            ds::match_search_batch(opts, search_batch);
+        } catch (const sp::SpError& e) {
+            throw cb2::Error(e.code, e.msg);
+        }
+        std::unique_ptr<cattus_b200_match> r(new cattus_b200_match());
+        cb2::match_run(model_a, model_b, *cfg, side_b, search_batch, n, fens, moves, move_offsets, r->res);
+        *out = r.release();
+    });
+}
+int cattus_b200_match_batches(const cattus_b200_match_t* r, uint32_t side, uint64_t* minibatches, uint64_t* collisions) {
+    return r ? ds::match_batches(r->res, side, minibatches, collisions) : CATTUS_B200_EINVAL;
 }
 
 int cattus_b200_match_summary_get(const cattus_b200_match_t* r, cattus_b200_match_summary* out) {

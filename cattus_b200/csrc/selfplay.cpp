@@ -1307,6 +1307,7 @@ static void make_dirs(const char* path) {
 
 struct cattus_b200_selfplay {
     cattus_b200_selfplay_summary summary;
+    uint64_t minibatches = 0, collisions = 0;
     std::vector<sp::GameRecord> records;
 };
 
@@ -1328,11 +1329,14 @@ static void run_games(const Rules& rules, const cattus_b200_selfplay_cfg& cfg, c
     workers[0]->run();  // the calling thread does job 0 (self_play.rs:127-137); run() itself never throws
 }
 
-static int selfplay_impl(sp::Evaluator& e1, sp::Evaluator* e2_or_null, const cattus_b200_selfplay_cfg* cfg, cattus_b200_selfplay_t** out) {
+static int selfplay_impl(sp::Evaluator& e1, sp::Evaluator* e2_or_null, const cattus_b200_selfplay_cfg* cfg, cattus_b200_selfplay_t** out,
+                         const cattus_b200_selfplay_opts* opts = nullptr) {
     try {
         if (!cfg || !out) throw sp::SpError{CATTUS_B200_EINVAL, "null argument"};
         if (cfg->struct_size != sizeof(cattus_b200_selfplay_cfg)) throw sp::SpError{CATTUS_B200_EINVAL, "selfplay cfg struct_size mismatch"};
         *out = nullptr;
+        const uint32_t L = sp::selfplay_search_batch(opts, *cfg);
+        const uint32_t search_batch[2] = {L, L};
         if (cfg->games_num % 2 != 0) throw sp::SpError{CATTUS_B200_EINVAL, "Games num should be a multiple of 2 (self_play.rs:100)"};
         if ((cfg->out_dir1 == nullptr) != (cfg->out_dir2 == nullptr)) throw sp::SpError{CATTUS_B200_EINVAL, "out_dir1 and out_dir2 must both be set or both NULL"};
         const sp::Params p = sp::parse_params(cfg);
@@ -1361,7 +1365,7 @@ static int selfplay_impl(sp::Evaluator& e1, sp::Evaluator* e2_or_null, const cat
             // trees in HBM, one warp per game (dsearch_core.hpp): needs the B200 evaluator's device buffers
             if (!e1.async_handle || (e2_or_null && !e2_or_null->async_handle))
                 throw sp::SpError{CATTUS_B200_EINVAL, "device_games needs the B200 evaluator (cattus_b200_selfplay_run); a callback evaluator has no device buffers"};
-            cb2::dsearch_run(e1.async_handle, e2_or_null ? e2_or_null->async_handle : nullptr, *cfg, params, sh);
+            cb2::dsearch_run(e1.async_handle, e2_or_null ? e2_or_null->async_handle : nullptr, *cfg, params, search_batch, sh);
         } else if (cfg->game == CATTUS_B200_GAME_HEX) {
             if (cfg->board_size <= 8) {
                 sp::HexRulesT<uint64_t> rules(static_cast<int>(cfg->board_size));
@@ -1396,6 +1400,9 @@ static int selfplay_impl(sp::Evaluator& e1, sp::Evaluator* e2_or_null, const cat
         s.search_duration = sh.search_duration;
         s.eval_wait_seconds = sh.eval_wait;
         s.speculative_evaluations = sh.speculative;
+        // the host-tree driver keeps one leaf in flight: a round per simulation
+        r->minibatches = cfg->device_games ? sh.minibatches[0] + sh.minibatches[1] : sh.simulations;
+        r->collisions = sh.collisions[0] + sh.collisions[1];
         r->records = std::move(sh.records);
         std::sort(r->records.begin(), r->records.end(), [](const sp::GameRecord& a, const sp::GameRecord& b) { return a.game_idx < b.game_idx; });
         *out = r.release();
@@ -1422,6 +1429,11 @@ static int engine_eval_thunk(void* ctx, const uint64_t* planes, const uint8_t* l
 extern "C" {
 
 int cattus_b200_selfplay_run(cattus_b200_t* model1, cattus_b200_t* model2, const cattus_b200_selfplay_cfg* cfg, cattus_b200_selfplay_t** out) {
+    return cattus_b200_selfplay_run_opts(model1, model2, cfg, nullptr, out);
+}
+
+int cattus_b200_selfplay_run_opts(cattus_b200_t* model1, cattus_b200_t* model2, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_selfplay_opts* opts,
+                                  cattus_b200_selfplay_t** out) {
     if (!model1) {
         g_sp_error = "null evaluator handle (there is no CPU fallback)";
         return CATTUS_B200_EINVAL;
@@ -1440,7 +1452,7 @@ int cattus_b200_selfplay_run(cattus_b200_t* model1, cattus_b200_t* model2, const
         e2.max_rows = handle_max_batch(model2);
         if (cfg && cfg->leaf_queue) e2.leaf_handle = model2;
     }
-    return selfplay_impl(e1, two ? &e2 : nullptr, cfg, out);
+    return selfplay_impl(e1, two ? &e2 : nullptr, cfg, out, opts);
 }
 
 int cattus_b200_selfplay_run_with(cattus_b200_eval_fn eval1, void* ctx1, cattus_b200_eval_fn eval2, void* ctx2, const cattus_b200_selfplay_cfg* cfg,
@@ -1463,6 +1475,13 @@ int cattus_b200_selfplay_run_with(cattus_b200_eval_fn eval1, void* ctx1, cattus_
 int cattus_b200_selfplay_summary_get(const cattus_b200_selfplay_t* r, cattus_b200_selfplay_summary* out) {
     if (!r || !out) return CATTUS_B200_EINVAL;
     *out = r->summary;
+    return CATTUS_B200_OK;
+}
+
+int cattus_b200_selfplay_batches(const cattus_b200_selfplay_t* r, uint64_t* minibatches, uint64_t* collisions) {
+    if (!r) return CATTUS_B200_EINVAL;
+    if (minibatches) *minibatches = r->minibatches;
+    if (collisions) *collisions = r->collisions;
     return CATTUS_B200_OK;
 }
 

@@ -107,6 +107,17 @@ inline Params parse_params(const cattus_b200_selfplay_cfg* cfg) {
     return p;
 }
 
+// Descents per minibatch of cattus_b200_selfplay_run_opts: NULL, 0 or 1 is one leaf in flight.  Minibatches run on the
+// device-resident search only.
+inline uint32_t selfplay_search_batch(const cattus_b200_selfplay_opts* opts, const cattus_b200_selfplay_cfg& cfg) {
+    if (!opts) return 1;
+    if (opts->struct_size != sizeof(cattus_b200_selfplay_opts)) throw SpError{CATTUS_B200_EINVAL, "selfplay opts struct_size mismatch"};
+    const uint32_t L = opts->search_batch ? opts->search_batch : 1u;
+    if (L > 1 && !cfg.device_games)
+        throw SpError{CATTUS_B200_EINVAL, "search_batch > 1 needs the device-resident search (device_games > 0); the host-tree driver keeps one leaf in flight"};
+    return L;
+}
+
 // How a game of the device-resident driver ended (GameRecord::termination; the host driver leaves it 0)
 enum Termination : uint8_t { kEndRules = 1, kEndRepetition = 2, kEndMaxMoves = 3 };
 
@@ -123,6 +134,7 @@ struct Shared {
     // merged from the workers' private counters when they finish (no shared cache line on the per-simulation path)
     uint64_t simulations = 0, searches = 0, evaluations = 0, cache_hits = 0, cache_misses = 0, batches = 0, terminal = 0, speculative = 0;
     uint32_t w1 = 0, w2 = 0, d = 0, games = 0;
+    uint64_t minibatches[2] = {0, 0}, collisions[2] = {0, 0};  // device search, per model (1, 2): rounds of descents, collided descents
     std::atomic<uint32_t> next_game{0};
     std::mutex mu;  // records, search_duration, first error
     std::vector<GameRecord> records;

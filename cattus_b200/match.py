@@ -22,7 +22,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 from dataclasses import dataclass
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Tuple
 
 from . import _lib
 from .analysis import encode_positions
@@ -101,6 +101,10 @@ class MatchResult:
     simulations: int
     evaluations: int
     seconds: float
+    # per side (A, B): rounds of descents (one leaf in flight: one per simulation) and descents that collided with an
+    # earlier one of their minibatch
+    minibatches: Tuple[int, int] = (0, 0)
+    collisions: Tuple[int, int] = (0, 0)
 
     @property
     def skipped(self) -> int:
@@ -120,8 +124,9 @@ def side_struct(sim_num_b: Optional[int], explore_factor_b: Optional[float]):
     return s
 
 
-def collect(summary_get, opening_status, game_get, game_moves, h) -> MatchResult:
-    """Reads a match result through its accessors (the library's, or the test emulation's of the same signatures)."""
+def collect(summary_get, opening_status, game_get, game_moves, h, batches=None) -> MatchResult:
+    """Reads a match result through its accessors (the library's, or the test emulation's of the same signatures);
+    `batches` (optional) reads each side's minibatch and collision counts."""
     s = _lib.MatchSummary()
     s.struct_size = C.sizeof(_lib.MatchSummary)
     if summary_get(h, C.byref(s)) != 0:
@@ -142,24 +147,49 @@ def collect(summary_get, opening_status, game_get, game_moves, h) -> MatchResult
         if mv is None or game_moves(h, k, mv, g.n_moves) != 0:
             raise RuntimeError(f"match game {k} cannot be read")
         games.append(MatchGame(int(g.opening), bool(g.a_is_player1), int(g.winner) or None, TERMINATIONS[g.termination], list(mv)[: g.n_moves]))
-    return MatchResult(games, status, int(s.a_wins), int(s.b_wins), int(s.draws), list(s.pairs), int(s.simulations), int(s.evaluations),
-                       float(s.seconds))
+    res = MatchResult(games, status, int(s.a_wins), int(s.b_wins), int(s.draws), list(s.pairs), int(s.simulations), int(s.evaluations),
+                      float(s.seconds))
+    if batches is not None:
+        mb, co = [], []
+        for side in (0, 1):
+            m, c = C.c_uint64(), C.c_uint64()
+            if batches(h, side, C.byref(m), C.byref(c)) != 0:
+                raise RuntimeError("match minibatch counts cannot be read")
+            mb.append(int(m.value))
+            co.append(int(c.value))
+        res.minibatches, res.collisions = tuple(mb), tuple(co)
+    return res
+
+
+def opts_struct(search_batch: Optional[int], search_batch_b: Optional[int]):
+    """cattus_b200_match_opts: search_batch for both sides, search_batch_b overriding B's; None when neither is given."""
+    if search_batch is None and search_batch_b is None:
+        return None
+    o = _lib.MatchOpts()
+    o.struct_size = C.sizeof(_lib.MatchOpts)
+    o.search_batch_a = int(search_batch or 1)
+    o.search_batch_b = int(search_batch_b if search_batch_b is not None else (search_batch or 1))
+    return o
 
 
 def play(model_a, model_b, game: str, openings: Sequence, cfg: dict, sim_num_b: Optional[int] = None,
-         explore_factor_b: Optional[float] = None) -> MatchResult:
+         explore_factor_b: Optional[float] = None, search_batch: Optional[int] = None, search_batch_b: Optional[int] = None) -> MatchResult:
     """model_a / model_b: CudaNetworks of the game (any precision each); model_b None or model_a: one handle, one
-    evaluator and one cache.  Raises CattusB200Error (EINVAL for a bad FEN or an illegal move, naming the opening index;
-    ERANGE when the tree memory runs out)."""
+    evaluator and one cache.  search_batch: descents per minibatch under virtual loss of both sides (DESIGN.md section
+    16; None or 1: one leaf in flight, the reference's search); search_batch_b overrides B's.  A side with L > 1 does not
+    play the reference's games.  Raises CattusB200Error (EINVAL for a bad FEN or an illegal move, naming the opening
+    index; ERANGE when the tree memory runs out or device_games x L exceeds a model's max_batch)."""
     lib = _lib.load()
     c = SelfPlayRunner(game, cfg)._fill(2, None, None, False, 0, 1)
     n, fa, ma, oa = encode_positions(game, openings)
     side = side_struct(sim_num_b, explore_factor_b)
+    opts = opts_struct(search_batch, search_batch_b)
     hb = model_b._h if (model_b is not None and model_b is not model_a) else None
     h = C.c_void_p()
-    _lib.check(lib.cattus_b200_match_run(model_a._h, hb, C.byref(c), C.byref(side) if side is not None else None, n, fa, ma, oa, C.byref(h)))
+    _lib.check(lib.cattus_b200_match_run_opts(model_a._h, hb, C.byref(c), C.byref(side) if side is not None else None,
+                                              C.byref(opts) if opts is not None else None, n, fa, ma, oa, C.byref(h)))
     try:
         return collect(lib.cattus_b200_match_summary_get, lib.cattus_b200_match_opening_status, lib.cattus_b200_match_game_get,
-                       lib.cattus_b200_match_game_moves, h)
+                       lib.cattus_b200_match_game_moves, h, lib.cattus_b200_match_batches)
     finally:
         lib.cattus_b200_match_free(h)

@@ -2,13 +2,15 @@
 
     python -m cattus_b200.play_match --model-a A.cb2 --model-b B.cb2 --config-file cfg.json [--game chess] \\
         [--precision-a bf16|fp8] [--precision-b bf16|fp8] [--sim-num-b N] [--explore-factor-b X] \\
-        (--openings FILE | --pairs N) [--out games.jsonl] [--pgn games.pgn]
+        [--search-batch L] [--search-batch-b L] (--openings FILE | --pairs N) [--out games.jsonl] [--pgn games.pgn]
 
 Each opening is played twice, A as player 1 in the first game and B in the second.  --model-b defaults to --model-a,
 so `--precision-b fp8` alone plays a blob's bf16 against its FP8 handle.  --sim-num-b / --explore-factor-b give B its
 own search settings (a search-odds match); everything else comes from cfg.json, the self-play config: "mcts" (sim_num,
 explore_factor, temperature_policy, prior noise, cache_size), "seed", "max_moves" and the device_* keys; "model.batch_size"
-sizes the evaluators (default 4096).
+sizes the evaluators (default 4096).  --search-batch L runs both sides' searches in minibatches of L descents under
+virtual loss (DESIGN.md section 16), --search-batch-b B's alone: a side with L > 1 does not play the reference's search,
+so `--search-batch-b 64` against the same net measures what the minibatches cost in games.
 
 --openings: chess lines are EPD records (the four FEN fields, operations ignored), `<FEN> [moves <LAN> ...]` or
 `startpos [moves ...]`; hex and tic-tac-toe lines are cell indices (`startpos` or an empty move list: the initial
@@ -16,7 +18,8 @@ position).  Blank lines and lines starting with # are skipped.  Without --openin
 --pairs times.
 
 Output: one JSON line per game to --out (default stdout), then a summary line on stderr (W/D/L from A's side, the
-pentanomial counts, score, Elo with its 95 % interval, games/s and simulations/s).  --pgn writes the chess games.
+pentanomial counts, score, Elo with its 95 % interval, games/s, simulations/s and each side's minibatches and
+collisions).  --pgn writes the chess games.
 """
 from __future__ import annotations
 
@@ -71,6 +74,8 @@ def main(argv=None) -> int:
     ap.add_argument("--precision-b", default="bf16", choices=("bf16", "fp8"))
     ap.add_argument("--sim-num-b", type=int)
     ap.add_argument("--explore-factor-b", type=float)
+    ap.add_argument("--search-batch", type=int, help="descents per minibatch of both sides (default 1: one leaf in flight)")
+    ap.add_argument("--search-batch-b", type=int, help="descents per minibatch of B (default: --search-batch)")
     ap.add_argument("--config-file", required=True, type=Path)
     ap.add_argument("--game", default="chess")
     src = ap.add_mutually_exclusive_group(required=True)
@@ -93,10 +98,10 @@ def main(argv=None) -> int:
     net_game = {v: k for k, v in _lib.GAME_IDS.items()}[game_id]
     with CudaNetwork(args.model_a, net_game, device=args.device, batch_size=batch, n_streams=1, precision=args.precision_a) as na:
         if model_b == args.model_a and args.precision_b == args.precision_a:
-            res = play(na, None, args.game, openings, cfg, args.sim_num_b, args.explore_factor_b)
+            res = play(na, None, args.game, openings, cfg, args.sim_num_b, args.explore_factor_b, args.search_batch, args.search_batch_b)
         else:
             with CudaNetwork(model_b, net_game, device=args.device, batch_size=batch, n_streams=1, precision=args.precision_b) as nb:
-                res = play(na, nb, args.game, openings, cfg, args.sim_num_b, args.explore_factor_b)
+                res = play(na, nb, args.game, openings, cfg, args.sim_num_b, args.explore_factor_b, args.search_batch, args.search_batch_b)
     out = args.out.open("w") if args.out else sys.stdout
     try:
         for k, st in enumerate(res.opening_status):
@@ -120,7 +125,8 @@ def main(argv=None) -> int:
                "pentanomial": res.pairs, "score": None if e is None else round(e.score, 6),
                "elo": None if e is None else fmt_elo(e.elo), "elo_95": None if e is None else [fmt_elo(e.lo), fmt_elo(e.hi)],
                "seconds": round(res.seconds, 3), "games_per_s": round(len(res.games) / max(res.seconds, 1e-9), 3),
-               "sims_per_s": round(res.simulations / max(res.seconds, 1e-9), 1)}
+               "sims_per_s": round(res.simulations / max(res.seconds, 1e-9), 1), "minibatches": list(res.minibatches),
+               "collisions": list(res.collisions)}
     print(json.dumps(summary), file=sys.stderr)
     return 0
 

@@ -13,10 +13,14 @@ invokes it (training/cattus_train/train_process.py:159-170, :341-352):
   and `seed` select this backend's many-games-per-thread arrangement (default 64 games per worker thread);
 * with few games per worker thread (`games_num / threads` <= 96) `speculate` defaults on: likely next leaves are evaluated
   ahead into the value-function cache in the otherwise nearly empty batches -- same games, several times fewer round trips;
+* the optional top-level key `search_batch` L > 1 runs every search in minibatches of L descents under virtual loss on
+  the device-resident search (DESIGN.md section 16): a hundred games then fill the evaluator's batch.  Such games are not
+  the reference's; `device_games` defaults to min(games_num, 4096 / L) and the evaluator's batch holds device_games x L;
 * `.traindata` files are byte-for-byte what the reference's serializers write (hex, tic-tac-toe and chess:
   serialize/{hex,ttt,chess}.rs), named `{game_idx:08}_{pos_idx:03}`;
 * the summary file has the reference's layout (:131-149): player1_wins, player2_wins, draws and the metric keys the
-  trainer reads -- model.activation_count, model.run_duration, mcts.search_duration, cache.hits, cache.misses.
+  trainer reads -- model.activation_count, model.run_duration, mcts.search_duration, cache.hits, cache.misses -- and
+  selfplay.minibatches / selfplay.collisions among the others.
 
 With `torchrun` / `--gpus N` style partitioning use `--first-game r --game-stride n --device r` per process.
 """
@@ -77,6 +81,9 @@ def main(argv=None) -> int:
     # their own (same games either way).  Small jobs keep their trees on the host, where speculative rows hide the latency.
     with open(args.model1_path, "rb") as f:
         filters = struct.unpack("<16I", f.read(64))[6]
+    search_batch = int(cfg.get("search_batch", 1) or 1)
+    if "device_games" not in cfg and search_batch > 1:  # minibatches run on the device-resident search only
+        cfg["device_games"] = max(1, min(args.games_num, 4096 // search_batch))
     if "device_games" not in cfg and args.games_num >= 2048:
         cfg["device_games"] = min(args.games_num, 4096 if filters >= 64 else 16384)
     device_games = int(cfg.get("device_games", 0))
@@ -88,7 +95,8 @@ def main(argv=None) -> int:
     if (cfg.get("mcts") or {}).get("cache_size"):
         cfg.setdefault("speculate", min(31, 192 // slots) if slots <= 96 else 0)
     cfg.setdefault("groups_per_thread", 2)  # a worker simulates one half of its games while the other half's leaves are on the GPU
-    max_batch = max(int(cfg["model"].get("batch_size", 64)), min(4096, int(cfg["games_per_thread"])), 256 if cfg.get("speculate") else 1, device_games)
+    max_batch = max(int(cfg["model"].get("batch_size", 64)), min(4096, int(cfg["games_per_thread"])), 256 if cfg.get("speculate") else 1,
+                    device_games * search_batch)
     kw = dict(device=device, batch_size=max_batch, n_streams=int(inference.get("streams", 4)), precision=inference.get("precision", "bf16"))
     if args.summary_file is not None and args.summary_file.exists():
         raise SystemExit(f"{args.summary_file} exists")  # File::create_new (self_play_cmd.rs:150)

@@ -120,6 +120,13 @@ class SelfPlayRunner:
         c.device_waves_in_flight = int(cfg.get("device_waves_in_flight", 0))
         c.seed = int(cfg.get("seed", 0)) & 0xFFFFFFFFFFFFFFFF
         self._c = c
+        # descents per minibatch under virtual loss (DESIGN.md section 16); absent or 1: one leaf in flight, the reference's
+        # search.  Needs device_games > 0, and its games are not the reference's.
+        self._opts = None
+        if "search_batch" in cfg:
+            self._opts = _lib.SelfPlayOpts()
+            self._opts.struct_size = C.sizeof(_lib.SelfPlayOpts)
+            self._opts.search_batch = int(cfg["search_batch"])
 
     def _fill(self, games_num, out_dir1, out_dir2, keep_records, first_game, game_stride):
         c = self._c
@@ -138,13 +145,16 @@ class SelfPlayRunner:
         c = self._fill(games_num, out_dir1, out_dir2, keep_records, first_game, game_stride)
         h = C.c_void_p()
         h2 = model2._h if (model2 is not None and model2 is not model1) else None
-        _check(self._lib, self._lib.cattus_b200_selfplay_run(model1._h, h2, C.byref(c), C.byref(h)))
+        opts = C.byref(self._opts) if self._opts is not None else None
+        _check(self._lib, self._lib.cattus_b200_selfplay_run_opts(model1._h, h2, C.byref(c), opts, C.byref(h)))
         return self._collect(h, keep_records)
 
     def run_with(self, eval1: Callable, eval2: Optional[Callable], games_num: int, out_dir1=None, out_dir2=None, *,
                  keep_records: bool = False, first_game: int = 0, game_stride: int = 1):
         """eval(planes u64 [n, words], n) -> (list of n probability arrays over the legal moves ascending, values[n]);
         for chess eval(planes, n, legal u8 [n, 235]) with the legal-move bitmaps over the nn indices."""
+        if self._opts is not None and self._opts.search_batch > 1:
+            raise SelfPlayError("search_batch > 1 needs the device-resident search of generate_data (device_games > 0)")
         c = self._fill(games_num, out_dir1, out_dir2, keep_records, first_game, game_stride)
         g, s = parse_game(self.game)
         chess = g == _lib.GAME_CHESS
@@ -169,6 +179,8 @@ class SelfPlayRunner:
         try:
             s = SelfPlaySummary()
             _check(lib, lib.cattus_b200_selfplay_summary_get(h, C.byref(s)))
+            mb, co = C.c_uint64(), C.c_uint64()
+            _check(lib, lib.cattus_b200_selfplay_batches(h, C.byref(mb), C.byref(co)))
             summary = {
                 "player1_wins": s.player1_wins, "player2_wins": s.player2_wins, "draws": s.draws,
                 "metrics": {
@@ -178,6 +190,7 @@ class SelfPlayRunner:
                     "selfplay.evaluations": s.evaluations, "selfplay.terminal_leaves": s.terminal_leaves,
                     "selfplay.seconds": s.seconds, "selfplay.eval_wait_seconds": s.eval_wait_seconds,
                     "selfplay.speculative_evaluations": s.speculative_evaluations,
+                    "selfplay.minibatches": mb.value, "selfplay.collisions": co.value,
                     "selfplay.sims_per_sec": (s.simulations / s.seconds) if s.seconds > 0 else 0.0,
                 },
             }

@@ -81,7 +81,26 @@ typedef struct cattus_b200_match_game {
 int cattus_b200_match_run(cattus_b200_t* model_a, cattus_b200_t* model_b, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_match_side* side_b,
                           uint32_t n, const char* const* fens, const uint16_t* moves, const uint32_t* move_offsets, cattus_b200_match_t** out);
 
+/* Options of cattus_b200_match_run_opts (struct_size = sizeof, checked for equality: EINVAL otherwise). */
+typedef struct cattus_b200_match_opts {
+    uint32_t struct_size;
+    uint32_t search_batch_a; /* descents per minibatch under virtual loss of A's searches (DESIGN.md section 16); 0 or 1: one leaf in flight */
+    uint32_t search_batch_b; /* the same for B */
+} cattus_b200_match_opts;
+
+/* cattus_b200_match_run with options; opts NULL is cattus_b200_match_run.  A side with search_batch L > 1 searches in
+ * minibatches of L descents under virtual loss (see cattus_b200_selfplay_run_opts): its games are deterministic but are
+ * NOT the reference's games, so a match between L = 1 and L > 1 of the same net measures what the minibatches cost in
+ * games.  device_games x the larger L above either model's max_batch is ERANGE; device_games 0 takes
+ * min(2n, max_batch / the larger L). */
+int cattus_b200_match_run_opts(cattus_b200_t* model_a, cattus_b200_t* model_b, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_match_side* side_b,
+                               const cattus_b200_match_opts* opts, uint32_t n, const char* const* fens, const uint16_t* moves,
+                               const uint32_t* move_offsets, cattus_b200_match_t** out);
+
 int cattus_b200_match_summary_get(const cattus_b200_match_t* r, cattus_b200_match_summary* out);
+/* side 0 = A, 1 = B (ERANGE otherwise): that side's rounds of descents over all its searches (one leaf in flight: one
+ * per simulation) and its descents that collided with an earlier one of their minibatch. */
+int cattus_b200_match_batches(const cattus_b200_match_t* r, uint32_t side, uint64_t* minibatches, uint64_t* collisions);
 /* status of opening k: 0 played; 1 / 2 already won by that player, 3 already drawn -- not played */
 int cattus_b200_match_opening_status(const cattus_b200_match_t* r, uint32_t k, uint32_t* status);
 /* The games played, by game index (opening, then colour); summary.games of them. */

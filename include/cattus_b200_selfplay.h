@@ -116,7 +116,26 @@ int cattus_b200_selfplay_run(cattus_b200_t* model1, cattus_b200_t* model2, const
 int cattus_b200_selfplay_run_with(cattus_b200_eval_fn eval1, void* ctx1, cattus_b200_eval_fn eval2, void* ctx2,
                                   const cattus_b200_selfplay_cfg* cfg, cattus_b200_selfplay_t** out);
 
+/* Options of cattus_b200_selfplay_run_opts (struct_size = sizeof, checked for equality: EINVAL otherwise). */
+typedef struct cattus_b200_selfplay_opts {
+    uint32_t struct_size;
+    uint32_t search_batch; /* descents per minibatch under virtual loss (DESIGN.md sections 15 and 16); 0 or 1: one leaf in flight */
+} cattus_b200_selfplay_opts;
+
+/* cattus_b200_selfplay_run with options; opts NULL is cattus_b200_selfplay_run.  With search_batch L > 1 every search of
+ * both models runs in minibatches: L descents in order on a frozen tree under virtual loss, then their leaves are
+ * evaluated together and backed up in descent order, so that a few games fill the evaluator's batch.  Such games are
+ * deterministic but are NOT the reference's games (a minibatched search is not MctsPlayer's); each game's random stream,
+ * the temperature policy, root noise, tree reuse, repetition, max_moves and the .traindata format are unchanged, and
+ * `simulations` still counts sim_num per search.  L > 1 needs the device-resident search (device_games > 0: EINVAL
+ * otherwise); device_games x L above either model's max_batch is ERANGE. */
+int cattus_b200_selfplay_run_opts(cattus_b200_t* model1, cattus_b200_t* model2, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_selfplay_opts* opts,
+                                  cattus_b200_selfplay_t** out);
+
 int cattus_b200_selfplay_summary_get(const cattus_b200_selfplay_t* r, cattus_b200_selfplay_summary* out);
+/* Over all searches of the call: rounds of descents (one leaf in flight: one per simulation) and descents that ended on
+ * a leaf an earlier descent of their minibatch had claimed (not simulations; 0 with one leaf in flight). */
+int cattus_b200_selfplay_batches(const cattus_b200_selfplay_t* r, uint64_t* minibatches, uint64_t* collisions);
 /* Number of games played by this call and, for the k-th of them (k in 0..n), its index / winner (0 none, 1, 2)
  * / move count. */
 int cattus_b200_selfplay_game_count(const cattus_b200_selfplay_t* r, uint32_t* n);
