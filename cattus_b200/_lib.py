@@ -126,6 +126,32 @@ class MatchGame(C.Structure):
     _fields_ = [(n, C.c_uint32) for n in ("struct_size", "opening", "a_is_player1", "winner", "termination", "n_moves")]
 
 
+class SessionOpts(C.Structure):
+    """cattus_b200_session_opts (include/cattus_b200_session.h)."""
+    _fields_ = [("struct_size", C.c_uint32), ("search_batch", C.c_uint32), ("tree_kwords", C.c_uint32)]
+
+
+class SessionLimits(C.Structure):
+    """cattus_b200_session_limits (include/cattus_b200_session.h)."""
+    _fields_ = [("struct_size", C.c_uint32), ("nodes", C.c_uint32), ("minibatches", C.c_uint32), ("pad", C.c_uint32), ("deadline_us", C.c_uint64)]
+
+
+class SessionSnapshot(C.Structure):
+    """cattus_b200_session_snapshot (include/cattus_b200_session.h)."""
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("valid", C.c_uint32), ("searching", C.c_uint32), ("simulations", C.c_uint32), ("minibatches", C.c_uint32),
+        ("collisions", C.c_uint32), ("best_move", C.c_uint16), ("pv_len", C.c_uint16), ("q", C.c_float), ("seconds", C.c_double),
+        ("pv", C.c_uint16 * 16),
+    ]
+
+
+class SessionStats(C.Structure):
+    """cattus_b200_session_stats (include/cattus_b200_session.h)."""
+    _fields_ = [("struct_size", C.c_uint32), ("stop_reason", C.c_uint32), ("reused_visits", C.c_uint32), ("pad", C.c_uint32), ("seconds", C.c_double)]
+
+
+SESSION_RUNNING = 1
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 _H = C.c_void_p
 _u16p = C.POINTER(C.c_uint16)
@@ -187,6 +213,16 @@ SYMBOLS = {
     "cattus_b200_match_game_get": (C.c_int, [_H, C.c_uint32, C.POINTER(MatchGame)]),
     "cattus_b200_match_game_moves": (C.c_int, [_H, C.c_uint32, _u16p, C.c_uint32]),
     "cattus_b200_match_free": (None, [_H]),
+    # include/cattus_b200_session.h
+    "cattus_b200_session_create": (C.c_int, [_H, C.POINTER(SelfPlayCfg), C.POINTER(SessionOpts), C.POINTER(_H)]),
+    "cattus_b200_session_set_position": (C.c_int, [_H, C.c_char_p, _u16p, C.c_uint32]),
+    "cattus_b200_session_new_game": (C.c_int, [_H]),
+    "cattus_b200_session_go": (C.c_int, [_H, C.POINTER(SessionLimits)]),
+    "cattus_b200_session_stop": (C.c_int, [_H]),
+    "cattus_b200_session_info": (C.c_int, [_H, C.POINTER(SessionSnapshot)]),
+    "cattus_b200_session_wait": (C.c_int, [_H, C.c_uint32, C.POINTER(_H)]),
+    "cattus_b200_session_result_stats": (C.c_int, [_H, C.POINTER(SessionStats)]),
+    "cattus_b200_session_destroy": (None, [_H]),
     # include/cattus_b200_chess.h
     "cattus_b200_chess_position": (C.c_int, [C.c_char_p, _u16p, C.c_uint32, C.POINTER(ChessInfo)]),
     "cattus_b200_chess_perft": (C.c_int, [C.c_char_p, C.c_uint32, C.POINTER(C.c_uint64)]),

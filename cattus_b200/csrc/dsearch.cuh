@@ -13,6 +13,7 @@
 #include "dsearch_api.hpp"
 #include "dsearch_host.hpp"
 #include "dsearch_match.hpp"
+#include "dsearch_session.hpp"
 #include "engine.hpp"
 
 namespace cb2 {
@@ -32,6 +33,17 @@ __global__ void __launch_bounds__(128) ds_begin_kernel(ds::Params<Rules> p) {
     if (warp >= n_cmds) return;
     decltype(auto) R = ds::RulesRef<Rules>::get(p.rules);
     ds::Core<Rules>::begin_slot(R, p, warp, wave);
+}
+
+// A session's begin (Core::begin_slot<true>, DESIGN.md section 17): its wave graph takes this one instead of ds_begin_kernel.
+template <class Rules>
+__global__ void __launch_bounds__(128) ds_begin_session_kernel(ds::Params<Rules> p) {
+    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const uint32_t* hdr = reinterpret_cast<const uint32_t*>(p.cmds);
+    const uint32_t n_cmds = hdr[0], wave = hdr[1];
+    if (warp >= n_cmds) return;
+    decltype(auto) R = ds::RulesRef<Rules>::get(p.rules);
+    ds::Core<Rules>::template begin_slot<true>(R, p, warp, wave);
 }
 
 template <class Rules>
@@ -93,11 +105,14 @@ class DsCudaBackend {
     // `roots_cap` > 0 adds the per-wave root upload of kCmdSetRoot (analysis, matches from openings): up to that many
     // history positions per wave.  `search_batch` (optional) is each side's descents per minibatch: when one of them is
     // above 1 the waves run the minibatch kernels.  `analysis` (optional) switches the finished searches to the analysis
-    // result layout.  Without them everything is the self-play arrangement.
+    // result layout.  `session_kwords` (optional, with analysis and search_batch > 1: a session, dsearch_session.hpp) makes
+    // one slot whose tree buffers hold that many kwords (0: the most the tree address space allows), takes a free
+    // evaluator lane or fails, and adds the session's control words and snapshot in mapped memory.  Without them
+    // everything is the self-play arrangement.
     DsCudaBackend(const void* rules_blob, size_t rules_bytes, uint32_t max_children, Engine* e1, Engine* e2, const cattus_b200_selfplay_cfg& cfg,
                   const sp::Params params[2], uint32_t n_slots, uint32_t roots_cap = 0, const uint32_t* search_batch = nullptr,
-                  const ds::AnalysisOpts* analysis = nullptr)
-        : max_children_(max_children), n_slots_(n_slots) {
+                  const ds::AnalysisOpts* analysis = nullptr, const uint32_t* session_kwords = nullptr)
+        : max_children_(max_children), n_slots_(n_slots), device_(e1->device()), session_(session_kwords != nullptr) {
         if (search_batch) {
             side_batch_[0] = std::max<uint32_t>(1, search_batch[0]);
             side_batch_[1] = std::max<uint32_t>(1, search_batch[1]);
@@ -115,7 +130,10 @@ class DsCudaBackend {
         try {
             // evaluator lanes: one per population and evaluator; a second population needs a second free stream in every evaluator
             for (uint32_t e = 0; e < n_evals_; ++e) {
-                pop_[0].io[e] = eng_[e]->resident_acquire(true);
+                pop_[0].io[e] = eng_[e]->resident_acquire(!session_);
+                if (pop_[0].io[e].lane < 0)
+                    throw Error(CATTUS_B200_EINVAL, "session: the model has no free evaluator lane; a session holds one for its lifetime, so create "
+                                                    "the model with n_streams >= 2");
                 if (search_batch_ > 1 && pop_[0].io[e].max_batch < static_cast<uint64_t>(n_slots) * search_batch_)
                     throw Error(CATTUS_B200_ERANGE, "device search: device_games (" + std::to_string(n_slots) + ") x search_batch (" +
                                                         std::to_string(search_batch_) + ") exceeds the evaluator's max_batch (" +
@@ -157,7 +175,14 @@ class DsCudaBackend {
             const uint64_t budget = static_cast<uint64_t>(static_cast<double>(free_b) * 0.7) / (static_cast<uint64_t>(n_slots) * 3u * 4u);
             if (!cfg.device_tree_kwords) want = std::min(want, budget);
             want &= ~static_cast<uint64_t>(3);
-            if (want > budget || want < per_search + per_search / 4 || want >= (static_cast<uint64_t>(0xFFFFFE) << 2))
+            if (session_) {  // sized by the session's options, not by sim_num (a session's searches have no fixed size)
+                try {
+                    want = ds::session_tree_words(*session_kwords, static_cast<unsigned long long>(search_batch_) * T::block_words(static_cast<int>(max_children)));
+                } catch (const sp::SpError& se) {
+                    throw Error(se.code, se.msg);
+                }
+            }
+            if (want > budget || (!session_ && want < per_search + per_search / 4) || want >= (static_cast<uint64_t>(0xFFFFFE) << 2))
                 throw Error(CATTUS_B200_ENOMEM, "device search: " + std::to_string(n_slots) + " games x 3 tree buffers of " + std::to_string(want) +
                                                     " words do not fit the device (or its 2^26-word tree address space); lower device_games");
             pool_words_ = static_cast<uint32_t>(want);
@@ -194,7 +219,13 @@ class DsCudaBackend {
             std::memset(h_status_, 0, 64 * n_bufs_);
             events_.resize(n_bufs_);
             for (auto& ev : events_) CB2_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            const uint32_t begin_lead = std::getenv("CATTUS_B200_DSEARCH_SERIAL_BEGIN") ? 0u : 1u;
+            // a session's begin runs before the first minibatch of its search, in the same wave
+            const uint32_t begin_lead = (session_ || std::getenv("CATTUS_B200_DSEARCH_SERIAL_BEGIN")) ? 0u : 1u;
+            if (session_) {
+                CB2_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&h_session_), sizeof(ds::SessionCtl) + ds::kSnapshotHdr + result_stride_, cudaHostAllocMapped));
+                std::memset(h_session_, 0, sizeof(ds::SessionCtl) + ds::kSnapshotHdr + result_stride_);
+                CB2_CUDA(cudaHostGetDevicePointer(reinterpret_cast<void**>(&d_session_), h_session_, 0));
+            }
             uint32_t visit_budget = 24;  // measured on hex5 (sim_num 1400, whole games): 24 -> 57.1 M sims/s, 48 -> 54.4 M, 96 -> 49.4 M
             if (const char* vb = std::getenv("CATTUS_B200_DSEARCH_VISIT_BUDGET")) visit_budget = static_cast<uint32_t>(std::max(1, std::atoi(vb)));
 
@@ -231,7 +262,7 @@ class DsCudaBackend {
                     p.eval[e].prob_stride = io.moves < max_children ? io.moves : max_children;
                     p.eval[e].max_rows = io.max_batch;
                     p.eval[e].plane_words = io.plane_words;
-                    p.sim_num[e] = params[e].sim_num;
+                    p.sim_num[e] = session_ ? 0u : params[e].sim_num;
                     p.explore[e] = params[e].explore_factor;
                     p.noise_eps[e] = params[e].noise_eps;
                     p.cache[e] = ds::CacheIo{};
@@ -282,6 +313,10 @@ class DsCudaBackend {
                     p.descents = static_cast<ds::BatchDescent*>(d_descents_) + static_cast<size_t>(base) * search_batch_;
                     p.bpaths = static_cast<ds::PathStep*>(d_bpaths_) + static_cast<size_t>(base) * search_batch_ * path_cap;
                     p.vcount = static_cast<uint32_t*>(d_vcount_) + static_cast<size_t>(base) * (pool_words_ >> 2);
+                }
+                if (session_) {
+                    p.session = reinterpret_cast<volatile ds::SessionCtl*>(d_session_);
+                    p.snapshot = d_session_ + sizeof(ds::SessionCtl);
                 }
                 if (begin_lead) {
                     CB2_CUDA(cudaStreamCreateWithFlags(&P.side, cudaStreamNonBlocking));
@@ -355,6 +390,22 @@ class DsCudaBackend {
     uint32_t max_used() const { return max_used_; }
     uint64_t waves() const { return waves_; }
     uint32_t kernels_per_wave() const { return kernels_per_wave_; }
+    // a session's control words and snapshot (mapped pinned memory the device reads and writes while the host does)
+    volatile ds::SessionCtl* session_ctl() { return reinterpret_cast<volatile ds::SessionCtl*>(h_session_); }
+    const uint8_t* snapshot() const { return h_session_ + sizeof(ds::SessionCtl); }
+    void bind_thread() { CB2_CUDA(cudaSetDevice(device_)); }
+    // A session goes on after a search that met a device error (ErrBits): the sticky error word is cleared, and so are the
+    // virtual counts the failed minibatch left behind (its backup never ran).  The next search starts from a fresh root.
+    void clear_error() {
+        DsPopulation<Rules>& P = pop_[0];
+        CB2_CUDA(cudaMemsetAsync(static_cast<uint32_t*>(P.d_status) + 1, 0, 4, P.stream));
+        if (d_vcount_) CB2_CUDA(cudaMemsetAsync(d_vcount_, 0, sizeof(uint32_t) * static_cast<size_t>(n_slots_) * (pool_words_ >> 2), P.stream));
+        CB2_CUDA(cudaStreamSynchronize(P.stream));
+    }
+    int error_code(const std::exception& e) const {
+        const Error* ce = dynamic_cast<const Error*>(&e);
+        return ce ? ce->code : CATTUS_B200_EDEVICE;
+    }
 
   private:
     void alloc(void*& ptr, size_t bytes) {
@@ -376,6 +427,8 @@ class DsCudaBackend {
                 CB2_CUDA(cudaStreamWaitEvent(P.side, P.fork, 0));
                 ds_begin_kernel<Rules><<<blocks, 128, 0, P.side>>>(P.p);
                 CB2_CUDA(cudaEventRecord(P.join, P.side));
+            } else if (session_) {
+                ds_begin_session_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             } else {
                 ds_begin_kernel<Rules><<<blocks, 128, 0, P.stream>>>(P.p);
             }
@@ -435,7 +488,8 @@ class DsCudaBackend {
         if (h_cmds_) cudaFreeHost(h_cmds_);
         if (h_status_) cudaFreeHost(h_status_);
         if (h_roots_) cudaFreeHost(h_roots_);
-        h_results_ = h_cmds_ = h_status_ = nullptr;
+        if (h_session_) cudaFreeHost(h_session_);
+        h_results_ = h_cmds_ = h_status_ = h_session_ = d_session_ = nullptr;
         h_roots_ = nullptr;
     }
 
@@ -447,7 +501,9 @@ class DsCudaBackend {
     size_t cmd_bytes_ = 0, result_buf_bytes_ = 0;
     void *d_rules_ = nullptr, *d_slots_ = nullptr, *d_pools_ = nullptr, *d_paths_ = nullptr, *d_noise_ = nullptr, *d_hist_ = nullptr;
     void *d_descents_ = nullptr, *d_bpaths_ = nullptr, *d_vcount_ = nullptr;
-    uint8_t *h_results_ = nullptr, *h_cmds_ = nullptr, *h_status_ = nullptr;
+    uint8_t *h_results_ = nullptr, *h_cmds_ = nullptr, *h_status_ = nullptr, *h_session_ = nullptr, *d_session_ = nullptr;
+    int device_ = 0;
+    bool session_ = false;
     typename Rules::Pos* h_roots_ = nullptr;
     std::vector<cudaEvent_t> events_;
     std::vector<uint32_t> wave_pop_;
@@ -607,6 +663,55 @@ void match_run(cattus_b200_t* ma, cattus_b200_t* mb, const cattus_b200_selfplay_
         } else {
             throw Error(CATTUS_B200_EINVAL, "unknown game");
         }
+    } catch (const sp::SpError& e) {
+        throw Error(e.code ? e.code : CATTUS_B200_EINVAL, e.msg);
+    }
+}
+
+// A session (dsearch_session.hpp) on model's device: the analysis backend with one slot, the session's begin and the
+// session's tree size; the driver owns the backend and its evaluator lane.
+template <class Rules>
+static std::unique_ptr<ds::SessionBase> session_rules(const Rules& rules, const void* blob, size_t blob_bytes, uint32_t max_children, Engine* e,
+                                                      const cattus_b200_selfplay_cfg& cfg, const cattus_b200_session_opts* opts) {
+    cattus_b200_selfplay_cfg c = cfg;
+    c.sim_num = std::max<uint32_t>(c.sim_num, 2u);  // not used by a session; analysis_params checks it
+    const sp::Params params[2] = {ds::analysis_params(c), ds::analysis_params(c)};
+    cattus_b200_info info;
+    e->get_info(&info);
+    if (info.game != cfg.game || (cfg.game == CATTUS_B200_GAME_HEX && info.board_size != cfg.board_size))
+        throw Error(CATTUS_B200_EINVAL, "session: the model was made for another game or board size than cfg");
+    if (info.n_streams < 2)
+        throw Error(CATTUS_B200_EINVAL, "session: a session holds one evaluator lane for its lifetime; create the model with n_streams >= 2");
+    const uint32_t L = ds::session_search_batch(opts, info.max_batch);
+    const uint32_t sides[2] = {L, L};
+    const ds::AnalysisOpts aopts{ds::kPvMax};
+    const uint32_t kwords = opts->tree_kwords;
+    std::unique_ptr<DsCudaBackend<Rules>> be(
+        new DsCudaBackend<Rules>(blob, blob_bytes, max_children, e, nullptr, c, params, 1, ds::hist_cap_for<Rules>(), sides, &aopts, &kwords));
+    return std::unique_ptr<ds::SessionBase>(new ds::SessionDriver<Rules, DsCudaBackend<Rules>>(rules, params[0], std::move(be), L));
+}
+
+std::unique_ptr<ds::SessionBase> session_create(cattus_b200_t* m, const cattus_b200_selfplay_cfg& cfg, const cattus_b200_session_opts* opts) {
+    try {
+        if (!m) throw Error(CATTUS_B200_EINVAL, "null evaluator handle (there is no CPU fallback)");
+        if (cfg.struct_size != sizeof(cattus_b200_selfplay_cfg)) throw Error(CATTUS_B200_EINVAL, "selfplay cfg struct_size mismatch");
+        if (cfg.game == CATTUS_B200_GAME_HEX) {
+            const int s = static_cast<int>(cfg.board_size);
+            if (s < 2 || s > 11) throw Error(CATTUS_B200_EINVAL, "hex board_size must be 2..11");
+            if (s <= 8) {
+                sp::HexRulesT<uint64_t> rules(s);
+                return session_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, opts);
+            }
+            sp::HexRulesT<sp::u128> rules(s);
+            return session_rules(rules, &rules, sizeof(rules), static_cast<uint32_t>(s * s), m->engine, cfg, opts);
+        } else if (cfg.game == CATTUS_B200_GAME_CHESS) {
+            sp::ChessRules rules;
+            return session_rules(rules, &sp::chess_tables(), sizeof(sp::ChessTables), static_cast<uint32_t>(sp::ChessRules::kMaxMoves), m->engine, cfg, opts);
+        } else if (cfg.game == CATTUS_B200_GAME_TTT) {
+            sp::TttRules rules;
+            return session_rules(rules, &rules, sizeof(rules), 9u, m->engine, cfg, opts);
+        }
+        throw Error(CATTUS_B200_EINVAL, "unknown game");
     } catch (const sp::SpError& e) {
         throw Error(e.code ? e.code : CATTUS_B200_EINVAL, e.msg);
     }

@@ -82,7 +82,73 @@ struct AnalysisResult {
     std::vector<uint16_t> pv;
     uint32_t minibatches = 0;  // rounds of descents (one leaf in flight: one per simulation)
     uint32_t collisions = 0;   // descents that ended on a leaf an earlier descent of their minibatch had claimed
+    // a session's search (dsearch_session.hpp): the root's visits kept from the previous search, why it ended
+    // (cattus_b200_session.h's CATTUS_B200_STOP_*) and its seconds; zero elsewhere
+    uint32_t reused = 0, stop_reason = 0;
+    double seconds = 0.0;
 };
+
+// a move of the device's tree in the game's real encoding (chess trees hold the side to move's view)
+template <class Rules>
+uint16_t analysis_real_move(const typename Rules::Pos& p, uint32_t m) {
+    if constexpr (Rules::kChess)
+        return Rules::real_move(p, static_cast<typename Rules::Move>(m));
+    else
+        return static_cast<uint16_t>(m);
+}
+
+// Fills `r` from a posted analysis entry `e` of the search of `root` (count and pv_len already checked): the children in
+// edges() order, the best move, q and the principal variation; with minibatches (search_batch > 1) the entry's counts.
+template <class Rules>
+void read_analysis_entry(const Rules& R, const sp::Params& params, const typename Rules::Pos& root, const uint8_t* e, uint32_t maxc,
+                         uint32_t result_stride, uint32_t search_batch, AnalysisResult& r,
+                         std::vector<std::pair<typename Rules::Move, float>>& probs, std::vector<float>& weights) {
+    using Pos = typename Rules::Pos;
+    using Move = typename Rules::Move;
+    const AnalysisHdr* ah = reinterpret_cast<const AnalysisHdr*>(e);
+    const uint32_t count = ah->count, pv_len = ah->pv_len;
+    const uint16_t* pv = reinterpret_cast<const uint16_t*>(e + sizeof(AnalysisHdr));
+    const uint32_t* rn = reinterpret_cast<const uint32_t*>(e + sizeof(AnalysisHdr) + 2u * kPvMax);
+    const float* rw = reinterpret_cast<const float*>(rn + maxc);
+    const float* ri = rw + maxc;
+    const uint16_t* rm = reinterpret_cast<const uint16_t*>(ri + maxc);
+    r.status = 0;
+    r.simulations = params.sim_num;
+    r.minibatches = params.sim_num;
+    r.collisions = 0;
+    if (search_batch > 1) {
+        const uint32_t* counts = reinterpret_cast<const uint32_t*>(e + result_stride - 16u);
+        r.minibatches = counts[0];
+        r.collisions = counts[1];
+    }
+    uint32_t total = 0;
+    double sw = 0.0;
+    for (uint32_t i = 0; i < count; ++i) {
+        total += rn[i];
+        sw += static_cast<double>(rw[i]);
+    }
+    r.moves.clear();
+    r.visits.clear();
+    r.w.clear();
+    r.prior.clear();
+    r.pv.clear();
+    probs.clear();
+    for (int32_t i = static_cast<int32_t>(count) - 1; i >= 0; --i) {  // edges() order
+        r.moves.push_back(analysis_real_move<Rules>(root, rm[i]));
+        r.visits.push_back(rn[i]);
+        r.w.push_back(rw[i]);
+        r.prior.push_back(ri[i]);
+        probs.emplace_back(static_cast<Move>(rm[i]), static_cast<float>(rn[i]) / static_cast<float>(total));
+    }
+    sp::SplitMix64 unused(0);
+    r.best = r.moves[static_cast<size_t>(sp::choose_move(params, 0, probs, unused, weights))];
+    r.q = total ? static_cast<float>(sw / static_cast<double>(total)) : 0.0f;
+    Pos p = root;
+    for (uint32_t j = 0; j < pv_len; ++j) {
+        r.pv.push_back(analysis_real_move<Rules>(p, pv[j]));
+        if (j + 1 < pv_len) p = R.moved(p, static_cast<Move>(pv[j]));
+    }
+}
 
 // MctsParams of an analysis: the mcts.* fields without root noise (a noisy search would not be an analysis of the
 // position, and its samples would depend on the order of the positions).
@@ -285,56 +351,11 @@ class AnalysisDriver {
             throw sp::SpError{CATTUS_B200_EDEVICE, "device search posted a malformed result"};
         const size_t k = static_cast<size_t>(job_of_slot_[slot]);
         job_of_slot_[slot] = -1;
-        const uint16_t* pv = reinterpret_cast<const uint16_t*>(e + sizeof(AnalysisHdr));
-        const uint32_t* rn = reinterpret_cast<const uint32_t*>(e + sizeof(AnalysisHdr) + 2u * kPvMax);
-        const float* rw = reinterpret_cast<const float*>(rn + maxc);
-        const float* ri = rw + maxc;
-        const uint16_t* rm = reinterpret_cast<const uint16_t*>(ri + maxc);
-        const Pos& root = hist_[k].back();
-        AnalysisResult& r = out_[k];
-        r.status = 0;
-        r.simulations = params_.sim_num;
-        r.minibatches = params_.sim_num;
-        r.collisions = 0;
-        if (search_batch_ > 1) {
-            const uint32_t* counts = reinterpret_cast<const uint32_t*>(e + result_stride_ - 16u);
-            r.minibatches = counts[0];
-            r.collisions = counts[1];
-        }
-        uint32_t total = 0;
-        double sw = 0.0;
-        for (uint32_t i = 0; i < count; ++i) {
-            total += rn[i];
-            sw += static_cast<double>(rw[i]);
-        }
-        probs_.clear();
-        for (int32_t i = static_cast<int32_t>(count) - 1; i >= 0; --i) {  // edges() order
-            r.moves.push_back(real(root, rm[i]));
-            r.visits.push_back(rn[i]);
-            r.w.push_back(rw[i]);
-            r.prior.push_back(ri[i]);
-            probs_.emplace_back(static_cast<Move>(rm[i]), static_cast<float>(rn[i]) / static_cast<float>(total));
-        }
-        sp::SplitMix64 unused(0);
-        r.best = r.moves[static_cast<size_t>(sp::choose_move(params_, 0, probs_, unused, weights_))];
-        r.q = total ? static_cast<float>(sw / static_cast<double>(total)) : 0.0f;
-        Pos p = root;
-        for (uint32_t j = 0; j < pv_len; ++j) {
-            r.pv.push_back(real(p, pv[j]));
-            if (j + 1 < pv_len) p = R.moved(p, static_cast<Move>(pv[j]));
-        }
+        read_analysis_entry(R, params_, hist_[k].back(), e, maxc, result_stride_, search_batch_, out_[k], probs_, weights_);
         const uint32_t pop = be_.population_of(slot);
         free_[pop].push_back(slot);
         active_ -= 1;
         active_pop_[pop] -= 1;
-    }
-
-    // a move of the device's tree in the game's real encoding (chess trees hold the side to move's view)
-    static uint16_t real(const Pos& p, uint32_t m) {
-        if constexpr (kChess)
-            return Rules::real_move(p, static_cast<Move>(m));
-        else
-            return static_cast<uint16_t>(m);
     }
 
     const Rules& R;

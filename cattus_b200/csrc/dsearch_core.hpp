@@ -143,6 +143,14 @@ CB2_HD inline void atomic_add_u64(unsigned long long* p, unsigned long long v) {
     *p += v;
 #endif
 }
+// orders this thread's earlier writes to mapped host memory before its later ones, as the host sees them
+CB2_HD inline void fence_system() {
+#if DS_DEVICE
+    __threadfence_system();
+#else
+    __atomic_thread_fence(__ATOMIC_SEQ_CST);
+#endif
+}
 CB2_HD inline void atomic_max_u32(uint32_t* p, uint32_t v) {
 #if DS_DEVICE
     atomicMax(p, v);
@@ -184,7 +192,7 @@ CB2_HD inline float fsqrt(float a) {
 
 // ------------------------------------------------------------------------------------------------ layouts
 enum Phase : uint32_t { kIdle = 0, kRun = 1, kWaitEval = 2, kDone = 3 };
-enum CmdFlags : uint32_t { kCmdNewGame = 1, kCmdMove = 2, kCmdStop = 4, kCmdSetRoot = 8 };
+enum CmdFlags : uint32_t { kCmdNewGame = 1, kCmdMove = 2, kCmdStop = 4, kCmdSetRoot = 8, kCmdKeepTree = 16 };
 enum ErrBits : uint32_t { kErrPool = 1, kErrPath = 2, kErrRows = 4, kErrNoise = 8 };
 
 // One per concurrent game.  Scalars only; the per-slot arrays (tree pools, path, noise, history) are separate.
@@ -279,6 +287,20 @@ struct SearchBatch {
     }
 };
 
+// A session (dsearch_session.hpp, DESIGN.md section 17) keeps one tree across searches.  Its control words live in mapped
+// pinned memory: the host writes them, the device reads them in begin and at every minibatch boundary.
+enum StopReason : uint32_t { kStopNone = 0, kStopNodes = 1, kStopMinibatches = 2, kStopRequest = 3, kStopDeadline = 4, kStopCapacity = 5 };
+struct SessionCtl {
+    uint32_t nodes;            // node budget of the search: new simulations on top of the kept tree (0xFFFFFFFF: none)
+    uint32_t max_minibatches;  // minibatch cap (0xFFFFFFFF: none)
+    uint32_t stop;             // kStopRequest / kStopDeadline: end at the next minibatch boundary
+    uint32_t info;             // 1: post a snapshot after the next minibatch (the device clears it)
+};
+// A session's snapshot buffer: [u32 seq][u32 sims_done][u32 minibatches][u32 collisions] then one entry of the analysis
+// result layout (result_stride bytes).  seq is odd while the device writes it; the last write is the even seq, behind a
+// system-scope fence.
+constexpr uint32_t kSnapshotHdr = 16;
+
 template <class Rules>
 struct Params {
     const void* rules;  // device copy of the rule tables (HexRulesT / ChessTables; unused for tic-tac-toe)
@@ -318,6 +340,10 @@ struct Params {
     BatchDescent* descents;     // [n_slots][search_batch.max]
     PathStep* bpaths;           // [n_slots][search_batch.max][path_cap]
     uint32_t* vcount;           // [n_slots][pool_words / 4]: virtual count of each child row (16-byte pool unit) of the tree
+    // session (one slot searched in minibatches, begin_slot<true>); null outside sessions.  A session's sim_num is 0:
+    // its budget is SessionCtl::nodes, and its begin resets the minibatch counts.
+    volatile SessionCtl* session;
+    uint8_t* snapshot;
 };
 
 template <class Pos>
@@ -495,11 +521,18 @@ struct Core {
     // Returns the posted entry.
     CB2_HD static uint8_t* post_analysis(const P& p, uint32_t wave, uint32_t si, uint32_t* pool, int32_t root) {
         const int ln = lane();
-        const int count = T::hdr(pool, root)->count;
         uint32_t k = 0;
         if (ln == 0) k = atomic_add_u32(p.done_count, 1u);
         k = wbcast(k);
         uint8_t* e = p.results + static_cast<unsigned long long>(wave % p.n_result_bufs) * p.result_buf_bytes + static_cast<size_t>(k) * p.result_stride;
+        write_analysis(p, e, si, pool, root);
+        return e;
+    }
+
+    // The analysis entry of the tree at `root`, written at `e`.
+    CB2_HD static void write_analysis(const P& p, uint8_t* e, uint32_t si, uint32_t* pool, int32_t root) {
+        const int ln = lane();
+        const int count = T::hdr(pool, root)->count;
         uint16_t* pv = reinterpret_cast<uint16_t*>(e + sizeof(AnalysisHdr));
         uint32_t* rn = reinterpret_cast<uint32_t*>(e + sizeof(AnalysisHdr) + 2u * kPvMax);
         float* rw = reinterpret_cast<float*>(rn + p.max_children);
@@ -544,7 +577,6 @@ struct Core {
             ah->pv_len = len;
             ah->pad = 0;
         }
-        return e;
     }
 
     // MctsPlayer::detect_repetition (mod.rs:133-154), as the host driver does it: each path position is counted
@@ -1176,15 +1208,23 @@ struct Core {
         const uint32_t left = Q.sims_left - n_sims, minibatches = Q.pad[0] + 1u, collisions = Q.pad[1] + n_coll;
         wsync();
         uint32_t phase = kRun;
-        if (left == 0) {
+        uint32_t reason = left == 0 ? kStopNodes : kStopNone;
+        // the host writes the session's words at any time: lane 0 reads them and the warp takes its decision
+        if (p.session && reason == kStopNone) reason = wbcast(ln == 0 ? session_stop(p, Q.used[cur & 1u], minibatches) : 0u);
+        if (reason != kStopNone) {
             uint8_t* entry = post_results(p, wave, si, pool, root);
             if (ln == 0) {  // the analysis entry ends in the two counts; the self-play one has them in ResultHdr::pad
                 uint32_t* counts = p.analysis ? reinterpret_cast<uint32_t*>(entry + p.result_stride - 16u) : reinterpret_cast<ResultHdr*>(entry)->pad;
                 counts[0] = minibatches;
                 counts[1] = collisions;
+                if (p.session) {  // a session's entry also carries the visits the search kept and why it ended
+                    counts[2] = Q.row;
+                    counts[3] = reason;
+                }
             }
             phase = kDone;
         }
+        if (p.session && (reason != kStopNone || wbcast(ln == 0 ? p.session->info : 0u) != 0u)) post_snapshot(p, si, pool, root, left, minibatches, collisions);
         if (ln == 0) {
             Q.phase = phase;
             Q.sims_left = left;
@@ -1192,6 +1232,43 @@ struct Core {
             Q.pad[1] = collisions;
             if (n_sims) atomic_add_u64(p.counters + 0, n_sims);
             if (n_scored) atomic_add_u64(p.counters + 2, n_scored);
+        }
+    }
+
+    // Why a session's search ends at this minibatch boundary besides its node budget (kStopNone: it goes on): the minibatch
+    // cap, a stop or deadline the host wrote, or a tree buffer that might not hold another minibatch's new leaves.
+    CB2_HD static uint32_t session_stop(const P& p, uint32_t used, uint32_t minibatches) {
+        if (minibatches >= p.session->max_minibatches) return kStopMinibatches;
+        const uint32_t stop = p.session->stop;
+        if (stop != kStopNone) return stop;
+        if (static_cast<unsigned long long>(used) + minibatch_words(p) > p.pool_words) return kStopCapacity;
+        return kStopNone;
+    }
+    // the most a minibatch can add to a tree: each descent materialises at most one node
+    CB2_HD static unsigned long long minibatch_words(const P& p) {
+        return static_cast<unsigned long long>(p.search_batch.max) * T::block_words(static_cast<int>(p.max_children));
+    }
+
+    // The session's snapshot: the analysis entry of the tree as it stands, with the search's counts, behind a sequence
+    // word the host checks before and after it reads.
+    CB2_HD static void post_snapshot(const P& p, uint32_t si, uint32_t* pool, int32_t root, uint32_t left, uint32_t minibatches, uint32_t collisions) {
+        const int ln = lane();
+        volatile uint32_t* hdr = reinterpret_cast<volatile uint32_t*>(p.snapshot);
+        const uint32_t seq = wbcast(ln == 0 ? hdr[0] : 0u) | 1u;
+        if (ln == 0) hdr[0] = seq;
+        fence_system();
+        wsync();
+        write_analysis(p, p.snapshot + kSnapshotHdr, si, pool, root);
+        if (ln == 0) {
+            hdr[1] = p.session->nodes - left;
+            hdr[2] = minibatches;
+            hdr[3] = collisions;
+        }
+        wsync();
+        fence_system();
+        if (ln == 0) {
+            hdr[0] = seq + 1u;
+            p.session->info = 0;
         }
     }
 
@@ -1368,6 +1445,10 @@ struct Core {
 
     // One host command: optional new game / move, then calc_moves_probabilities up to develop_tree (mod.rs:335-362) for
     // the player `cur`: find the position in the kept tree, keep its subtree, else start from a fresh root.
+    // kSession (a session's begin, DESIGN.md section 17): kCmdSetRoot | kCmdKeepTree installs the history but looks for its
+    // last position in the kept tree; a kept tree that cannot be copied, or has no room for one more minibatch, gives way
+    // to a fresh root; the budget is SessionCtl::nodes, and the slot records the root's visits before the search in `row`.
+    template <bool kSession = false>
     CB2_HD static void begin_slot(const Rules& R, const P& p, uint32_t ci, uint32_t wave) {
         const uint8_t* cb = p.cmds + 16 + static_cast<size_t>(ci) * p.cmd_stride;
         const Cmd cmd = *reinterpret_cast<const Cmd*>(cb);
@@ -1396,10 +1477,12 @@ struct Core {
             if (ln == 0) hist[0] = R.initial();
         } else if (cmd.flags & kCmdSetRoot) {
             // a fresh tree at a position the host gives, with the history detect_repetition looks back into
-            root[0] = root[1] = -1;
-            used[0] = used[1] = 0;
-            buf[0] = 0;
-            buf[1] = 1;
+            if (!kSession || !(cmd.flags & kCmdKeepTree)) {
+                root[0] = root[1] = -1;
+                used[0] = used[1] = 0;
+                buf[0] = 0;
+                buf[1] = 1;
+            }
             hist_len = cmd.root_len;
             for (uint32_t i = static_cast<uint32_t>(ln); i < hist_len; i += DS_LANES) hist[i] = p.roots[cmd.root_at + i];
         } else if (cmd.flags & kCmdMove) {
@@ -1424,7 +1507,7 @@ struct Core {
         bool reused = false;
         if (t.root >= 0) {
             const int32_t node = find_node_with_position(R, p, t, position);
-            if (node == -2) {
+            if (node == -2 && !kSession) {
                 err = kErrPool;
             } else if (node >= 0) {
                 if (node != t.root) {
@@ -1437,11 +1520,18 @@ struct Core {
                         buf[cur] = spare;
                         t = nt;
                         reused = true;
+                    } else if (kSession) {
+                        t.root = -1;
+                        t.used = 0;
                     } else {
                         err = kErrPool;
                     }
                 }
             } else {
+                t.root = -1;
+                t.used = 0;
+            }
+            if (kSession && !err && t.root >= 0 && static_cast<unsigned long long>(t.used) + minibatch_words(p) > p.pool_words) {
                 t.root = -1;
                 t.used = 0;
             }
@@ -1464,6 +1554,14 @@ struct Core {
                 noise_n = 0;
             }
         }
+        uint32_t kept = 0;  // sessions: the root's visits before the search
+        if (kSession && !err) {
+            const Hdr* rh = T::hdr(t.pool, t.root);
+            int part = 0;
+            if (rh->expanded)
+                for (int i = ln; i < rh->count; i += DS_LANES) part += T::child(t.pool, t.root)[i].n;
+            kept = static_cast<uint32_t>(wsum(part));
+        }
         if (ln == 0) {
             root[cur] = t.root;
             used[cur] = t.used;
@@ -1479,6 +1577,12 @@ struct Core {
             S.noise_n = noise_n;
             S.leaf = -1;
             S.path_len = 0;
+            if (kSession) {
+                S.sims_left = p.session->nodes;
+                S.row = kept;
+                S.pad[0] = 0;
+                S.pad[1] = 0;
+            }
             if (err) {
                 atomic_or_u32(p.error, err);
                 S.error = err;

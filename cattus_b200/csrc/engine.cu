@@ -2078,6 +2078,18 @@ static int guarded(F&& f) {
     }
 }
 
+// a session call: SpError (the host driver's) carries its own code
+template <class F>
+static int session_guarded(F&& f) {
+    return guarded([&] {
+        try {
+            f();
+        } catch (const sp::SpError& e) {
+            throw cb2::Error(e.code ? e.code : CATTUS_B200_EINVAL, e.msg);
+        }
+    });
+}
+
 extern "C" {
 
 int cattus_b200_create_from_memory(const cattus_b200_desc* desc, const void* blob, size_t blob_bytes, cattus_b200_t** out) {
@@ -2262,6 +2274,70 @@ int cattus_b200_analysis_batches(const cattus_b200_analysis_t* r, uint32_t k, ui
     return r ? ds::analysis_batches(r->res, k, minibatches, collisions) : CATTUS_B200_EINVAL;
 }
 void cattus_b200_analysis_free(cattus_b200_analysis_t* r) { delete r; }
+
+// ---------------------------------------------------------------- persistent search sessions (include/cattus_b200_session.h)
+struct cattus_b200_session {
+    std::unique_ptr<ds::SessionBase> s;
+};
+
+int cattus_b200_session_create(cattus_b200_t* model, const cattus_b200_selfplay_cfg* cfg, const cattus_b200_session_opts* opts,
+                               cattus_b200_session_t** out) {
+    return session_guarded([&] {
+        if (!cfg || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        *out = nullptr;
+        std::unique_ptr<cattus_b200_session> r(new cattus_b200_session());
+        r->s = cb2::session_create(model, *cfg, opts);
+        *out = r.release();
+    });
+}
+int cattus_b200_session_set_position(cattus_b200_session_t* s, const char* fen, const uint16_t* moves, uint32_t n) {
+    return session_guarded([&] {
+        if (!s) throw cb2::Error(CATTUS_B200_EINVAL, "null session");
+        s->s->set_position(fen, moves, n);
+    });
+}
+int cattus_b200_session_new_game(cattus_b200_session_t* s) {
+    return session_guarded([&] {
+        if (!s) throw cb2::Error(CATTUS_B200_EINVAL, "null session");
+        s->s->new_game();
+    });
+}
+int cattus_b200_session_go(cattus_b200_session_t* s, const cattus_b200_session_limits* limits) {
+    return session_guarded([&] {
+        if (!s || !limits) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        s->s->go(*limits);
+    });
+}
+int cattus_b200_session_stop(cattus_b200_session_t* s) {
+    return session_guarded([&] {
+        if (!s) throw cb2::Error(CATTUS_B200_EINVAL, "null session");
+        s->s->stop();
+    });
+}
+int cattus_b200_session_info(cattus_b200_session_t* s, cattus_b200_session_snapshot* out) {
+    return session_guarded([&] {
+        if (!s || !out) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        if (out->struct_size != sizeof(cattus_b200_session_snapshot)) throw cb2::Error(CATTUS_B200_EINVAL, "session snapshot struct_size mismatch");
+        s->s->info(*out);
+    });
+}
+int cattus_b200_session_wait(cattus_b200_session_t* s, uint32_t timeout_ms, cattus_b200_analysis_t** result) {
+    bool done = false;
+    std::unique_ptr<cattus_b200_analysis> r(new cattus_b200_analysis());
+    const int rc = session_guarded([&] {
+        if (!s || !result) throw cb2::Error(CATTUS_B200_EINVAL, "null argument");
+        *result = nullptr;
+        done = s->s->wait(timeout_ms, r->res);
+    });
+    if (rc != CATTUS_B200_OK) return rc;
+    if (!done) return CATTUS_B200_SESSION_RUNNING;
+    *result = r.release();
+    return CATTUS_B200_OK;
+}
+int cattus_b200_session_result_stats(const cattus_b200_analysis_t* r, cattus_b200_session_stats* out) {
+    return r ? ds::session_stats(r->res, out) : CATTUS_B200_EINVAL;
+}
+void cattus_b200_session_destroy(cattus_b200_session_t* s) { delete s; }
 
 // ---------------------------------------------------------------- match play from openings (include/cattus_b200_match.h)
 struct cattus_b200_match {
